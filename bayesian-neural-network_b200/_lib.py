@@ -65,6 +65,7 @@ _SIGS = {
     'bbb_snr': ([P, P, I64, P, P], C.c_int),
     'bbb_snr_prune': ([P, P, I64, F32, P, P], C.c_int),
     'bbb_softmax_mean': ([P, I64, I64, I64, P, P], C.c_int),
+    'bbb_predictive_stats': ([P, P, I64, I64, I64, I32, F32, I32, P, P, P, P, P], C.c_int),
     'bbb_nll_ce': ([P, P, I64, I64, I64, F32, P, P, P], C.c_int),
     'bbb_nll_gauss': ([P, P, F32, I64, I64, I64, F32, P, P, P], C.c_int),
     'bbb_head_fwd': ([P, I64, P, P, P, P, P, P, P, P, I64, I64, I64, I64, I32, I32, P, F32, F32, P, P, P, P, P, F32,

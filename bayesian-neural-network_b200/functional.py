@@ -904,3 +904,127 @@ def softmax_mean(logits):
     out = torch.empty((B, Cc), dtype=torch.float32, device=z.device)
     L.check(L.lib().bbb_softmax_mean(L.ptr(z), S, B, Cc, L.ptr(out), L.stream()), 'bbb_softmax_mean')
     return out
+
+
+# =========================================================================================
+# posterior predictive: uncertainty and calibration of the sampled outputs (bbb_predictive_stats)
+# =========================================================================================
+PREDICTIVE_BUDGET_BYTES = 256 << 20      # bound on one chunk's fp32 activations, S * rows * sum of widths * 4 B
+
+
+def predictive_acc_len(mode, n_bins):
+    """Length of the fp64 aggregate vector of bbb_predictive_stats (include/bbb.h)."""
+    return 5 + 3 * n_bins if mode == 'classification' else 4
+
+
+def _predictive_launch(out, target, mode, sigma, n_bins, mean, row_stats, pred, acc):
+    S, B, Cc = out.shape
+    kind = L.NLL_CE if mode == 'classification' else L.NLL_GAUSS
+    L.check(L.lib().bbb_predictive_stats(L.ptr(out), L.ptr(target), S, B, Cc, kind, float(sigma), int(n_bins),
+                                         L.ptr(mean), L.ptr(row_stats), L.ptr(pred), L.ptr(acc), L.stream()),
+            'bbb_predictive_stats')
+
+
+def _predictive_target(target, mode, B, Cc):
+    """The target as the kernel reads it, row for row: int64 [B] labels, or float [B, D] ([B] when D = 1)."""
+    if target is None:
+        return None
+    L.require_cuda(target)
+    if mode == 'classification':
+        if target.dtype != torch.int64 or tuple(target.shape) != (B,):
+            raise ValueError(f'classification target must be int64 of shape ({B},), got {target.dtype} '
+                             f'{tuple(target.shape)}')
+        return target.contiguous()
+    if not (tuple(target.shape) == (B, Cc) or (Cc == 1 and tuple(target.shape) == (B,))):
+        raise ValueError(f'regression target must have shape ({B}, {Cc})' + (f' or ({B},)' if Cc == 1 else '') +
+                         f', got {tuple(target.shape)}')
+    return _f32c(target).reshape(B, Cc)
+
+
+def _predictive_outputs(B, Cc, mode, n_bins, target, device):
+    k = 5 if mode == 'classification' else Cc + 1
+    mean = torch.empty((B, Cc), dtype=torch.float32, device=device)
+    row_stats = torch.empty((B, k), dtype=torch.float32, device=device)
+    pred = torch.empty(B, dtype=torch.int64, device=device) if mode == 'classification' else None
+    acc = torch.zeros(predictive_acc_len(mode, n_bins), dtype=torch.float64, device=device) if target is not None \
+        else None
+    return mean, row_stats, pred, acc
+
+
+def predictive_stats(out, target=None, mode='classification', sigma=1.0, n_bins=15):
+    """[S,B,C] sampled outputs -> (mean [B,C], row_stats [B,K], pred [B] or None, acc or None), device tensors, one
+    launch (bbb_predictive_stats; include/bbb.h gives every definition and the layout of row_stats and acc).
+    mode 'classification': the outputs are logits and target int64 [B]; 'regression': a Gaussian likelihood with
+    std `sigma` and target [B,D] ([B] when D = 1).  acc (the aggregates) only with a target."""
+    if mode not in ('classification', 'regression'):
+        raise ValueError(f"mode must be 'classification' or 'regression', got {mode!r}")
+    L.require_cuda(out)
+    z = _f32c(out)
+    S, B, Cc = z.shape
+    tgt = _predictive_target(target, mode, B, Cc)
+    mean, row_stats, pred, acc = _predictive_outputs(B, Cc, mode, n_bins, tgt, z.device)
+    _predictive_launch(z, tgt, mode, sigma, n_bins, mean, row_stats, pred, acc)
+    return mean, row_stats, pred, acc
+
+
+def predictive_chunk_rows(S, widths, budget=PREDICTIVE_BUDGET_BYTES):
+    """Rows per chunk that keep S * rows * sum(widths) * 4 bytes of activations under `budget`."""
+    return max(1, budget // (4 * S * sum(widths)))
+
+
+def predictive(x2, params, S, mode, target=None, sigma=1.0, n_bins=15, chunk_rows=None, prior=None, sigma_p=None,
+               tf32=False):
+    """Posterior predictive of a whole input set: the sampled forward (the kernels sample_predict runs) chunk by chunk,
+    each chunk's [S, rows, C] outputs summarised by bbb_predictive_stats into one set of per-row outputs and one set of
+    device aggregates.  Weight sampling when `prior` is given, local reparameterisation when `sigma_p` is.
+    Returns (mean, row_stats, pred, acc) as predictive_stats does.  Nothing here waits for the device.
+
+    Noise, and what chunking changes:
+      * weight sampling: eps is planned ONCE per call and every chunk reuses the plan (the same injected tensors in
+        the reference eps mode, the same Philox (seed, step) otherwise), so every row is scored by the same S posterior
+        networks and the result does not depend on chunk_rows beyond the kernels' round-off.  The call consumes one
+        Philox step, as sample_predict does.
+      * local reparameterisation: the noise is per row by construction; each chunk draws its own, which equals calling
+        the reference's predict chunk by chunk in order.  The call consumes one Philox step PER CHUNK.
+    chunk_rows=None picks the largest row count whose activations, S * rows * sum of layer widths * 4 bytes, stay
+    under PREDICTIVE_BUDGET_BYTES, and splits the rows into chunks of equal size."""
+    if mode not in ('classification', 'regression'):
+        raise ValueError(f"mode must be 'classification' or 'regression', got {mode!r}")
+    if (prior is None) == (sigma_p is None):
+        raise ValueError('give exactly one of prior (weight sampling) and sigma_p (local reparameterisation)')
+    L.require_cuda(x2, *[t for p in params for t in p])
+    x2 = _f32c(x2)
+    dev = x2.device
+    B = x2.shape[0]
+    params = [tuple(_f32c(t) for t in p) for p in params]
+    lr = sigma_p is not None
+    widths = [p[0].shape[1] if lr else p[0].shape[0] for p in params]
+    Cc = widths[-1]
+    tgt = _predictive_target(target, mode, B, Cc)
+    mean, row_stats, pred, acc = _predictive_outputs(B, Cc, mode, n_bins, tgt, dev)
+    if B == 0:
+        return mean, row_stats, pred, acc
+    if chunk_rows is None:
+        # (the local-reparameterisation forward also keeps a delta buffer per layer)
+        n_chunks = -(-B // predictive_chunk_rows(S, widths * (2 if lr else 1)))
+        chunk_rows = -(-B // n_chunks)
+    chunk_rows = int(chunk_rows)
+    if chunk_rows < 1:
+        raise ValueError(f'chunk_rows must be >= 1, got {chunk_rows}')
+    if not lr:
+        eps = plan_eps([(tuple(p[0].shape), (p[0].shape[0],)) for p in params], S, dev, True)
+    scratch = torch.zeros(2 * S, dtype=torch.float64, device=dev)    # log-prob slots the forward does not fill
+    for r0 in range(0, B, chunk_rows):
+        r1 = min(B, r0 + chunk_rows)
+        xc = x2[r0:r1]
+        if xc.data_ptr() % 16:     # keep the 16-byte row loads (and so the kernel family) of an unchunked call
+            xc = xc.clone()
+        if lr:
+            eps = plan_eps(_lr_eps_shapes(params, r1 - r0), S, dev, True)
+            ys, _ = _net_lr_forward(xc, params, float(sigma_p), S, eps, True, False, scratch[:1], tf32)
+        else:
+            ys = _net_ws_forward(xc, params, prior, S, eps, True, False, tf32, scratch[:S], scratch[S:])
+        _predictive_launch(ys[-1], None if tgt is None else tgt[r0:r1], mode, sigma, n_bins, mean[r0:r1],
+                           row_stats[r0:r1], None if pred is None else pred[r0:r1], acc)
+        del ys                     # free this chunk's activations before the next chunk allocates its own
+    return mean, row_stats, pred, acc

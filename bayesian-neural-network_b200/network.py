@@ -1,12 +1,59 @@
 """BayesianNetwork (networks.py:140-225) on the CUDA kernels, plus the two stock baselines the
 reference's callers import by name (MLP, MLP_Dropout: plain torch.nn, not part of the hot path)."""
+import math
 import os
+from dataclasses import dataclass
+from typing import Optional
 
 import torch
 from torch import nn
 
 from . import functional as F
 from .layers import BayesianLinear, BayesianLinearLR
+
+
+@dataclass
+class PredictiveResult:
+    """What BayesianNetwork.predictive returns: per-row device tensors and the device aggregates behind metrics().
+
+    classification: mean [B,C] (mean over the samples of softmax), pred [B] (argmax of mean, lowest index on ties),
+    confidence [B] (mean[pred]), entropy [B] (of mean), expected_entropy [B] (mean over the samples of each softmax's
+    entropy: aleatoric), mutual_info [B] (entropy - expected_entropy, clamped at 0: epistemic).
+    regression: mean [B,D], variance [B,D] (epistemic, over the samples; total = variance + sigma**2).
+    log_pred [B]: log predictive density of each row's target (None without a target)."""
+    mean: torch.Tensor
+    pred: Optional[torch.Tensor] = None
+    confidence: Optional[torch.Tensor] = None
+    entropy: Optional[torch.Tensor] = None
+    expected_entropy: Optional[torch.Tensor] = None
+    mutual_info: Optional[torch.Tensor] = None
+    variance: Optional[torch.Tensor] = None
+    log_pred: Optional[torch.Tensor] = None
+    acc: Optional[torch.Tensor] = None       # fp64 aggregates of bbb_predictive_stats (include/bbb.h)
+    n_bins: int = 0
+
+    def metrics(self):
+        """The aggregates as python numbers; the one host read of a prediction.  Classification: dict(n, accuracy,
+        nll, brier, ece, bins) with bins[m] = (count, mean confidence, accuracy) of the confidences in (m/M, (m+1)/M]
+        (NaN for an empty bin) and ece = sum_m count_m |accuracy_m - confidence_m| / n.  Regression: dict(n, nll, rmse),
+        rmse over all n * D outputs.  nll is the mean negative log predictive density.  Raises ValueError without a
+        target, or when a label was outside [0, C)."""
+        if self.acc is None:
+            raise ValueError('metrics() needs the target: call predictive(x, samples, target=...)')
+        a = self.acc.cpu().tolist()
+        if a[1]:
+            raise ValueError(f'{int(a[1])} target label(s) outside [0, {self.mean.shape[1]}): those rows were not scored')
+        n = int(a[0])
+        div = (lambda v: v / n) if n else (lambda v: math.nan)
+        if self.pred is None:
+            return dict(n=n, nll=div(a[2]), rmse=math.sqrt(div(a[3]) / self.mean.shape[1]))
+        bins = []
+        ece = 0.0
+        for m in range(self.n_bins):
+            cnt, conf, cor = a[5 + 3 * m:8 + 3 * m]
+            bins.append((int(cnt), conf / cnt if cnt else math.nan, cor / cnt if cnt else math.nan))
+            ece += abs(cor - conf)
+        return dict(n=n, accuracy=div(a[3]), nll=div(a[2]), brier=div(a[4]), ece=div(ece), bins=bins)
 
 
 class BayesianNetwork(nn.Module):
@@ -100,6 +147,31 @@ class BayesianNetwork(nn.Module):
     def predict_proba(self, x, samples):
         """BNN_Classification.predict (class_task.py:81-87): softmax of every sampled forward, averaged."""
         return F.softmax_mean(self.sample_predict(x, samples))
+
+    def predictive(self, x, samples, target=None, sigma=1.0, n_bins=15, chunk_rows=None):
+        """Posterior predictive of `samples` sampled networks on the rows of x, with its uncertainty and, given the
+        targets, its calibration -> PredictiveResult (device tensors; .metrics() reads the aggregates).  Eval
+        semantics (sampled weights, no log-probs), no autograd, any depth, both estimators, fp32 or TF32 as the
+        network is set.  Classification: the outputs are logits and target int64 [B]; regression: likelihood
+        N(y; f, sigma^2) and target [B, D] ([B] when D = 1), matched row for row.
+        The rows are processed in chunks of chunk_rows (None: as many as keep the activations under a fixed budget,
+        functional.predictive).  With weight sampling every chunk is scored by the same `samples` networks, so the
+        result does not depend on chunk_rows beyond round-off, and the call consumes one Philox step, as
+        sample_predict does; with local reparameterisation each chunk draws its own noise (one step per chunk)."""
+        x2 = self._flat_input(x)
+        params = [l.params() for l in self.layers()]
+        with torch.no_grad():
+            if self.local_reparam:
+                mean, rs, pred, acc = F.predictive(x2, params, samples, self.mode, target, sigma, n_bins, chunk_rows,
+                                                   sigma_p=float(self.prior_init[0]), tf32=self.tf32)
+            else:
+                mean, rs, pred, acc = F.predictive(x2, params, samples, self.mode, target, sigma, n_bins, chunk_rows,
+                                                   prior=self._prior, tf32=self.tf32)
+        log_pred = rs[:, -1] if target is not None else None
+        if self.mode == 'classification':
+            return PredictiveResult(mean, pred, rs[:, 0], rs[:, 1], rs[:, 2], rs[:, 3], log_pred=log_pred, acc=acc,
+                                    n_bins=n_bins)
+        return PredictiveResult(mean, variance=rs[:, :-1], log_pred=log_pred, acc=acc)
 
     # ---- SNR pruning (SURVEY 8 f3; weight_pruning.py:81-115) on the (mu, rho) stream, one kernel pass per tensor ----
     def snr(self):

@@ -192,6 +192,33 @@ int bbb_snr(const float *mu, const float *rho, int64_t n, float *snr_out, void *
 int bbb_snr_prune(float *mu, float *rho, int64_t n, float threshold_db, unsigned long long *kept, void *stream);
 int bbb_softmax_mean(const float *logits, int64_t S, int64_t B, int64_t C, float *probs, void *stream);
 
+/* ---- posterior predictive: uncertainty and calibration of sampled outputs (one pass over [S,B,C]) ---------------------
+ * replaces the host-side analysis after the prediction loops of class_task.py:81-87 / reg_task.py:76-83 (mean +- std
+ * of reg_task.evaluate) and the ECE of the reference's compute_ece.py.  One warp per row, the row's S samples read once.
+ *   out     [S,B,C] sampled outputs (logits, or regression outputs with C = D);  1 <= C <= 1024, S >= 1
+ *   target  nullable: int64 [B] labels (BBB_NLL_CE) or float [B,D] (BBB_NLL_GAUSS; [B] when D = 1), row for row
+ *   kind    BBB_NLL_CE: p_s = softmax(out[s,b,:]).
+ *             mean [B,C] = pbar = (1/S) sum_s p_s;  pred [B] (nullable) = argmax pbar (lowest index on ties);
+ *             row_stats [B,5] = { confidence pbar[pred], entropy H[pbar] (0 log 0 = 0),
+ *               expected entropy (1/S) sum_s H[p_s] (aleatoric), mutual information max(H[pbar] - E H[p_s], 0)
+ *               (epistemic), log pbar[y] formed as LSE_s(log p_s[y]) - log S (NaN without a valid target) }
+ *           BBB_NLL_GAUSS: likelihood N(y; f_s, sigma^2).
+ *             mean [B,D] = mu = (1/S) sum_s f_s;  row_stats [B,D+1] = { epistemic variance (1/S) sum_s (f_s - mu)^2 per
+ *               output (total = that + sigma^2), log predictive density LSE_s(sum_d log N(y_d; f_s,d, sigma^2)) - log S }
+ *   n_bins  BBB_NLL_CE: 1..1024 confidence bins; bin m holds confidences in (m/M, (m+1)/M], i.e.
+ *           m = clamp(ceil(conf M) - 1, 0, M - 1)
+ *   acc     fp64 aggregates, ADDED to (required with a target, ignored without):
+ *             [0] rows counted n  [1] rows whose label is outside [0, C) (not read out of bounds, not counted in n or
+ *             the bins: the host reports them)  [2] sum -log pbar[y] / sum -lpd
+ *             BBB_NLL_CE:    [3] sum correct  [4] sum Brier sum_c (pbar_c - [c = y])^2
+ *                            [5 + 3m ..] bin m: count, sum confidence, sum correct      (5 + 3 n_bins doubles)
+ *             BBB_NLL_GAUSS: [3] sum_d (mu_d - y_d)^2                                    (4 doubles)
+ *           ECE = (1/n) sum_m |sum correct_m - sum confidence_m|.  Counts are integers, exact in fp64.
+ * B == 0 is a no-op.  Bad kind or shape, n_bins out of range, sigma <= 0, a null required pointer: BBB_EINVAL. */
+int bbb_predictive_stats(const float *out, const void *target, int64_t S, int64_t B, int64_t C, int32_t kind,
+                         float sigma, int32_t n_bins, float *mean, float *row_stats, int64_t *pred, double *acc,
+                         void *stream);
+
 /* ---- likelihood terms (BayesianNetwork.get_nll, networks.py:183-190) --------------------
  * nll += sum over (s, b) of the negative log likelihood; dout (nullable) = grad_scale * d nll / d out.
  * bbb_nll_ce:    logits [S,B,C], target int64 [B]       (CrossEntropyLoss(reduction='sum'))
