@@ -186,14 +186,15 @@ extern "C" int bbb_lr_linear_bwd(const float *dy, const float *dy_mask_src, cons
                                  float g_kl, const float *g_kl_dev, const float *out_scale_dev, float *dx,
                                  float *grad_w_mu, float *grad_w_rho, float *grad_b_mu, float *grad_b_rho,
                                  void *stream) {
-  BBB_CHECK_ARG(dy && x && w_mu && w_rho && b_mu && b_rho, "null pointer");
+  // empty batches carry null activations, as in bbb_linear_bwd
+  BBB_CHECK_ARG(w_mu && w_rho && b_mu && b_rho && ((dy && x) || S * B == 0), "null pointer");
   BBB_CHECK_ARG((flags & BBB_F_NO_WGRAD) || (grad_w_mu && grad_w_rho && grad_b_mu && grad_b_rho),
                 "null gradient pointer");
-  BBB_CHECK_ARG((flags & BBB_F_NO_DX) || dx, "dx required unless BBB_F_NO_DX");
+  BBB_CHECK_ARG((flags & BBB_F_NO_DX) || dx || S * B == 0, "dx required unless BBB_F_NO_DX");
   BBB_CHECK_ARG(S >= 0 && B >= 0 && in >= 0 && out >= 0 && S <= 65535 && sigma_p > 0, "bad shape or sigma_p");
   BBB_CHECK_ARG(x_sample_stride == 0 || x_sample_stride == B * in, "x_sample_stride must be 0 or B*in");
   const bool sample = flags & BBB_F_SAMPLE;
-  BBB_CHECK_ARG(!sample || delta, "delta (saved by the forward) required when sampling");
+  BBB_CHECK_ARG(!sample || delta || S * B == 0, "delta (saved by the forward) required when sampling");
   BBB_CHECK_ARG(!sample || (eps_a && eps_b) || (!eps_a && !eps_b && rng), "give both eps pointers or an rng");
   if (out == 0 || in == 0) return BBB_OK;
   LrArgs a{};

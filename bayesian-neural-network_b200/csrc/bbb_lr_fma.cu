@@ -376,7 +376,7 @@ int launch_lr_fwd_fma(const LrArgs &a, cudaStream_t st) {
 }
 
 int launch_lr_bwd_fma(const LrArgs &a, cudaStream_t st) {
-  if (!(a.flags & BBB_F_NO_DX)) {
+  if (!(a.flags & BBB_F_NO_DX) && a.S > 0 && a.B > 0) {   // an empty batch has no dx (and a zero grid is no launch)
     dim3 grid(cdiv(a.in, TN), cdiv(a.B, TM), (unsigned)a.S);
     lr_dgrad_kernel<<<grid, NT, 0, st>>>(a);
     BBB_CHECK_LAUNCH();

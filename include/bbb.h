@@ -95,6 +95,7 @@ uint64_t bbb_launch_count(void);
  *   w_mu,w_rho [out,in]; b_mu,b_rho [out]; eps_w [S,out,in] / eps_b [S,out] or NULL
  *   y      [S,B,out]   written
  *   logp, logq [S]     += sum log prior / sum log posterior over W and b (BBB_F_LOGPROB)
+ * S, B or out == 0: nothing is launched and no output is touched (logp / logq included).
  */
 int bbb_linear_fwd(const float *x, int64_t x_sample_stride, const float *w_mu, const float *w_rho,
                    const float *b_mu, const float *b_rho, const float *eps_w, const float *eps_b,
@@ -112,8 +113,11 @@ int bbb_linear_fwd_relu_out_supported(int64_t B, int64_t in, int64_t out, int32_
  *             (stride 0: one value for all samples, 1: per sample) -- autograd hands these over as
  *             device tensors and reading them on the device avoids a host synchronisation
  *   out_scale_dev optional device scalar multiplying every parameter gradient written (d loss upstream)
- *   dx        [S,B,in] written unless BBB_F_NO_DX (gradient w.r.t. the post-ReLU input)
- *   grad_*    same shapes as the parameters; overwritten, or added to with BBB_F_ACCUM
+ *   dx        [S,B,in] written unless BBB_F_NO_DX (gradient w.r.t. the post-ReLU input); with BBB_F_NO_DX a
+ *             non-NULL dx is left untouched
+ *   grad_*    same shapes as the parameters; overwritten, or added to with BBB_F_ACCUM; with BBB_F_NO_WGRAD
+ *             non-NULL gradient buffers are left untouched
+ *   B == 0 (or S == 0): no dx; the gradients reduce to the prior / posterior terms of the S samples
  */
 int bbb_linear_bwd(const float *dy, const float *dy_mask_src, const float *x, int64_t x_sample_stride,
                    const float *w_mu, const float *w_rho, const float *b_mu, const float *b_rho,
@@ -148,7 +152,8 @@ int bbb_linear_bwd_adam(const float *dy, const float *dy_mask_src, const float *
  * replaces BayesianLinearLR.forward (networks.py:116-138) and compute_kl_cost (109-114).
  *   w_mu,w_rho [in,out] (the reference's LR layout, networks.py:95-96)
  *   eps_a [S,B,out] / eps_b [S,out] or NULL (Philox)
- *   y [S,B,out] written;  delta [S,B,out] = sqrt(x^2 sigma^2) written when non-NULL (backward needs it)
+ *   y [S,B,out] written;  delta [S,B,out] = sqrt(x^2 sigma^2) written when non-NULL (backward needs it);
+ *     with BBB_F_OUT_ZEROED both y and delta must arrive zero-filled (the tcgen05 path adds partial sums into both)
  *   kl  += closed-form KL(q || N(0,sigma_p)) of W and b, ONCE per call (it is sample-independent)
  */
 int bbb_lr_linear_fwd(const float *x, int64_t x_sample_stride, const float *w_mu, const float *w_rho,
@@ -157,7 +162,9 @@ int bbb_lr_linear_fwd(const float *x, int64_t x_sample_stride, const float *w_mu
                       int32_t flags, float *y, float *delta, double *kl, void *stream);
 
 /* backward of the above (SURVEY App. A-3).  g_kl = d loss / d kl (host scalar), times
- * g_kl_dev[0] when non-NULL; out_scale_dev as in bbb_linear_bwd.
+ * g_kl_dev[0] when non-NULL, applied with BBB_F_LOGPROB only; out_scale_dev, BBB_F_NO_DX, BBB_F_NO_WGRAD,
+ * BBB_F_ACCUM and BBB_F_DX_PREACT as in bbb_linear_bwd.  B == 0 (or S == 0): dy, x, delta and dx may be NULL; no dx, and
+ * the gradients reduce to the KL terms.
  * With BBB_F_TF32 (tcgen05 path: B <= 128, in and out multiples of 4, no dy_mask_src) the call OVERWRITES `delta`
  * with dV = dz eps_a / (2 delta), which the two contractions of the backward consume; delta has no other use in
  * the backward, but a caller must not run the backward twice on the same forward buffers in that mode. */

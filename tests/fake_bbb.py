@@ -18,11 +18,11 @@ F_OUT_ZEROED, F_DX_PREACT, F_RELU_OUT = 256, 512, 1024
 
 
 def _arr(ptr, ctype, *shape):
+    n = int(np.prod(shape)) if shape else 1
+    if n == 0:                      # an empty tensor may carry a null pointer
+        return np.zeros(shape, dtype=np.dtype(ctype))
     if not ptr:
         return None
-    n = int(np.prod(shape)) if shape else 1
-    if n == 0:
-        return np.zeros(shape, dtype=np.dtype(ctype))
     return np.ctypeslib.as_array((ctype * n).from_address(ptr)).reshape(shape)
 
 
@@ -54,6 +54,8 @@ class FakeLib:
     # ---------------------------------------------------------------- weight sampling
     def bbb_linear_fwd(self, x, xs, wm, wr, bm, br, ew, eb, rng, prior, S, B, inn, out, flags, y, logp, logq, st):
         self.calls.append('linear_fwd')
+        if S == 0 or B == 0 or out == 0:       # an empty call launches nothing and touches no output (bbb.h)
+            return 0
         sample, lpq, relu = flags & F_SAMPLE, flags & F_LOGPROB, flags & F_RELU_IN
         assert not sample or (ew and eb), 'fake lib: inject eps (reference eps mode)'
         X = _f(x, S if xs else 1, B, inn).astype(np.float64)
@@ -125,6 +127,8 @@ class FakeLib:
                 if flags & F_DX_PREACT:      # x_pre: the stored input, pre- (with F_RELU_IN) or post-activation
                     d = d * (x_pre > 0)
                 DX[s] = d.astype(np.float32)
+        if flags & F_NO_WGRAD:                # the gradient buffers are not touched
+            return 0
         for ptr, shape, val in ((gwm, (out, inn), a_wm), (gwr, (out, inn), a_wr), (gbm, (out,), a_bm),
                                 (gbr, (out,), a_br)):
             G = _f(ptr, *shape)
@@ -153,6 +157,8 @@ class FakeLib:
     # ---------------------------------------------------------------- local reparameterisation
     def bbb_lr_linear_fwd(self, x, xs, wm, wr, bm, br, ea, eb, rng, sigma_p, S, B, inn, out, flags, y, delta, kl, st):
         self.calls.append('lr_fwd')
+        if S == 0 or B == 0 or out == 0:
+            return 0
         sample, calc, relu = flags & F_SAMPLE, flags & F_LOGPROB, flags & F_RELU_IN
         assert not sample or (ea and eb)
         X = _f(x, S if xs else 1, B, inn).astype(np.float64)
@@ -214,12 +220,13 @@ class FakeLib:
             if DX is not None:
                 v = dz @ WM.T + 2 * xs_ * (dV @ (sw * sw).T)
                 v = v * (osc if flags & F_SCALE_DX else 1.0)
-                if flags & F_DX_PREACT:
-                    assert relu
+                if flags & F_DX_PREACT:      # x_pre: the stored input, pre- (with F_RELU_IN) or post-activation
                     v = v * (x_pre > 0)
                 DX[s] = v.astype(np.float32)
         a_wr = CF.sigmoid(WR) * (2 * sw * acc_v + gk * (sw / sp2 - 1 / sw))
         a_br = CF.sigmoid(BR) * (acc_b + gk * (sb / sp2 - 1 / sb))
+        if flags & F_NO_WGRAD:
+            return 0
         for ptr, shape, val in ((gwm, (inn, out), a_wm), (gwr, (inn, out), a_wr), (gbm, (out,), a_bm),
                                 (gbr, (out,), a_br)):
             G = _f(ptr, *shape)
