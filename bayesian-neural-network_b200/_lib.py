@@ -10,7 +10,7 @@ LIB_PATH = os.environ.get('BBB_LIB') or os.path.join(_HERE, 'libbbb.so')   # BBB
 
 # flags (include/bbb.h)
 F_SAMPLE, F_LOGPROB, F_RELU_IN, F_ACCUM, F_TF32, F_NO_DX, F_SCALE_DX, F_NO_WGRAD = 1, 2, 4, 8, 16, 32, 64, 128
-F_OUT_ZEROED, F_DX_PREACT, F_RELU_OUT, F_ADAM_OVERLAP = 256, 512, 1024, 2048
+F_OUT_ZEROED, F_DX_PREACT, F_RELU_OUT = 256, 512, 1024
 PRIOR_GAUSSIAN, PRIOR_MIXTURE = 0, 1
 NLL_NONE, NLL_CE, NLL_GAUSS = 0, 1, 2
 
@@ -24,13 +24,6 @@ class Prior(C.Structure):
     _fields_ = [('kind', C.c_int32), ('pi', C.c_float), ('sigma1', C.c_float), ('sigma2', C.c_float)]
 
 
-class AdamFuse(C.Structure):
-    """struct bbb_adam_fuse: optimiser state of (w_mu, w_rho, b_mu, b_rho) + hyper-parameters"""
-    _fields_ = [('exp_avg', C.c_void_p * 4), ('exp_avg_sq', C.c_void_p * 4), ('lr', C.c_double),
-                ('beta1', C.c_double), ('beta2', C.c_double), ('eps', C.c_double), ('step', C.c_uint32),
-                ('step_dev', C.c_void_p), ('lr_scale_dev', C.c_void_p)]
-
-
 class PeerComm(C.Structure):
     """struct bbb_peer_comm: every rank's gradient bucket / parameter buffer / flag words as mapped in this process"""
     _fields_ = [('world', C.c_int32), ('rank', C.c_int32), ('grads', C.c_void_p * 8), ('params', C.c_void_p * 8),
@@ -42,7 +35,7 @@ class MlpLayer(C.Structure):
     """struct bbb_mlp_layer: one layer of a network-level call (bbb_mlp_fwd / bbb_mlp_bwd)"""
     _fields_ = [('w_mu', C.c_void_p), ('w_rho', C.c_void_p), ('b_mu', C.c_void_p), ('b_rho', C.c_void_p),
                 ('eps_w', C.c_void_p), ('eps_b', C.c_void_p), ('inn', C.c_int64), ('out', C.c_int64),
-                ('y', C.c_void_p), ('w_sample', C.c_void_p), ('dz', C.c_void_p),
+                ('y', C.c_void_p), ('dz', C.c_void_p),
                 ('g_w_mu', C.c_void_p), ('g_w_rho', C.c_void_p), ('g_b_mu', C.c_void_p), ('g_b_rho', C.c_void_p)]
 
 
@@ -54,8 +47,6 @@ _SIGS = {
     'bbb_linear_fwd': ([P, I64, P, P, P, P, P, P, P, P, I64, I64, I64, I64, I32, P, P, P, P], C.c_int),
     'bbb_linear_bwd': ([P, P, P, I64, P, P, P, P, P, P, P, P, I64, I64, I64, I64, I32, F32, F32, P, P, I64, P,
                         P, P, P, P, P, P], C.c_int),
-    'bbb_linear_bwd_adam': ([P, P, P, I64, P, P, P, P, P, P, P, P, I64, I64, I64, I64, I32, F32, F32, P, P, I64, P,
-                             P, P, P], C.c_int),
     'bbb_lr_linear_fwd': ([P, I64, P, P, P, P, P, P, P, F32, I64, I64, I64, I64, I32, P, P, P, P], C.c_int),
     'bbb_lr_linear_bwd': ([P, P, P, I64, P, P, P, P, P, P, P, P, F32, I64, I64, I64, I64, I32, F32, P, P,
                            P, P, P, P, P, P], C.c_int),
@@ -73,7 +64,7 @@ _SIGS = {
     'bbb_mlp_supported': ([P, I32, I64, I64, I32], C.c_int),
     'bbb_linear_fwd_relu_out_supported': ([I64, I64, I64, I32], C.c_int),
     'bbb_mlp_fwd': ([P, I32, P, I64, I64, P, P, I32, I32, P, F32, F32, P, P, P, P, F32, P, P, P, P], C.c_int),
-    'bbb_mlp_bwd': ([P, I32, P, I64, I64, P, P, I32, F32, F32, P, P, I64, P, P, P], C.c_int),
+    'bbb_mlp_bwd': ([P, I32, P, I64, I64, P, P, I32, F32, F32, P, P, I64, P, P], C.c_int),
     'bbb_elbo_finalize': ([P, P, P, P, I64, F32, P, P, P], C.c_int),
     'bbb_adam_step': ([I32, P, P, P, P, P, F64, F64, F64, F64, U32, P, P, P], C.c_int),
     'bbb_enable_peer_access': ([I32], C.c_int),

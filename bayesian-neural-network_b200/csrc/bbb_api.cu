@@ -44,8 +44,7 @@ extern "C" int bbb_linear_fwd(const float *x, int64_t x_sample_stride, const flo
                                   "(bbb_linear_fwd_relu_out_supported)");
   if (head_supported(a)) return launch_linear_fwd_head(a, st);                // out <= 16, both modes, exact fp32
   if ((flags & BBB_F_TF32) && linear_sk_supported(a)) return launch_linear_fwd_sk(a, st);
-  if (big)   // batch >= 384: TMA-fed, weight tiles shared in a cluster
-    return wide_disabled() ? launch_linear_fwd_big(a, st) : launch_linear_fwd_wide(a, st);
+  if (big) return launch_linear_fwd_wide(a, st);   // batch >= 384: TMA-fed, weight tiles shared in a cluster
   if ((flags & BBB_F_TF32) && linear_tc_supported(a)) return launch_linear_fwd_tc(a, st);
   if (linear_narrow_supported(a)) return launch_linear_fwd_narrow(a, st);   // exact-fp32 mode, out <= 16
   return launch_linear_fwd_fma(a, st);
@@ -60,16 +59,15 @@ extern "C" int bbb_linear_fwd_relu_out_supported(int64_t B, int64_t in, int64_t 
   return ((flags & BBB_F_TF32) && !head_supported(a) && !linear_sk_supported(a) && linear_big_fwd_supported(a)) ? 1 : 0;
 }
 
-namespace {
-int linear_bwd_impl(const float *dy, const float *dy_mask_src, const float *x, int64_t x_sample_stride,
-                    const float *w_mu, const float *w_rho, const float *b_mu, const float *b_rho,
-                    const float *eps_w, const float *eps_b, const bbb_rng *rng, const bbb_prior *prior,
-                    int64_t S, int64_t B, int64_t in, int64_t out, int32_t flags, float gp, float gq,
-                    const float *gp_dev, const float *gq_dev, int64_t g_dev_stride,
-                    const float *out_scale_dev, float *dx, float *grad_w_mu, float *grad_w_rho,
-                    float *grad_b_mu, float *grad_b_rho, const bbb_adam_fuse *adam, void *stream) {
+extern "C" int bbb_linear_bwd(const float *dy, const float *dy_mask_src, const float *x, int64_t x_sample_stride,
+                              const float *w_mu, const float *w_rho, const float *b_mu, const float *b_rho,
+                              const float *eps_w, const float *eps_b, const bbb_rng *rng, const bbb_prior *prior,
+                              int64_t S, int64_t B, int64_t in, int64_t out, int32_t flags, float gp, float gq,
+                              const float *gp_dev, const float *gq_dev, int64_t g_dev_stride,
+                              const float *out_scale_dev, float *dx, float *grad_w_mu, float *grad_w_rho,
+                              float *grad_b_mu, float *grad_b_rho, void *stream) {
   BBB_CHECK_ARG(w_mu && w_rho && b_mu && b_rho && ((dy && x) || S * B == 0), "null pointer");
-  BBB_CHECK_ARG((flags & BBB_F_NO_WGRAD) || adam || (grad_w_mu && grad_w_rho && grad_b_mu && grad_b_rho),
+  BBB_CHECK_ARG((flags & BBB_F_NO_WGRAD) || (grad_w_mu && grad_w_rho && grad_b_mu && grad_b_rho),
                 "null gradient pointer");
   BBB_CHECK_ARG((flags & BBB_F_NO_DX) || dx || S * B == 0, "dx required unless BBB_F_NO_DX");
   BBB_CHECK_ARG(S >= 0 && B >= 0 && in >= 0 && out >= 0 && S <= 65535, "bad shape");
@@ -93,28 +91,14 @@ int linear_bwd_impl(const float *dy, const float *dy_mask_src, const float *x, i
   a.vec_out = (out % 4 == 0) && all16({dy, dy_mask_src});
   if (S == 0 || B == 0) a.S = (B == 0) ? a.S : 0;  // degenerate: gradients reduce to the prior/posterior terms
   cudaStream_t st = (cudaStream_t)stream;
-  if (adam) {  // the optimiser step rides in the fused kernel's gradient epilogue, or the call is refused
-    if (!((flags & BBB_F_TF32) && a.S > 0 && linear_bwd_fused_supported(a)) || (flags & (BBB_F_ACCUM | BBB_F_NO_WGRAD)))
-      return fail(BBB_EUNSUPPORTED, "bbb_linear_bwd_adam: needs the fused tcgen05 backward (BBB_F_TF32, batch <= 128, "
-                                    "16-byte aligned rows) without BBB_F_ACCUM / BBB_F_NO_WGRAD");
-    for (int k = 0; k < 4; ++k) {
-      BBB_CHECK_ARG(adam->exp_avg[k] && adam->exp_avg_sq[k], "null optimiser state");
-      a.adam_m[k] = adam->exp_avg[k];
-      a.adam_v[k] = adam->exp_avg_sq[k];
-    }
-    BBB_CHECK_ARG(adam->step + (adam->step_dev ? 1u : 0u) >= 1u, "Adam step is 1-based");
-    a.adam_on = true;
-    a.adam_lr = adam->lr; a.adam_b1 = adam->beta1; a.adam_b2 = adam->beta2; a.adam_eps = (float)adam->eps;
-    a.adam_step = adam->step; a.adam_step_dev = adam->step_dev; a.adam_lr_scale_dev = adam->lr_scale_dev;
-  }
-  if (!adam && a.S > 0 && head_supported(a)) return launch_linear_bwd_head(a, st);   // out <= 16, both modes, exact fp32
+  if (a.S > 0 && head_supported(a)) return launch_linear_bwd_head(a, st);   // out <= 16, both modes, exact fp32
   if ((flags & BBB_F_TF32) && a.S > 0 && linear_bwd_fused_supported(a)) return launch_linear_bwd_fused(a, st);
   if ((flags & BBB_F_TF32) && linear_tc_supported(a)) {
-    // batch >= 384: batch-resident dgrad and the MN-major wgrad (bbb_linear_big.cu); anything they do not cover
-    // goes to the batch-tiled kernels
+    // batch >= 384: batch-resident dgrad (bbb_wide.cu) and the MN-major wgrad (bbb_linear_big.cu); anything they do
+    // not cover goes to the batch-tiled kernels
     LinArgs rest = a;
     if (a.S > 0 && !(flags & BBB_F_NO_DX) && linear_big_dgrad_supported(a)) {
-      if (int r = wide_disabled() ? launch_linear_dgrad_big(a, st) : launch_linear_dgrad_wide(a, st)) return r;
+      if (int r = launch_linear_dgrad_wide(a, st)) return r;
       rest.flags |= BBB_F_NO_DX;
     }
     if (a.S > 0 && !(flags & BBB_F_NO_WGRAD) && linear_big_wgrad_supported(a)) {
@@ -126,31 +110,6 @@ int linear_bwd_impl(const float *dy, const float *dy_mask_src, const float *x, i
   }
   if (a.S > 0 && linear_narrow_supported(a)) return launch_linear_bwd_narrow(a, st);   // exact-fp32 mode, out <= 16
   return launch_linear_bwd_fma(a, st);
-}
-}  // namespace
-
-extern "C" int bbb_linear_bwd(const float *dy, const float *dy_mask_src, const float *x, int64_t x_sample_stride,
-                              const float *w_mu, const float *w_rho, const float *b_mu, const float *b_rho,
-                              const float *eps_w, const float *eps_b, const bbb_rng *rng, const bbb_prior *prior,
-                              int64_t S, int64_t B, int64_t in, int64_t out, int32_t flags, float gp, float gq,
-                              const float *gp_dev, const float *gq_dev, int64_t g_dev_stride,
-                              const float *out_scale_dev, float *dx, float *grad_w_mu, float *grad_w_rho,
-                              float *grad_b_mu, float *grad_b_rho, void *stream) {
-  return linear_bwd_impl(dy, dy_mask_src, x, x_sample_stride, w_mu, w_rho, b_mu, b_rho, eps_w, eps_b, rng, prior, S, B, in,
-                         out, flags, gp, gq, gp_dev, gq_dev, g_dev_stride, out_scale_dev, dx, grad_w_mu, grad_w_rho,
-                         grad_b_mu, grad_b_rho, nullptr, stream);
-}
-
-extern "C" int bbb_linear_bwd_adam(const float *dy, const float *dy_mask_src, const float *x, int64_t x_sample_stride,
-                                   float *w_mu, float *w_rho, float *b_mu, float *b_rho, const float *eps_w,
-                                   const float *eps_b, const bbb_rng *rng, const bbb_prior *prior, int64_t S, int64_t B,
-                                   int64_t in, int64_t out, int32_t flags, float gp, float gq, const float *gp_dev,
-                                   const float *gq_dev, int64_t g_dev_stride, const float *out_scale_dev, float *dx,
-                                   const bbb_adam_fuse *adam, void *stream) {
-  BBB_CHECK_ARG(adam, "null optimiser descriptor");
-  return linear_bwd_impl(dy, dy_mask_src, x, x_sample_stride, w_mu, w_rho, b_mu, b_rho, eps_w, eps_b, rng, prior, S, B, in,
-                         out, flags, gp, gq, gp_dev, gq_dev, g_dev_stride, out_scale_dev, dx, nullptr, nullptr, nullptr,
-                         nullptr, adam, stream);
 }
 
 extern "C" int bbb_lr_linear_fwd(const float *x, int64_t x_sample_stride, const float *w_mu, const float *w_rho,

@@ -312,8 +312,7 @@ __device__ __forceinline__ float logsigma_quad_fast(const float sg[4]) {
 }
 
 // ---------------------------------------------------------------------------------------
-// Adam (torch.optim.Adam, no amsgrad, no weight decay).  Shared by the stand-alone multi-tensor kernel
-// (bbb_adam.cu) and by the fused backward, which can apply the update in its gradient epilogue.
+// Adam (torch.optim.Adam, no amsgrad, no weight decay): the update rule of the multi-tensor kernels (bbb_adam.cu).
 // ---------------------------------------------------------------------------------------
 struct AdamConst {
   float b1, b2, omb1, omb2, step_size, bc2_sqrt, eps;

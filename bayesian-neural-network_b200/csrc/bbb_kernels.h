@@ -24,14 +24,6 @@ struct LinArgs {
   int64_t g_dev_stride;
   const float *out_scale_dev;
   float *dx, *g_w_mu, *g_w_rho, *g_b_mu, *g_b_rho;
-  // optional optimiser step fused into the backward (bbb_linear_bwd_adam): state of w_mu, w_rho, b_mu, b_rho
-  bool adam_on;
-  float *adam_m[4], *adam_v[4];
-  double adam_lr, adam_b1, adam_b2;
-  float adam_eps;
-  uint32_t adam_step;
-  const uint32_t *adam_step_dev;
-  const float *adam_lr_scale_dev;
   // derived
   bool vec_in;   // in % 4 == 0 and every [*, in] base pointer 16-byte aligned
   bool vec_out;  // out % 4 == 0 and every [*, out] base pointer 16-byte aligned
@@ -72,17 +64,13 @@ bool linear_tc_supported(const LinArgs &a);
 int launch_linear_fwd_tc(const LinArgs &a, cudaStream_t st);
 int launch_linear_bwd_tc(const LinArgs &a, cudaStream_t st);
 
-// tcgen05 kind::tf32 forward / dgrad for large batches (bbb_linear_big.cu): the batch is the MMA's N dimension, a CTA's
-// accumulator [128 weight rows x 512 batch rows] fills TMEM, every sampled weight tile is used for 512 batch rows
+// tcgen05 kind::tf32 forward / dgrad for large batches (bbb_wide.cu): the batch is the MMA's N dimension, a CTA's
+// accumulator [128 weight rows x 512 batch rows] fills TMEM, activation tiles arrive by TMA and every sampled weight
+// tile is shared by the CTAs of a cluster.  Support conditions and wgrad in bbb_linear_big.cu.
 bool linear_big_fwd_supported(const LinArgs &a);
 bool linear_big_dgrad_supported(const LinArgs &a);
-int launch_linear_fwd_big(const LinArgs &a, cudaStream_t st);
-int launch_linear_dgrad_big(const LinArgs &a, cudaStream_t st);
-// second generation of the two (bbb_wide.cu): activation tiles by TMA, sampled weight tiles shared by the CTAs of a
-// cluster; same support conditions.  BBB_NO_WIDE=1 in the environment selects the first generation (A/B measurements).
 int launch_linear_fwd_wide(const LinArgs &a, cudaStream_t st);
 int launch_linear_dgrad_wide(const LinArgs &a, cudaStream_t st);
-bool wide_disabled();
 bool linear_big_wgrad_supported(const LinArgs &a);
 int launch_linear_wgrad_big(const LinArgs &a, cudaStream_t st);   // plain MN-major GEMM over the batch + sampling epilogue
 

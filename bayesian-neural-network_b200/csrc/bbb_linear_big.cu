@@ -1,27 +1,14 @@
 // Weight-sampling Bayesian linear layer on tcgen05 kind::tf32 for LARGE batches (BASELINE.json config 5: 4096-wide
-// layers, batch 4096): forward and dgrad.
+// layers, batch 4096): the weight gradient, and the support conditions of the large-batch path.  The forward and dgrad
+// of these shapes run in bbb_wide.cu (wide_kernel), behind the same conditions.
 //
-// At these sizes the contraction is dense (137 GFLOP per layer and sample) but every weight that enters it costs
-// ~100 CUDA-core instructions to sample (Philox + Box-Muller + softplus [+ log-densities]).  What decides the speed is
-// therefore how many batch rows a sampled weight tile is used for before it is thrown away.  bbb_linear_tc.cu gives a
-// CTA one 128-row batch tile, so W is re-sampled B / 128 = 32 times; here the operands are swapped so that the BATCH
-// is the MMA's N dimension and a CTA's accumulator fills all of TMEM:
-//
-//   D^T[m][b] (+)= A[m][k] * Bop[b][k]     M = 128 weight rows, N = 512 batch rows (two N = 256 MMAs), K = 32 / stage
-//     forward:  A = W_s[o][k]   sampled in registers, K-major SWIZZLE_128B      Bop = x_s[b][k]  (ReLU on load)
-//     dgrad:    A = W_s^T[i][o] sampled along i (coalesced), scattered K-major   Bop = dz_s[b][o]
-//
-// so a weight tile is sampled B / 512 = 8 times (4x less sampling work for the same MMAs), and the drain needs no
-// shared-memory transpose: TMEM hands a warp 32 consecutive weight rows of one batch column, which is a coalesced
-// 128-byte store into the row-major y[b][o] / dx[b][i].
-//   Warp-specialised: 16 producer warps stage the activation tile and sample the weight tile into a 2-stage ring
-//   (full / empty mbarriers), one warp issues the MMAs; 1 CTA per SM (160 KB of operands, 512 TMEM columns).
-//   Grid (weight-row tiles, batch tiles of 512, samples); batch tile 0 also accumulates the log-prob terms.
-// W never leaves the SM; eps is regenerated from the same Philox coordinates in the backward.
+// wgrad is a dense contraction over the batch, G_s[o][i] = sum_b dz_s[b][o] x_s[b][i], followed by an epilogue that
+// regenerates eps from the forward's Philox coordinates and folds in the prior and posterior terms; W never leaves the
+// SM.  Warp-specialised: 16 worker warps, one MMA-issuing warp and (TMA variant) one TMA warp; 1 CTA per SM (512 TMEM
+// columns).
 #include "bbb_tc_tiles.cuh"
 #include "bbb_tma.cuh"
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 
 namespace bbb {
@@ -33,214 +20,9 @@ using namespace tcx;
 constexpr int PW = 16;                    // producer warps
 constexpr int PT = PW * 32;               // producer threads
 constexpr int BT = PT + 32;               // + the MMA-issuing warp
-constexpr int NBT = 512;                  // batch rows per CTA tile = TMEM columns
-constexpr int NSTG = 2;
-constexpr int A_BYTES = BM * 128;         // [128 weight rows][32 k]
-constexpr int B_BYTES = NBT * 128;        // [512 batch rows][32 k]
-constexpr int STAGE = A_BYTES + B_BYTES;  // 80 KB
-constexpr int kBigDyn = NSTG * STAGE + 1024;
-
-struct BCtl {
-  uint64_t full[NSTG], empty[NSTG], acc;
-  uint32_t tmem_base;
-};
 
 __device__ __forceinline__ void mbar_arrive1(uint32_t bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-// 32 consecutive accumulator columns of this thread's TMEM lane
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float v[32]) {
-  uint32_t r[32];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr)
-      : "memory");
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
-
-// kDgrad = false: forward (A = W tile, rows = output features o, K = input features)
-// kDgrad = true : dgrad   (A = W^T tile, rows = input features i, K = output features)
-template <bool kDgrad, bool kLogProb>
-__global__ void __launch_bounds__(BT, 1) big_kernel(const LinArgs a_in) {
-  extern __shared__ uint8_t dsm[];
-  __shared__ BCtl ctl;
-  __shared__ float red[64];
-  LinArgs a = a_in;
-  uint8_t *tiles = align1024(dsm);
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const bool sample = a.flags & BBB_F_SAMPLE, relu = !kDgrad && (a.flags & BBB_F_RELU_IN);
-  const int s = blockIdx.z;
-  const int64_t m0 = (int64_t)blockIdx.x * BM, n0 = (int64_t)blockIdx.y * NBT;
-  const int64_t Mdim = kDgrad ? a.in : a.out, Kdim = kDgrad ? a.out : a.in;
-  const int nkb = (int)((Kdim + BK - 1) / BK);
-  const bool lpcta = kLogProb && blockIdx.y == 0;   // one batch tile per (weight tile, sample) owns the log-prob terms
-
-  // ---- setup: TMEM (all 512 columns), barriers ------------------------------------------------
-  if (warp == PW) tmem_alloc(smem_u32(&ctl.tmem_base), 512);
-  if (tid == 0) {
-#pragma unroll
-    for (int st = 0; st < NSTG; ++st) {
-      mbar_init(smem_u32(&ctl.full[st]), PW);
-      mbar_init(smem_u32(&ctl.empty[st]), 1);
-    }
-    mbar_init(smem_u32(&ctl.acc), 1);
-    mbar_fence_init();
-  }
-  tc_fence_before_sync();
-  __syncthreads();
-  tc_fence_after_sync();
-  const uint32_t tmem = ctl.tmem_base;
-  pdl_wait();
-  rng_resolve(a.rng);
-  float lp = 0.0f, lq = 0.0f;
-
-  if (warp == PW) {
-    // ---- MMA warp ---------------------------------------------------------------------------
-    if (lane == 0) {
-      // forward: both operands K-major; dgrad: A = W^T MN-major (see the producers), B = dz K-major
-      constexpr uint32_t idesc = kDgrad ? idesc_tf32_major(BM, 256, 1, 0) : idesc_tf32(BM, 256);
-      for (int kb = 0; kb < nkb; ++kb) {
-        const int st = kb % NSTG;
-        mbar_wait_parked(smem_u32(&ctl.full[st]), (uint32_t)((kb / NSTG) & 1));
-        tc_fence_after_sync();
-        const uint32_t As = smem_u32(tiles + st * STAGE), Bs = As + A_BYTES;
-        const uint64_t da = smem_desc_sw128(As);
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          const uint64_t db = smem_desc_sw128(Bs + h * 256 * 128);
-#pragma unroll
-          for (int kk = 0; kk < 4; ++kk)
-            mma_tf32(tmem + h * 256, kDgrad ? smem_desc_mn32(As + kk * 1024, 4096) : da + 2u * kk, db + 2u * kk, idesc,
-                     (kb == 0 && kk == 0) ? 0u : 1u);
-        }
-        mma_commit(smem_u32(&ctl.empty[st]));
-      }
-      mma_commit(smem_u32(&ctl.acc));
-    }
-    __syncwarp();
-  } else {
-    // ---- producers --------------------------------------------------------------------------
-    // activation tile: thread t stages rows t/8 + 64 j (j < 8), 16-byte chunk t%8; rows past the batch are clamped
-    // onto the last row (their accumulator columns are never stored)
-    const int prow = tid >> 3, chunk = tid & 7;
-    const uint32_t p_off = sw128_off(prow, chunk);       // rows r and r + 64 share (r & 7)
-    const float *act = kDgrad ? a.dy + (int64_t)s * a.B * a.out : a.x + (int64_t)s * a.x_sstride;
-    const float *arow[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      int64_t b = n0 + prow + 64 * j;
-      if (b > a.B - 1) b = a.B - 1;
-      arow[j] = act + b * Kdim + chunk * 4;
-    }
-    for (int kb = 0; kb < nkb; ++kb) {
-      const int st = kb % NSTG;
-      if (kb >= NSTG) mbar_wait(smem_u32(&ctl.empty[st]), (uint32_t)(((kb / NSTG) - 1) & 1));
-      uint8_t *As = tiles + st * STAGE, *Bs = As + A_BYTES;
-      const int64_t k0 = (int64_t)kb * BK;
-      const bool kc_ok = k0 + chunk * 4 < Kdim;
-      float4 xv[8];
-#pragma unroll
-      for (int j = 0; j < 8; ++j)
-        xv[j] = kc_ok ? __ldg(reinterpret_cast<const float4 *>(arow[j] + k0)) : make_float4(0.f, 0.f, 0.f, 0.f);
-      if (!kDgrad) {
-        // W tile [128 o rows][32 k]: thread t samples the quads (row t/8 + 64 j, chunk t%8), j < 2
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {
-          const int64_t o = m0 + prow + 64 * j;
-          float4 wv = make_float4(0.f, 0.f, 0.f, 0.f);
-          if (o < a.out && kc_ok) {
-            const int64_t e = o * a.in + k0 + chunk * 4;
-            Quad q;
-            load_quad(a, e, sample || lpcta, q);
-            float ep[4], w[4];
-            sample_quad(a, s, e, q, sample, ep, w);
-            wv = make_float4(to_tf32(w[0]), to_tf32(w[1]), to_tf32(w[2]), to_tf32(w[3]));
-            if (lpcta) {
-              lp += logp_quad_fast(a.prior, w);
-              lq += -4.0f * kHalfLog2Pi - logsigma_quad_fast(q.sg) -
-                    0.5f * (ep[0] * ep[0] + ep[1] * ep[1] + ep[2] * ep[2] + ep[3] * ep[3]);
-            }
-          }
-          *reinterpret_cast<float4 *>(As + p_off + j * 64 * 128) = wv;
-        }
-      } else {
-        // W^T tile as an MN-major operand: 4 regions of [32 o rows][128 B = 32 i] (SWIZZLE_128B_BASE32B), so a quad of
-        // 4 consecutive i of one weight row o is ONE 16-byte store and nothing is transposed.  Lane -> i quad (a warp
-        // reads 512 contiguous bytes of a weight row), warp w -> rows o = w and w + 16 of the k block.
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {
-          const int ol = warp + 16 * j;
-          const int64_t o = k0 + ol, i = m0 + 4 * lane;
-          float4 wv = make_float4(0.f, 0.f, 0.f, 0.f);
-          if (o < a.out && i < a.in) {
-            const int64_t e = o * a.in + i;
-            Quad q;
-            load_quad(a, e, sample, q);
-            float ep[4], w[4];
-            sample_quad(a, s, e, q, sample, ep, w);
-            wv = make_float4(to_tf32(w[0]), to_tf32(w[1]), to_tf32(w[2]), to_tf32(w[3]));
-          }
-          *reinterpret_cast<float4 *>(As + (lane >> 3) * 4096 + mn32_off(ol, lane & 7)) = wv;
-        }
-      }
-      // activations: fp32 as they are (the tensor core reads the upper 19 bits: TF32 by truncation)
-#pragma unroll
-      for (int j = 0; j < 8; ++j)
-        *reinterpret_cast<float4 *>(Bs + p_off + j * 64 * 128) = relu ? relu4(xv[j]) : xv[j];
-      fence_proxy_async_smem();
-      __syncwarp();
-      if (lane == 0) mbar_arrive1(smem_u32(&ctl.full[st]));
-    }
-
-    // ---- drain: warp w reads TMEM lanes 32 (w % 4) .. +31 (weight rows) and columns 128 (w / 4) .. +127 (batch) ----
-    mbar_wait_parked(smem_u32(&ctl.acc), 0);
-    tc_fence_after_sync();
-    const int q4 = warp & 3, cq = warp >> 2;
-    const int64_t m = m0 + q4 * 32 + lane;
-    const bool m_ok = m < Mdim;
-    float bias = 0.0f;
-    if (!kDgrad && m_ok) {
-      float sg, ep;
-      bias_elem(a, s, m, sample, lpcta, bias, sg, ep);
-      if (lpcta && cq == 0) { lp += logp_elem(a.prior, bias); lq += logq_elem(sg, ep); }
-    }
-    const float osc = (kDgrad && (a.flags & BBB_F_SCALE_DX) && a.out_scale_dev) ? __ldg(a.out_scale_dev) : 1.0f;
-    const bool preact = kDgrad && (a.flags & BBB_F_DX_PREACT), relu_out = !kDgrad && (a.flags & BBB_F_RELU_OUT);
-    float *dst = kDgrad ? a.dx + (int64_t)s * a.B * a.in : a.y + (int64_t)s * a.B * a.out;
-    const float *msk = preact ? a.x + (int64_t)s * a.x_sstride : nullptr;
-#pragma unroll 1
-    for (int c0 = 0; c0 < 128; c0 += 32) {
-      const int col = cq * 128 + c0;
-      if (n0 + col >= a.B) break;                 // warp-uniform: the rest of this warp's columns are past the batch
-      float v[32];
-      tmem_ld32(tmem + ((uint32_t)(q4 * 32) << 16) + (uint32_t)col, v);
-      if (m_ok) {
-#pragma unroll
-        for (int j = 0; j < 32; ++j) {
-          const int64_t b = n0 + col + j;
-          if (b < a.B) {
-            float r = kDgrad ? osc * v[j] : v[j] + bias;
-            if (relu_out) r = fmaxf(r, 0.0f);
-            if (preact && !(__ldg(msk + b * Mdim + m) > 0.0f)) r = 0.0f;
-            dst[b * Mdim + m] = r;
-          }
-        }
-      }
-    }
-    tc_fence_before_sync();
-  }
-  pdl_launch_dependents();
-  if (kLogProb) block_sum2_atomic(lp, lq, red, a.logp + s, a.logq + s);
-  tc_fence_before_sync();
-  __syncthreads();
-  if (warp == PW) tmem_dealloc(tmem, 512);
 }
 
 // ==================================================================================================
@@ -271,19 +53,6 @@ struct WCtl {
 struct WgradPart {
   float *w_mu, *w_rho, *b_mu, *b_rho;
 };
-
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float v[16]) {
-  uint32_t r[16];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr)
-      : "memory");
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
-}
 
 // kTma: the slabs are loaded by TMA (one extra warp; grouped 4-D maps, bbb_tma.cuh: one box = the 4 dz regions, one =
 // the 8 x regions of a stage, already in the MN-major layout), which streams them from L2 several times faster than
@@ -610,15 +379,6 @@ big_wgrad_kernel(const __grid_constant__ CUtensorMap tm_dz, const __grid_constan
 
 inline int cdiv_i(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
 
-template <bool kDgrad, bool kLogProb>
-int launch_big(const LinArgs &a, cudaStream_t st) {
-  BBB_CHECK_CUDA(cudaFuncSetAttribute(big_kernel<kDgrad, kLogProb>, cudaFuncAttributeMaxDynamicSharedMemorySize, kBigDyn));
-  dim3 grid(cdiv_i(kDgrad ? a.in : a.out, BM), cdiv_i(a.B, NBT), (unsigned)a.S);
-  BBB_CHECK_CUDA(launch_pdl(big_kernel<kDgrad, kLogProb>, grid, dim3(BT), kBigDyn, st, a));
-  BBB_CHECK_LAUNCH();
-  return BBB_OK;
-}
-
 }  // namespace
 
 // Batches of at least 384 rows (3/4 of one 512-row tile) with 16-byte aligned rows; the weight matrix must be wide
@@ -631,15 +391,9 @@ bool linear_big_dgrad_supported(const LinArgs &a) {
   return a.vec_in && a.vec_out && a.B >= 384 && a.out >= 32 && a.in >= 32 && a.S >= 1 && !a.mask;
 }
 
-int launch_linear_fwd_big(const LinArgs &a, cudaStream_t st) {
-  if (a.flags & BBB_F_LOGPROB) return launch_big<false, true>(a, st);
-  return launch_big<false, false>(a, st);
-}
-int launch_linear_dgrad_big(const LinArgs &a, cudaStream_t st) { return launch_big<true, false>(a, st); }
-
 // wgrad: rows of dz and x must be 16-byte multiples (slab copies), no dy mask
 bool linear_big_wgrad_supported(const LinArgs &a) {
-  return a.vec_in && a.vec_out && a.B >= 384 && a.out >= 32 && a.in >= 32 && a.S >= 1 && !a.mask && !a.adam_on;
+  return a.vec_in && a.vec_out && a.B >= 384 && a.out >= 32 && a.in >= 32 && a.S >= 1 && !a.mask;
 }
 namespace {
 // g += p for the four gradient tensors (float4 where the weight matrices allow it: in % 4 == 0 on this path)

@@ -321,14 +321,8 @@ __global__ void __launch_bounds__(FT, 1) bwd_fused_kernel(const LinArgs a_in, in
   }
 
   pdl_launch_dependents();   // the sample loop is done: let the next kernel of the chain become resident
-  // ---- parameter gradients, or (bbb_linear_bwd_adam) the Adam update of this CTA's own weights in place ------------
+  // ---- parameter gradients ----------------------------------------------------------------------------------------
   if (wgrad) {
-    __shared__ AdamConst adam_c;
-    if (a.adam_on) {
-      if (tid == 0)
-        adam_c = adam_consts(a.adam_lr, a.adam_b1, a.adam_b2, a.adam_eps, a.adam_step, a.adam_step_dev, a.adam_lr_scale_dev);
-      __syncthreads();
-    }
 #pragma unroll
     for (int j = 0; j < QMAX; ++j) {
       const int q = tid + FT * j;
@@ -338,44 +332,17 @@ __global__ void __launch_bounds__(FT, 1) bwd_fused_kernel(const LinArgs a_in, in
         float g1[4], g2[4];
 #pragma unroll
         for (int c = 0; c < 4; ++c) { g1[c] = osc * gm[j][c]; g2[c] = osc * gr[j][c]; }
-        if (a.adam_on) {
-          // every weight belongs to exactly one CTA, which is also its only reader in this kernel
-          float *pp[2] = {const_cast<float *>(a.w_mu) + e, const_cast<float *>(a.w_rho) + e};
-#pragma unroll
-          for (int k = 0; k < 2; ++k) {
-            float4 P = *reinterpret_cast<float4 *>(pp[k]);
-            float4 M = *reinterpret_cast<float4 *>(a.adam_m[k] + e), V = *reinterpret_cast<float4 *>(a.adam_v[k] + e);
-            const float *g = k ? g2 : g1;
-            adam1(P.x, g[0], M.x, V.x, adam_c);
-            adam1(P.y, g[1], M.y, V.y, adam_c);
-            adam1(P.z, g[2], M.z, V.z, adam_c);
-            adam1(P.w, g[3], M.w, V.w, adam_c);
-            *reinterpret_cast<float4 *>(pp[k]) = P;
-            *reinterpret_cast<float4 *>(a.adam_m[k] + e) = M;
-            *reinterpret_cast<float4 *>(a.adam_v[k] + e) = V;
-          }
-        } else {
-          float4 *pm = reinterpret_cast<float4 *>(a.g_w_mu + e), *pr = reinterpret_cast<float4 *>(a.g_w_rho + e);
-          float4 om = make_float4(0.f, 0.f, 0.f, 0.f), orr = om;
-          if (accum) { om = *pm; orr = *pr; }
-          *pm = make_float4(g1[0] + om.x, g1[1] + om.y, g1[2] + om.z, g1[3] + om.w);
-          *pr = make_float4(g2[0] + orr.x, g2[1] + orr.y, g2[2] + orr.z, g2[3] + orr.w);
-        }
+        float4 *pm = reinterpret_cast<float4 *>(a.g_w_mu + e), *pr = reinterpret_cast<float4 *>(a.g_w_rho + e);
+        float4 om = make_float4(0.f, 0.f, 0.f, 0.f), orr = om;
+        if (accum) { om = *pm; orr = *pr; }
+        *pm = make_float4(g1[0] + om.x, g1[1] + om.y, g1[2] + om.z, g1[3] + om.w);
+        *pr = make_float4(g2[0] + orr.x, g2[1] + orr.y, g2[2] + orr.z, g2[3] + orr.w);
       }
     }
     if (bias_cta && tid < rows) {
       const int64_t o = o_t0 + tid;
-      if (a.adam_on) {
-        float P = a.b_mu[o], M = a.adam_m[2][o], V = a.adam_v[2][o];
-        adam1(P, osc * gbm, M, V, adam_c);
-        const_cast<float *>(a.b_mu)[o] = P; a.adam_m[2][o] = M; a.adam_v[2][o] = V;
-        P = a.b_rho[o]; M = a.adam_m[3][o]; V = a.adam_v[3][o];
-        adam1(P, osc * gbr, M, V, adam_c);
-        const_cast<float *>(a.b_rho)[o] = P; a.adam_m[3][o] = M; a.adam_v[3][o] = V;
-      } else {
-        a.g_b_mu[o] = accum ? fmaf(osc, gbm, a.g_b_mu[o]) : osc * gbm;
-        a.g_b_rho[o] = accum ? fmaf(osc, gbr, a.g_b_rho[o]) : osc * gbr;
-      }
+      a.g_b_mu[o] = accum ? fmaf(osc, gbm, a.g_b_mu[o]) : osc * gbm;
+      a.g_b_rho[o] = accum ? fmaf(osc, gbr, a.g_b_rho[o]) : osc * gbr;
     }
   }
   tc_fence_before_sync();

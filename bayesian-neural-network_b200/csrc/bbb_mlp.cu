@@ -136,7 +136,7 @@ MlpLayerDesc make_desc(const bbb_mlp_layer &L, const float *x, bool x_shared) {
   d.x = x; d.x_shared = x_shared;
   d.w_mu = L.w_mu; d.w_rho = L.w_rho; d.b_mu = L.b_mu; d.b_rho = L.b_rho; d.eps_w = L.eps_w; d.eps_b = L.eps_b;
   d.in = L.in; d.out = L.out;
-  d.y = L.y; d.w_sample = L.w_sample;
+  d.y = L.y;
   d.dz = L.dz; d.g_w_mu = L.g_w_mu; d.g_w_rho = L.g_w_rho; d.g_b_mu = L.g_b_mu; d.g_b_rho = L.g_b_rho;
   return d;
 }
@@ -193,63 +193,16 @@ extern "C" int bbb_mlp_fwd(const bbb_mlp_layer *layers, int32_t n_layers, const 
   r.layer = (uint32_t)(n_layers - 1);
   const int32_t head_flags = (flags & (BBB_F_SAMPLE | BBB_F_LOGPROB)) | BBB_F_RELU_IN;    // its input is a pre-activation
   ScopedTimer tm("head_fwd[%lldx%lld]", (long long)H.in, (long long)H.out, st);
-  if (H.w_sample && head2_supported(S, B, H.in, H.out) && (!out4 || done_counter)) {
-    BBB_CHECK_ARG(nll_kind == BBB_NLL_NONE || nll_kind == BBB_NLL_CE || nll_kind == BBB_NLL_GAUSS, "bad nll_kind");
-    BBB_CHECK_ARG(nll_kind == BBB_NLL_NONE || (target && nll), "target and nll accumulator required");
-    BBB_CHECK_ARG(nll_kind != BBB_NLL_GAUSS || sigma > 0, "sigma must be positive");
-    BBB_CHECK_ARG(done_counter, "the full-grid head needs done_counter (two zeroed words)");
-    MlpLayerDesc d = make_desc(H, inp, false);
-    return launch_head2_fwd(d, S, B, make_rng_dev(rng ? &r : nullptr), pd, head_flags, nll_kind, target, sigma, grad_scale,
-                            d_out, logp, logq, nll, beta, beta_dev, out4, done_counter, st);
-  }
   return bbb_head_fwd(inp, B * H.in, H.w_mu, H.w_rho, H.b_mu, H.b_rho, H.eps_w, H.eps_b, rng ? &r : nullptr, prior, S, B,
                       H.in, H.out, head_flags, nll_kind, target, sigma, grad_scale, H.y, d_out, logp, logq, nll, beta,
                       beta_dev, out4, done_counter, stream);
 }
 
-namespace {
-// Side stream of the overlapped optimiser (BBB_F_ADAM_OVERLAP), one per device, with a small ring of events for the
-// fork / join edges.  An event may be re-recorded by the next call: a wait binds to the record that preceded it.
-struct SideStream {
-  cudaStream_t stream = nullptr;
-  cudaEvent_t ev[8] = {};
-  int next = 0;
-};
-int side_stream(SideStream **out) {
-  static SideStream side[64];
-  int dev = 0;
-  BBB_CHECK_CUDA(cudaGetDevice(&dev));
-  if (dev < 0 || dev >= 64) return fail(BBB_ECUDA, "device index out of range");
-  SideStream &s = side[dev];
-  if (!s.stream) {
-    BBB_CHECK_CUDA(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
-    for (auto &e : s.ev) BBB_CHECK_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-  }
-  *out = &s;
-  return BBB_OK;
-}
-// layer `L`'s Adam update on the side stream, after everything issued so far on `main`
-int adam_on_side(SideStream &side, cudaStream_t main, const bbb_mlp_layer &L, const bbb_adam_fuse &A) {
-  cudaEvent_t e = side.ev[side.next++ & 7];
-  BBB_CHECK_CUDA(cudaEventRecord(e, main));
-  BBB_CHECK_CUDA(cudaStreamWaitEvent(side.stream, e, 0));
-  float *params[4] = {const_cast<float *>(L.w_mu), const_cast<float *>(L.w_rho), const_cast<float *>(L.b_mu), const_cast<float *>(L.b_rho)};
-  const float *grads[4] = {L.g_w_mu, L.g_w_rho, L.g_b_mu, L.g_b_rho};
-  const int64_t sizes[4] = {L.in * L.out, L.in * L.out, L.out, L.out};
-  return bbb_adam_step(4, params, grads, A.exp_avg, A.exp_avg_sq, sizes, A.lr, A.beta1, A.beta2, A.eps, A.step, A.step_dev,
-                       A.lr_scale_dev, side.stream);
-}
-}  // namespace
-
 extern "C" int bbb_mlp_bwd(const bbb_mlp_layer *layers, int32_t n_layers, const float *x, int64_t S, int64_t B,
                            const bbb_rng *rng, const bbb_prior *prior, int32_t flags, float gp, float gq,
                            const float *gp_dev, const float *gq_dev, int64_t g_dev_stride, const float *out_scale_dev,
-                           const bbb_adam_fuse *adam, void *stream) {
+                           void *stream) {
   BBB_CHECK_ARG(layers && x && n_layers >= 2 && n_layers <= 64, "null pointer or bad layer count");
-  const bool overlap = adam && (flags & BBB_F_ADAM_OVERLAP);
-  if (overlap && (flags & BBB_F_ACCUM)) return fail(BBB_EUNSUPPORTED, "bbb_mlp_bwd: BBB_F_ADAM_OVERLAP with BBB_F_ACCUM");
-  if (adam && !overlap && (S > 2 || (flags & BBB_F_ACCUM)))
-    return fail(BBB_EUNSUPPORTED, "bbb_mlp_bwd: the fused optimiser needs S <= 2 (one sample group) and no BBB_F_ACCUM");
   BBB_CHECK_ARG(flags & BBB_F_TF32, "the network-level kernels are the tcgen05 kind::tf32 path: pass BBB_F_TF32");
   BBB_CHECK_ARG(g_dev_stride == 0 || g_dev_stride == 1, "g_dev_stride must be 0 or 1");
   BBB_CHECK_ARG(((gp == 0.0f) && !gp_dev) || prior, "prior required when gp != 0");
@@ -259,11 +212,7 @@ extern "C" int bbb_mlp_bwd(const bbb_mlp_layer *layers, int32_t n_layers, const 
   for (int l = 0; l < n_layers; ++l) {
     const bbb_mlp_layer &L = layers[l];
     BBB_CHECK_ARG(L.w_mu && L.w_rho && L.b_mu && L.b_rho && L.dz, "null layer pointer");
-    // (with the fused optimiser only the head still writes its gradients: its update is a separate small launch)
-    BBB_CHECK_ARG((adam && !overlap && l + 1 < n_layers) || (L.g_w_mu && L.g_w_rho && L.g_b_mu && L.g_b_rho),
-                  "null gradient pointer");
-    if (adam)
-      for (int k = 0; k < 4; ++k) BBB_CHECK_ARG(adam[l].exp_avg[k] && adam[l].exp_avg_sq[k], "null optimiser state");
+    BBB_CHECK_ARG(L.g_w_mu && L.g_w_rho && L.g_b_mu && L.g_b_rho, "null gradient pointer");
     BBB_CHECK_ARG(!sample || (L.eps_w && L.eps_b) || (!L.eps_w && !L.eps_b && rng), "give both eps pointers or an rng");
     BBB_CHECK_ARG(L.in == dims[l], "layer widths do not chain");
     BBB_CHECK_ARG(l + 1 == n_layers || L.y, "hidden layers need their stored pre-activation");
@@ -282,22 +231,11 @@ extern "C" int bbb_mlp_bwd(const bbb_mlp_layer *layers, int32_t n_layers, const 
     bbb_rng r = rng ? *rng : bbb_rng{};
     r.layer = (uint32_t)(n_layers - 1);
     ScopedTimer tm("head_bwd[%lldx%lld]", (long long)H.in, (long long)H.out, st);
-    if (H.w_sample && head2_supported(S, B, H.in, H.out)) {
-      MlpLayerDesc d = make_desc(H, P.y, false);
-      d.dx = P.dz;
-      if (int rc = launch_head2_bwd(d, S, B, make_rng_dev(rng ? &r : nullptr), pd, keep | BBB_F_RELU_IN, gp, gq, gp_dev, gq_dev,
-                                    (int)g_dev_stride, out_scale_dev, st))
-        return rc;
-    } else if (int rc = bbb_linear_bwd(H.dz, nullptr, P.y, B * H.in, H.w_mu, H.w_rho, H.b_mu, H.b_rho, H.eps_w, H.eps_b,
+    if (int rc = bbb_linear_bwd(H.dz, nullptr, P.y, B * H.in, H.w_mu, H.w_rho, H.b_mu, H.b_rho, H.eps_w, H.eps_b,
                                 rng ? &r : nullptr, prior, S, B, H.in, H.out,
                                 keep | BBB_F_RELU_IN | BBB_F_DX_PREACT | BBB_F_OUT_ZEROED, gp, gq, gp_dev, gq_dev,
                                 g_dev_stride, out_scale_dev, P.dz, H.g_w_mu, H.g_w_rho, H.g_b_mu, H.g_b_rho, stream))
       return rc;
-  }
-  SideStream *side = nullptr;
-  if (overlap) {
-    if (int rc = side_stream(&side)) return rc;
-    if (int rc = adam_on_side(*side, st, layers[n_layers - 1], adam[n_layers - 1])) return rc;
   }
   for (int l = n_layers - 2; l >= 0; --l) {
     bbb_rng r = rng ? *rng : bbb_rng{};
@@ -308,26 +246,8 @@ extern "C" int bbb_mlp_bwd(const bbb_mlp_layer *layers, int32_t n_layers, const 
       return fail(BBB_EUNSUPPORTED, "bbb_mlp_bwd: layer %d needs 16-byte aligned tensors", l);
     ScopedTimer tm("mlp_bwd[%lldx%lld]", (long long)d.in, (long long)d.out, st);
     if (int rc = launch_mlp_bwd_layer(d, S, B, make_rng_dev(rng ? &r : nullptr), pd, keep | (l > 0 ? BBB_F_RELU_IN : 0), gp, gq, gp_dev, gq_dev,
-                                      (int)g_dev_stride, out_scale_dev, (adam && !overlap) ? &adam[l] : nullptr, st))
+                                      (int)g_dev_stride, out_scale_dev, st))
       return rc;
-    if (overlap)
-      if (int rc = adam_on_side(*side, st, layers[l], adam[l])) return rc;
-  }
-  if (overlap) {   // join: everything after this call on `stream` sees the updated parameters
-    cudaEvent_t e = side->ev[side->next++ & 7];
-    BBB_CHECK_CUDA(cudaEventRecord(e, side->stream));
-    BBB_CHECK_CUDA(cudaStreamWaitEvent(st, e, 0));
-    return BBB_OK;
-  }
-  if (adam) {      // the head's few thousand parameters: the stand-alone multi-tensor update on the gradients it wrote
-    const bbb_mlp_layer &H = layers[n_layers - 1];
-    const bbb_adam_fuse &A = adam[n_layers - 1];
-    float *params[4] = {const_cast<float *>(H.w_mu), const_cast<float *>(H.w_rho), const_cast<float *>(H.b_mu), const_cast<float *>(H.b_rho)};
-    const float *grads[4] = {H.g_w_mu, H.g_w_rho, H.g_b_mu, H.g_b_rho};
-    const int64_t sizes[4] = {H.in * H.out, H.in * H.out, H.out, H.out};
-    ScopedTimer tm("head_adam[%lldx%lld]", (long long)H.in, (long long)H.out, st);
-    return bbb_adam_step(4, params, grads, A.exp_avg, A.exp_avg_sq, sizes, A.lr, A.beta1, A.beta2, A.eps, A.step, A.step_dev,
-                         A.lr_scale_dev, stream);
   }
   return BBB_OK;
 }

@@ -12,7 +12,6 @@ struct MlpLayerDesc {
   const float *w_mu, *w_rho, *b_mu, *b_rho, *eps_w, *eps_b;
   int64_t in, out;
   float *y;                  // [S,B,out] zero-filled: the pre-activation output, split-K partial tiles are reduce-added into it
-  float *w_sample;           // head only: [S,out,in] + [S,16] scratch for the sampled weights / biases (bbb_head2.cu)
   // backward
   const float *dz;           // [S,B,out] gradient w.r.t. the layer's pre-activation output
   float *dx;                 // [S,B,in] zero-filled: gradient w.r.t. the pre-activation input (masked by x > 0), or NULL
@@ -46,14 +45,6 @@ struct MlpBwdArgs {
   const float *gp_dev, *gq_dev, *out_scale_dev;   // ... times optional device scalars (bbb_linear_bwd semantics)
   int g_dev_stride;
   unsigned long long *timeline;   // debug: 16 globaltimer stamps per CTA, or NULL
-  // optional optimiser step fused into the gradient write-back (bbb_mlp_bwd with an Adam descriptor, S <= 2): state of
-  // w_mu, w_rho, b_mu, b_rho; the parameters are updated in place and no gradient is written
-  float *adam_m[4], *adam_v[4];
-  double adam_lr, adam_b1, adam_b2;
-  float adam_eps;
-  uint32_t adam_step;
-  const uint32_t *adam_step_dev;
-  const float *adam_lr_scale_dev;
 };
 
 // debug: phase time stamps of the network-level kernels (tools/kernel_timeline.py)
@@ -68,23 +59,12 @@ __device__ __forceinline__ void stamp(unsigned long long *tl, int slot) {
   }
 }
 
-// the head (last layer, out <= 16) on a full grid: bbb_head2.cu
-bool head2_supported(int64_t S, int64_t B, int64_t in, int64_t out);
-int64_t head2_scratch_floats(int64_t S, int64_t in, int64_t out);
-int launch_head2_fwd(const MlpLayerDesc &l, int64_t S, int64_t B, const RngDev &rng, const PriorDev &prior, int flags,
-                     int nll_kind, const void *target, float sigma, float grad_scale, float *d_out, double *logp,
-                     double *logq, double *nll, float beta, const float *beta_dev, float *out4, uint32_t *done,
-                     cudaStream_t st);
-int launch_head2_bwd(const MlpLayerDesc &l, int64_t S, int64_t B, const RngDev &rng, const PriorDev &prior, int flags,
-                     float gp, float gq, const float *gp_dev, const float *gq_dev, int g_dev_stride,
-                     const float *out_scale_dev, cudaStream_t st);
-
 bool mlp_fwd_layer_supported(const MlpLayerDesc &l, int64_t S, int64_t B);
 int launch_mlp_fwd_layer(const MlpLayerDesc &l, int64_t S, int64_t B, const RngDev &rng, const PriorDev &prior, int flags,
                          double *logp, double *logq, cudaStream_t st);
 bool mlp_bwd_layer_supported(const MlpLayerDesc &l, int64_t S, int64_t B);
 int launch_mlp_bwd_layer(const MlpLayerDesc &l, int64_t S, int64_t B, const RngDev &rng, const PriorDev &prior, int flags,
                          float gp, float gq, const float *gp_dev, const float *gq_dev, int g_dev_stride,
-                         const float *out_scale_dev, const bbb_adam_fuse *adam, cudaStream_t st);
+                         const float *out_scale_dev, cudaStream_t st);
 
 }  // namespace bbb

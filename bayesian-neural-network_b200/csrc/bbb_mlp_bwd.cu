@@ -67,8 +67,8 @@ __device__ __forceinline__ void sts128(uint32_t addr, float a, float b, float c,
 // quarter-warp-per-row reader
 __device__ __forceinline__ uint32_t stg_off(int row, int c16) { return (uint32_t)((row << 7) + ((c16 ^ (row & 7)) << 4)); }
 
-// MODE 0: eps from Philox, 1: eps injected from memory, 2: w = mu;  kAdam: the optimiser's update replaces the gradient write
-template <int XWR, int MODE, bool kDx, bool kAdam>
+// MODE 0: eps from Philox, 1: eps injected from memory, 2: w = mu
+template <int XWR, int MODE, bool kDx>
 __global__ void __launch_bounds__(kThreadsB, 1)
 ws_bwd_kernel(const __grid_constant__ CUtensorMap tm_mu, const __grid_constant__ CUtensorMap tm_rho,
               const __grid_constant__ CUtensorMap tm_dz, const __grid_constant__ CUtensorMap tm_x,
@@ -78,7 +78,6 @@ ws_bwd_kernel(const __grid_constant__ CUtensorMap tm_mu, const __grid_constant__
   extern __shared__ uint8_t dsm[];
   __shared__ BwdCtl ctl;
   __shared__ float csum[2][128];
-  __shared__ AdamConst adam_c;
   const uint32_t base = (smem_u32(dsm) + 1023u) & ~1023u;
   const uint32_t w_s[2] = {base, base + Cfg::kW};        // weight-tile slots (mu / rho land here)
   const uint32_t area = base + 2 * Cfg::kW;              // MMA1 ring, later dz K-major (4 REG) + staging (2 REG)
@@ -97,8 +96,6 @@ ws_bwd_kernel(const __grid_constant__ CUtensorMap tm_mu, const __grid_constant__
   const bool bias_cta = blockIdx.x == 0;
 
   if (wid == 1) tmem_alloc(smem_u32(&ctl.tmem_base), 512);
-  if (kAdam && tid == 96)
-    adam_c = adam_consts(a.adam_lr, a.adam_b1, a.adam_b2, a.adam_eps, a.adam_step, a.adam_step_dev, a.adam_lr_scale_dev);
   if (tid == 0) {
     mbar_init(smem_u32(&ctl.murho_full), 1);
     for (int i = 0; i < NRING; ++i) {
@@ -296,19 +293,9 @@ ws_bwd_kernel(const __grid_constant__ CUtensorMap tm_mu, const __grid_constant__
             gbm += t;
             gbr += -expm1f(-bsg) * (t * ep - gqs[s] / bsg);
           }
-          if (kAdam) {       // (one sample group only: the gradient is complete)
-            const float ibc = 1.0f / adam_c.bc2_sqrt;
-            float P = bmu, M = a.adam_m[2][o], V = a.adam_v[2][o];
-            adam1_fast(P, osc * gbm, M, V, adam_c, ibc);
-            const_cast<float *>(a.b_mu)[o] = P; a.adam_m[2][o] = M; a.adam_v[2][o] = V;
-            P = brho; M = a.adam_m[3][o]; V = a.adam_v[3][o];
-            adam1_fast(P, osc * gbr, M, V, adam_c, ibc);
-            const_cast<float *>(a.b_rho)[o] = P; a.adam_m[3][o] = M; a.adam_v[3][o] = V;
-          } else {
-            const bool acc_b = accum_flag || g > 0;
-            a.g_b_mu[o] = acc_b ? fmaf(osc, gbm, a.g_b_mu[o]) : osc * gbm;
-            a.g_b_rho[o] = acc_b ? fmaf(osc, gbr, a.g_b_rho[o]) : osc * gbr;
-          }
+          const bool acc_b = accum_flag || g > 0;
+          a.g_b_mu[o] = acc_b ? fmaf(osc, gbm, a.g_b_mu[o]) : osc * gbm;
+          a.g_b_rho[o] = acc_b ? fmaf(osc, gbr, a.g_b_rho[o]) : osc * gbr;
         }
       }
       // ---- the block's weights, region by region (32 columns): two adjacent quads per thread ----------------------------
@@ -366,62 +353,25 @@ ws_bwd_kernel(const __grid_constant__ CUtensorMap tm_mu, const __grid_constant__
           __syncwarp();
           if (lane == 0) mbar_arrive_l(smem_u32(&ctl.w_full));
         }
-        // coalesced write-back of the region: a quarter warp per row.  With the fused optimiser the parameter and its
-        // Adam state are requested BEFORE the barrier (the sampling registers are dead by now), so their latency hides
-        // behind it; the update replaces the gradient store.
+        // coalesced write-back of the region: a quarter warp per row
+        bar_epi();
         {
           const int qd = 8 * r + c_chk;
-          const bool own = qd < tq;
-          float4 P[2][2], Mv[2][2], Vv[2][2];
-          if (kAdam && own) {
-#pragma unroll
-            for (int hh = 0; hh < 2; ++hh) {
-              const int rr = c_row + 64 * hh;
-              if (rr < rows) {
-                const int64_t e = (int64_t)(o_t0 + rr) * a.in + i_lo + 4 * qd;
-                P[hh][0] = *reinterpret_cast<const float4 *>(a.w_mu + e);
-                P[hh][1] = *reinterpret_cast<const float4 *>(a.w_rho + e);
-                Mv[hh][0] = *reinterpret_cast<const float4 *>(a.adam_m[0] + e);
-                Mv[hh][1] = *reinterpret_cast<const float4 *>(a.adam_m[1] + e);
-                Vv[hh][0] = *reinterpret_cast<const float4 *>(a.adam_v[0] + e);
-                Vv[hh][1] = *reinterpret_cast<const float4 *>(a.adam_v[1] + e);
-              }
-            }
-          }
-          bar_epi();
-          if (own) {
+          if (qd < tq) {
 #pragma unroll
             for (int hh = 0; hh < 2; ++hh) {
               const int rr = c_row + 64 * hh;
               if (rr < rows) {
                 const int64_t e = (int64_t)(o_t0 + rr) * a.in + i_lo + 4 * qd;
                 float4 vm = lds128(stg + stg_off(rr, c_chk)), vr = lds128(stg + REG + stg_off(rr, c_chk));
-                if (kAdam) {
-                  const float ibc = 1.0f / adam_c.bc2_sqrt;
-                  adam1_fast(P[hh][0].x, vm.x, Mv[hh][0].x, Vv[hh][0].x, adam_c, ibc);
-                  adam1_fast(P[hh][0].y, vm.y, Mv[hh][0].y, Vv[hh][0].y, adam_c, ibc);
-                  adam1_fast(P[hh][0].z, vm.z, Mv[hh][0].z, Vv[hh][0].z, adam_c, ibc);
-                  adam1_fast(P[hh][0].w, vm.w, Mv[hh][0].w, Vv[hh][0].w, adam_c, ibc);
-                  adam1_fast(P[hh][1].x, vr.x, Mv[hh][1].x, Vv[hh][1].x, adam_c, ibc);
-                  adam1_fast(P[hh][1].y, vr.y, Mv[hh][1].y, Vv[hh][1].y, adam_c, ibc);
-                  adam1_fast(P[hh][1].z, vr.z, Mv[hh][1].z, Vv[hh][1].z, adam_c, ibc);
-                  adam1_fast(P[hh][1].w, vr.w, Mv[hh][1].w, Vv[hh][1].w, adam_c, ibc);
-                  *reinterpret_cast<float4 *>(const_cast<float *>(a.w_mu) + e) = P[hh][0];
-                  *reinterpret_cast<float4 *>(const_cast<float *>(a.w_rho) + e) = P[hh][1];
-                  *reinterpret_cast<float4 *>(a.adam_m[0] + e) = Mv[hh][0];
-                  *reinterpret_cast<float4 *>(a.adam_m[1] + e) = Mv[hh][1];
-                  *reinterpret_cast<float4 *>(a.adam_v[0] + e) = Vv[hh][0];
-                  *reinterpret_cast<float4 *>(a.adam_v[1] + e) = Vv[hh][1];
-                } else {
-                  float4 *pm = reinterpret_cast<float4 *>(a.g_w_mu + e), *pr = reinterpret_cast<float4 *>(a.g_w_rho + e);
-                  if (accum_flag || g > 0) {
-                    const float4 om = *pm, orr = *pr;
-                    vm.x += om.x; vm.y += om.y; vm.z += om.z; vm.w += om.w;
-                    vr.x += orr.x; vr.y += orr.y; vr.z += orr.z; vr.w += orr.w;
-                  }
-                  *pm = vm;
-                  *pr = vr;
+                float4 *pm = reinterpret_cast<float4 *>(a.g_w_mu + e), *pr = reinterpret_cast<float4 *>(a.g_w_rho + e);
+                if (accum_flag || g > 0) {
+                  const float4 om = *pm, orr = *pr;
+                  vm.x += om.x; vm.y += om.y; vm.z += om.z; vm.w += om.w;
+                  vr.x += orr.x; vr.y += orr.y; vr.z += orr.z; vr.w += orr.w;
                 }
+                *pm = vm;
+                *pr = vr;
               }
             }
           }
@@ -488,23 +438,19 @@ ws_bwd_kernel(const __grid_constant__ CUtensorMap tm_mu, const __grid_constant__
 inline int cdiv_i(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
 inline bool al16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
-template <int XWR, int MODE, bool kDx, bool kAdam>
+template <int XWR, int MODE, bool kDx>
 int launch_one(const CUtensorMap *tm, const MlpBwdArgs &a, dim3 grid, cudaStream_t st) {
-  auto kernel = ws_bwd_kernel<XWR, MODE, kDx, kAdam>;
+  auto kernel = ws_bwd_kernel<XWR, MODE, kDx>;
   BBB_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, BwdCfg<XWR>::kDyn));
   BBB_CHECK_CUDA(launch_pdl(kernel, grid, dim3(kThreadsB), (size_t)BwdCfg<XWR>::kDyn, st, tm[0], tm[1], tm[2], tm[3], tm[4], a));
   BBB_CHECK_LAUNCH();
   return BBB_OK;
 }
 template <int XWR>
-int launch_x(const CUtensorMap *tm, const MlpBwdArgs &a, dim3 grid, int mode, bool dx, bool adam, cudaStream_t st) {
-  if (adam) {      // (the fused optimiser is a training-step feature: Philox eps)
-    if (mode != 0) return fail(BBB_EUNSUPPORTED, "bbb_mlp_bwd: the fused optimiser needs Philox eps (no injected eps)");
-    return dx ? launch_one<XWR, 0, true, true>(tm, a, grid, st) : launch_one<XWR, 0, false, true>(tm, a, grid, st);
-  }
-  if (mode == 0) return dx ? launch_one<XWR, 0, true, false>(tm, a, grid, st) : launch_one<XWR, 0, false, false>(tm, a, grid, st);
-  if (mode == 1) return dx ? launch_one<XWR, 1, true, false>(tm, a, grid, st) : launch_one<XWR, 1, false, false>(tm, a, grid, st);
-  return dx ? launch_one<XWR, 2, true, false>(tm, a, grid, st) : launch_one<XWR, 2, false, false>(tm, a, grid, st);
+int launch_x(const CUtensorMap *tm, const MlpBwdArgs &a, dim3 grid, int mode, bool dx, cudaStream_t st) {
+  if (mode == 0) return dx ? launch_one<XWR, 0, true>(tm, a, grid, st) : launch_one<XWR, 0, false>(tm, a, grid, st);
+  if (mode == 1) return dx ? launch_one<XWR, 1, true>(tm, a, grid, st) : launch_one<XWR, 1, false>(tm, a, grid, st);
+  return dx ? launch_one<XWR, 2, true>(tm, a, grid, st) : launch_one<XWR, 2, false>(tm, a, grid, st);
 }
 
 }  // namespace
@@ -520,7 +466,7 @@ bool mlp_bwd_layer_supported(const MlpLayerDesc &l, int64_t S, int64_t B) {
 // (zero-filled by the caller: the CTAs of different row tiles add their partial sums).
 int launch_mlp_bwd_layer(const MlpLayerDesc &l, int64_t S, int64_t B, const RngDev &rng, const PriorDev &prior, int flags,
                          float gp, float gq, const float *gp_dev, const float *gq_dev, int g_dev_stride,
-                         const float *out_scale_dev, const bbb_adam_fuse *adam, cudaStream_t st) {
+                         const float *out_scale_dev, cudaStream_t st) {
   const bool sample = flags & BBB_F_SAMPLE;
   const int mode = !sample ? 2 : (l.eps_w ? 1 : 0);
   MlpBwdArgs a{};
@@ -534,11 +480,6 @@ int launch_mlp_bwd_layer(const MlpLayerDesc &l, int64_t S, int64_t B, const RngD
   a.n_ot = cdiv_i(l.out, a.T_o);
   a.flags = flags; a.x_shared = l.x_shared ? 1 : 0;
   a.timeline = debug_timeline();
-  if (adam) {
-    for (int k = 0; k < 4; ++k) { a.adam_m[k] = adam->exp_avg[k]; a.adam_v[k] = adam->exp_avg_sq[k]; }
-    a.adam_lr = adam->lr; a.adam_b1 = adam->beta1; a.adam_b2 = adam->beta2; a.adam_eps = (float)adam->eps;
-    a.adam_step = adam->step; a.adam_step_dev = adam->step_dev; a.adam_lr_scale_dev = adam->lr_scale_dev;
-  }
   a.gp = gp; a.gq = gq; a.gp_dev = gp_dev; a.gq_dev = gq_dev; a.g_dev_stride = g_dev_stride; a.out_scale_dev = out_scale_dev;
   const int nq_i = (int)(l.in / 4);
   int n_c = sm_count() / a.n_ot;                                   // about one CTA per SM
@@ -559,9 +500,9 @@ int launch_mlp_bwd_layer(const MlpLayerDesc &l, int64_t S, int64_t B, const RngD
     if (int r = tma::make_map(&tm[4], l.dz, l.out, B, S, 32, 128, tma::kSw128)) return r;
   dim3 grid(n_c, a.n_ot);
   const bool dx = l.dx != nullptr;
-  if (xwr == 1) return launch_x<1>(tm, a, grid, mode, dx, adam != nullptr, st);
-  if (xwr == 2) return launch_x<2>(tm, a, grid, mode, dx, adam != nullptr, st);
-  return launch_x<3>(tm, a, grid, mode, dx, adam != nullptr, st);
+  if (xwr == 1) return launch_x<1>(tm, a, grid, mode, dx, st);
+  if (xwr == 2) return launch_x<2>(tm, a, grid, mode, dx, st);
+  return launch_x<3>(tm, a, grid, mode, dx, st);
 }
 
 }  // namespace bbb

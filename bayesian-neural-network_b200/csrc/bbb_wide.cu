@@ -357,20 +357,14 @@ int launch_wide(const LinArgs &a, cudaStream_t st) {
   }
   const int n_bt = cdiv_w(a.B, NBT);
   dim3 grid(cdiv_w(kDgrad ? a.in : a.out, BM), n_bt, (unsigned)a.S);
-  static const int max_cl = [] { const char *e = getenv("BBB_WIDE_CL"); return e ? atoi(e) : 4; }();   // (experiments)
   // (clusters of 8 -- 15 co-resident on a B200 -- were tried for the energy they would save and did not complete: not
   // instantiated)
-  if (n_bt % 4 == 0 && max_cl >= 4) return launch_wide_cl<kDgrad, kLogProb, 4>(tm, a, grid, st);
-  if (n_bt % 2 == 0 && max_cl >= 2) return launch_wide_cl<kDgrad, kLogProb, 2>(tm, a, grid, st);
+  if (n_bt % 4 == 0) return launch_wide_cl<kDgrad, kLogProb, 4>(tm, a, grid, st);
+  if (n_bt % 2 == 0) return launch_wide_cl<kDgrad, kLogProb, 2>(tm, a, grid, st);
   return launch_wide_cl<kDgrad, kLogProb, 1>(tm, a, grid, st);
 }
 
 }  // namespace
-
-bool wide_disabled() {
-  static const bool off = [] { const char *e = getenv("BBB_NO_WIDE"); return e && e[0] == '1'; }();
-  return off;
-}
 
 int launch_linear_fwd_wide(const LinArgs &a, cudaStream_t st) {
   if (a.flags & BBB_F_LOGPROB) return launch_wide<false, true>(a, st);

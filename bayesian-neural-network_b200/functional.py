@@ -160,18 +160,11 @@ def _ws_fwd(x, x_stride, p, eps, l, prior, S, B, flags, y, logp, logq):
 
 
 def _ws_bwd(dy, mask, x, x_stride, p, eps, l, prior, S, B, flags, gp, gq, gp_dev, gq_dev, g_stride, out_scale, dx,
-            grads, adam=None):
+            grads):
     wm, wr, bm, br = p
     out, inn = wm.shape
     ew, eb = eps.ptrs(l)
     rng = eps.rng(l)
-    if adam is not None:      # the optimiser's update is applied inside the kernel; no gradient is written
-        L.check(L.lib().bbb_linear_bwd_adam(L.ptr(dy), L.ptr(mask), L.ptr(x), x_stride, L.ptr(wm), L.ptr(wr),
-                                            L.ptr(bm), L.ptr(br), ew, eb, C.byref(rng), C.byref(prior), S, B, inn,
-                                            out, flags, gp, gq, L.ptr(gp_dev), L.ptr(gq_dev), g_stride,
-                                            L.ptr(out_scale), L.ptr(dx), C.byref(adam), L.stream()),
-                'bbb_linear_bwd_adam')
-        return
     L.check(L.lib().bbb_linear_bwd(L.ptr(dy), L.ptr(mask), L.ptr(x), x_stride, L.ptr(wm), L.ptr(wr), L.ptr(bm),
                                    L.ptr(br), ew, eb, C.byref(rng), C.byref(prior), S, B, inn, out, flags,
                                    gp, gq, L.ptr(gp_dev), L.ptr(gq_dev), g_stride, L.ptr(out_scale), L.ptr(dx),
@@ -267,14 +260,14 @@ def _net_ws_forward(x2, params, prior, S, eps, sample, logprob, tf32, logp, logq
 
 
 def _net_ws_backward(x2, ys, d_out, params, prior, S, eps, sample, tf32, gp, gq, gp_dev, gq_dev, g_stride,
-                     out_scale, need_dx0, fused_opt=None, live_params=None, dxs=None):
+                     out_scale, need_dx0, dxs=None):
     """Backward of _net_ws_forward.  Returns (dx0 or None, [grads per layer]).  Every layer above the first
     hands down the gradient w.r.t. the PRE-activation output of the layer below (BBB_F_DX_PREACT: the ReLU mask
     is applied where dx is produced), so no layer needs a separate mask pass over dy."""
     B = x2.shape[0]
     ro = _relu_out_layers(params, B, tf32)
     base = (L.F_SAMPLE if sample else 0) | (L.F_TF32 if tf32 else 0) | (L.F_OUT_ZEROED if _prezero(B) else 0)
-    grads = _alloc_grads(params) if fused_opt is None else [None] * len(params)
+    grads = _alloc_grads(params)
     dy, dx0 = d_out, None
     first = 0 if need_dx0 else 1
     if dxs is None:
@@ -291,10 +284,9 @@ def _net_ws_backward(x2, ys, d_out, params, prior, S, eps, sample, tf32, gp, gq,
         if l == 0 and need_dx0:
             flags |= L.F_SCALE_DX
         x_in, stride = (x2, 0) if l == 0 else (ys[l - 1], B * inn)
-        adam = fused_opt.fuse_descriptor(live_params[l]) if fused_opt is not None else None
         _ws_bwd(dy, None, x_in, stride, p, eps, l, prior, S, B, flags, gp, gq, gp_dev, gq_dev, g_stride, out_scale,
-                dx, g, adam)
-        if grad_ready_hook is not None and fused_opt is None:
+                dx, g)
+        if grad_ready_hook is not None:
             grad_ready_hook(l, g.flat)
         dy = dx
         if l == 0:
@@ -399,9 +391,6 @@ def mlp_forward(x2, layers, prior, S, sample=True, logprob=True, tf32=False):
 # sample_elbo in TF32 mode goes through ONE C call per network pass (bbb_mlp_fwd / bbb_mlp_bwd) when the library covers
 # the network (bbb_mlp_supported); False forces the per-layer calls (A/B measurements, tools/check_mlp.py)
 use_network_level_call = True
-# the head on a full grid (csrc/bbb_head2.cu) instead of the 8-CTA-cluster head: measured SLOWER on B200 (23.6 + 21.0 us
-# against 16.0 + 9.4 us by ncu, cfg2), so it stays opt-in -- DESIGN.md 4.7
-use_full_grid_head = False
 
 
 def _layerwise_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, need_grad, tf32, beta_h, beta_d, out4):
@@ -447,7 +436,7 @@ def _layerwise_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, n
     return ys, dxs, d_out
 
 
-def _mlp_layer_table(params, eps, ys, dzs, grads, head_scratch=None):
+def _mlp_layer_table(params, eps, ys, dzs, grads):
     tab = (L.MlpLayer * len(params))()
     for l, p in enumerate(params):
         t = tab[l]
@@ -457,7 +446,6 @@ def _mlp_layer_table(params, eps, ys, dzs, grads, head_scratch=None):
         t.y, t.dz = L.ptr(ys[l]), L.ptr(dzs[l])
         if grads is not None and grads[l] is not None:
             t.g_w_mu, t.g_w_rho, t.g_b_mu, t.g_b_rho = (g.data_ptr() for g in grads[l])
-    tab[len(params) - 1].w_sample = L.ptr(head_scratch)
     return tab
 
 
@@ -482,10 +470,7 @@ def _mlp_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, need_gr
     dzs = (ws[1 + len(hidden):] if need_grad else [None] * len(hidden))
     logp, logq, nll = acc[:S], acc[S:2 * S], acc[2 * S:]
     d_out = torch.empty((S, B, Cc), dtype=torch.float32, device=dev) if need_grad else None
-    # the head's sampled weights (+ biases): written once by its forward, reused by its backward
-    hs = (torch.empty(S * Cc * params[-1][0].shape[1] + 16 * S, dtype=torch.float32, device=dev)
-          if use_full_grid_head else None)
-    tab = _mlp_layer_table(params, eps, ys, list(dzs) + [d_out], None, hs)
+    tab = _mlp_layer_table(params, eps, ys, list(dzs) + [d_out], None)
     kind = L.NLL_CE if mode == 'classification' else L.NLL_GAUSS
     tgt = target if mode == 'classification' else _f32c(target)
     rng = eps.rng(0)
@@ -493,7 +478,7 @@ def _mlp_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, need_gr
                                 L.F_SAMPLE | L.F_LOGPROB | L.F_TF32, kind, L.ptr(tgt), float(sigma), 1.0 / S,
                                 L.ptr(d_out), L.ptr(logp), L.ptr(logq), L.ptr(nll), beta_h, L.ptr(beta_d), L.ptr(out4),
                                 L.ptr(done), L.stream()), 'bbb_mlp_fwd')
-    return ys, ([None] + list(dzs) + [hs] if need_grad else None), d_out
+    return ys, ([None] + list(dzs) if need_grad else None), d_out
 
 
 class _FusedELBO(torch.autograd.Function):
@@ -502,7 +487,7 @@ class _FusedELBO(torch.autograd.Function):
     launch per layer (+ likelihood + assembly).  Only `loss` is differentiable."""
 
     @staticmethod
-    def forward(ctx, x2, target, beta, S, sigma, mode, prior, tf32, fused_opt, *flat):
+    def forward(ctx, x2, target, beta, S, sigma, mode, prior, tf32, *flat):
         L.require_cuda(x2, target, *flat)
         x2 = _f32c(x2)
         dev = x2.device
@@ -514,9 +499,8 @@ class _FusedELBO(torch.autograd.Function):
         out4 = torch.empty(4, dtype=torch.float32, device=dev)
         beta_h, beta_d = _split_beta(beta)
         dims = [params[0][0].shape[1]] + [p[0].shape[0] for p in params]
-        # (the optimiser fused into the network-level backward needs one sample group: S <= 2)
-        use_mlp = (use_network_level_call and tf32 and (fused_opt is None or S <= 2) and
-                   mode in ('classification', 'regression') and L.mlp_supported(dims, S, B, L.F_TF32))
+        use_mlp = (use_network_level_call and tf32 and mode in ('classification', 'regression') and
+                   L.mlp_supported(dims, S, B, L.F_TF32))
         if use_mlp:
             ys, dxs, d_out = _mlp_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, need_grad, beta_h,
                                                beta_d, out4)
@@ -530,7 +514,6 @@ class _FusedELBO(torch.autograd.Function):
         ctx.cfg = (prior, S, beta_h, tf32, eps, len(params))
         ctx.beta_dev = beta_d
         ctx.set_materialize_grads(False)      # no zero-filled gradients for the three non-differentiable scalars
-        ctx.fused_opt, ctx.live = fused_opt if fused_opt is not None else (None, None)
         loss, lp, lq, nl = out4[0:1], out4[1], out4[2], out4[3:4]
         ctx.mark_non_differentiable(lp, lq, nl)
         return loss, lp, lq, nl
@@ -539,7 +522,7 @@ class _FusedELBO(torch.autograd.Function):
     def backward(ctx, g_loss, *unused):
         prior, S, beta, tf32, eps, nl = ctx.cfg
         if g_loss is None:
-            return (None,) * (9 + 4 * nl)
+            return (None,) * (8 + 4 * nl)
         if getattr(ctx, 'consumed', False):
             # the split-K backward kernels ADD into the dx workspace zero-filled by the forward (BBB_F_OUT_ZEROED)
             raise RuntimeError('sample_elbo: this graph was already differentiated (retain_graph=True is not '
@@ -551,42 +534,16 @@ class _FusedELBO(torch.autograd.Function):
         ys = list(sv[2 + 4 * nl:2 + 4 * nl + nl - 1]) + [None]
         scale = _f32c(g_loss).reshape(1)
         bd = ctx.beta_dev
-        if ctx.fused_opt is not None and ctx.used_mlp:
-            # ONE C call: backward of every layer with the optimiser's update applied in the kernels' gradient write-back
-            # (parameters change here, no .grad appears); only the head's gradients are materialised (scratch)
-            with torch.no_grad():
-                B = x2.shape[0]
-                overlap = bool(getattr(ctx.fused_opt, 'overlap_backward', False))
-                if overlap:     # ordinary backward kernels + per-layer Adam on a side stream: every layer writes gradients
-                    sg = _alloc_grads(params)
-                else:           # update in the write-back: only the head writes its gradients
-                    sg = [None] * (nl - 1) + [_alloc_grads(params[-1:])[0]]
-                tab = _mlp_layer_table(params, eps, ys, list(ctx.dxs[1:nl]) + [d_out], sg, ctx.dxs[nl])
-                adam = (L.AdamFuse * nl)()
-                for l in range(nl):
-                    d = ctx.fused_opt.fuse_descriptor(ctx.live[l])
-                    C.memmove(C.byref(adam[l]), C.byref(d), C.sizeof(L.AdamFuse))
-                rng = eps.rng(0)
-                L.check(L.lib().bbb_mlp_bwd(tab, nl, L.ptr(x2), S, B, C.byref(rng), C.byref(prior),
-                                            L.F_SAMPLE | L.F_TF32 | (L.F_ADAM_OVERLAP if overlap else 0), -beta / S,
-                                            beta / S, L.ptr(bd), L.ptr(bd), 0, L.ptr(scale), adam, L.stream()),
-                        'bbb_mlp_bwd')
-            return (None,) * (9 + 4 * nl)
-        if ctx.fused_opt is not None:     # Adam rides in the backward kernels: parameters change here, no .grad appears
-            with torch.no_grad():
-                _net_ws_backward(x2, ys, d_out, params, prior, S, eps, True, tf32, -beta / S, beta / S, bd, bd, 0,
-                                 scale, False, ctx.fused_opt, ctx.live, ctx.dxs)
-            return (None,) * (9 + 4 * nl)
         if ctx.used_mlp:
             # ONE C call for the whole backward (bbb_mlp_bwd): ys are the stored pre-activations, ctx.dxs[l + 1] the
             # zero-filled gradient w.r.t. hidden layer l's pre-activation output
             grads = _alloc_grads(params)
             B = x2.shape[0]
             dzs = list(ctx.dxs[1:nl]) + [d_out]
-            tab = _mlp_layer_table(params, eps, ys, dzs, grads, ctx.dxs[nl])
+            tab = _mlp_layer_table(params, eps, ys, dzs, grads)
             rng = eps.rng(0)
             L.check(L.lib().bbb_mlp_bwd(tab, nl, L.ptr(x2), S, B, C.byref(rng), C.byref(prior), L.F_SAMPLE | L.F_TF32,
-                                        -beta / S, beta / S, L.ptr(bd), L.ptr(bd), 0, L.ptr(scale), None, L.stream()),
+                                        -beta / S, beta / S, L.ptr(bd), L.ptr(bd), 0, L.ptr(scale), L.stream()),
                     'bbb_mlp_bwd')
             if grad_ready_hook is not None:
                 for l in reversed(range(nl)):
@@ -595,14 +552,12 @@ class _FusedELBO(torch.autograd.Function):
             _, grads = _net_ws_backward(x2, ys, d_out, params, prior, S, eps, True, tf32, -beta / S, beta / S,
                                         bd, bd, 0, scale, False, dxs=ctx.dxs)
         flat = [g for lg in grads for g in lg]
-        return (None,) * 9 + tuple(flat)
+        return (None,) * 8 + tuple(flat)
 
 
-def fused_elbo(x2, target, beta, S, sigma, mode, prior, layers, tf32=False, fused_opt=None):
-    """fused_opt: None, or a bnn_b200.FusedAdam whose next step the backward kernels apply themselves."""
+def fused_elbo(x2, target, beta, S, sigma, mode, prior, layers, tf32=False):
     flat = [t for layer in layers for t in layer]
-    fo = (fused_opt, [tuple(layer) for layer in layers]) if fused_opt is not None else None
-    return _FusedELBO.apply(x2, target, beta, S, sigma, mode, prior, tf32, fo, *flat)
+    return _FusedELBO.apply(x2, target, beta, S, sigma, mode, prior, tf32, *flat)
 
 
 # =========================================================================================

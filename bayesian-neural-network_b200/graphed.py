@@ -18,6 +18,12 @@ from . import parallel
 
 class GraphedTrainStep:
     def __init__(self, net, optimizer, x, y, samples, sigma=1.0, beta=1.0, world_size=1, warmup=3, fuse_optimizer=False):
+        # The optimiser's update applied inside the backward kernels (in their gradient write-back, or overlapped on a
+        # side stream) measured slower than, or no faster than, the stand-alone multi-tensor Adam launch; it was
+        # removed (DESIGN.md §4.6).  The keyword stays so that callers which pass fuse_optimizer=False keep working.
+        if fuse_optimizer:
+            raise ValueError('fuse_optimizer: the optimiser fused into the backward was removed (DESIGN.md §4.6); '
+                             'the step runs the backward, then one FusedAdam launch')
         L.require_cuda(x, y)
         self.net, self.opt, self.samples, self.sigma, self.world = net, optimizer, samples, sigma, world_size
         self.x, self.y = x.clone(), y.clone()
@@ -41,16 +47,6 @@ class GraphedTrainStep:
         if hasattr(optimizer, 'lr_scale_dev') and self._lr0 > 0:
             self.lr_scale = torch.ones(1, dtype=torch.float32, device=dev)
             optimizer.lr_scale_dev = self.lr_scale
-        # Opt-in, one GPU: the optimiser's update rides in the backward kernels' gradient epilogue (no gradient round
-        # trip, no optimiser launch).  Off by default: measured on B200 at the MNIST-shape config the update then runs
-        # as a memory-bound tail of every backward CTA and the step is slower (0.214 ms) than with the stand-alone
-        # multi-tensor kernel at 92 % of HBM peak (0.188 ms).  With several GPUs the gradients are all-reduced first.
-        # fuse_optimizer='overlap': the ordinary backward kernels, each layer's Adam update on a side stream under the
-        # backward of the layer below (a parallel branch of the captured graph)
-        self.optimizer_fused = bool(fuse_optimizer and world_size == 1 and hasattr(net, 'fuse_optimizer')
-                                    and x.shape[0] <= 128
-                                    and net.fuse_optimizer(optimizer, overlap=(fuse_optimizer == 'overlap')))
-        self.optimizer_overlapped = self.optimizer_fused and fuse_optimizer == 'overlap' 
         # warm-up and capture must not train the model: snapshot parameters and optimiser state, restore after
         params = [p for g in optimizer.param_groups for p in g['params']]
         p_snap = [p.detach().clone() for p in params]

@@ -98,27 +98,9 @@ class BayesianNetwork(nn.Module):
             if i + 1 < self.n_layers:
                 setattr(self, f'l{i + 1}_act', nn.ReLU())
         self._prior = None if self.local_reparam else F.make_prior(self.prior_init, self.mixture_prior)
-        self._fused_opt = None
 
     def layers(self):
         return [getattr(self, f'l{i + 1}') for i in range(self.n_layers)]
-
-    def fuse_optimizer(self, optimizer, overlap=False):
-        """Opt-in (single GPU): let the backward of sample_elbo apply `optimizer`'s (bnn_b200.FusedAdam) next step --
-        loss.backward() then UPDATES the parameters and leaves .grad unset, and the optimizer.step() that follows only
-        advances the step count.  overlap=False: the update rides in the backward kernels' gradient epilogue (measured
-        slower, DESIGN 4.6); overlap=True: the ordinary backward kernels run and every layer's Adam update is launched
-        on a side stream as soon as that layer's backward has finished, under the backward of the layer below
-        (BBB_F_ADAM_OVERLAP; network-level path only).  Returns False (and changes nothing) when this network cannot
-        run the fused tcgen05 backward.  fuse_optimizer(None) switches back."""
-        if optimizer is None:
-            self._fused_opt = None
-            return True
-        optimizer.overlap_backward = bool(overlap)
-        ok = (self.tf32 and self.fused and not self.local_reparam and self.batch_size <= 128 and
-              all(l.weight_mu.shape[1] % 4 == 0 for l in self.layers()) and hasattr(optimizer, 'fuse_descriptor'))
-        self._fused_opt = optimizer if ok else None
-        return ok
 
     def forward(self, x, sample=False):
         if self.mode == 'classification':
@@ -244,8 +226,7 @@ class BayesianNetwork(nn.Module):
         x2 = self._flat_input(input)
         params = [l.params() for l in self.layers()]
         if self._fusable(x2, target):
-            fo = self._fused_opt if (self._fused_opt is not None and self.training and x2.shape[0] <= 128) else None
-            return F.fused_elbo(x2, target, beta, samples, sigma, self.mode, self._prior, params, self.tf32, fo)
+            return F.fused_elbo(x2, target, beta, samples, sigma, self.mode, self._prior, params, self.tf32)
         outs, lps, lqs = F.mlp_forward(x2, params, self._prior, samples, True, True, self.tf32)
         negative_log_likelihood = torch.zeros(1, device=outs.device)
         for i in range(samples):

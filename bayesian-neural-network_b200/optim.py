@@ -29,24 +29,6 @@ class FusedAdam(torch.optim.Optimizer):
             st['exp_avg_sq'] = torch.zeros_like(p, memory_format=torch.preserve_format)
         return st
 
-    def fuse_descriptor(self, layer_params):
-        """bbb_adam_fuse for one layer's (w_mu, w_rho, b_mu, b_rho): lets the fused backward kernel apply THIS
-        optimiser's next step in its gradient epilogue (bbb_linear_bwd_adam).  The step() that follows finds no
-        gradients, launches nothing and only advances the step count."""
-        group = next(g for g in self.param_groups if any(q is layer_params[0] for q in g['params']))
-        d = L.AdamFuse()
-        for k, p in enumerate(layer_params):
-            if not (p.is_contiguous() and p.dtype == torch.float32):
-                raise RuntimeError('FusedAdam needs contiguous fp32 parameters')
-            st = self._ensure_state(p)
-            d.exp_avg[k], d.exp_avg_sq[k] = st['exp_avg'].data_ptr(), st['exp_avg_sq'].data_ptr()
-        b1, b2 = group['betas']
-        d.lr, d.beta1, d.beta2, d.eps = float(group['lr']), float(b1), float(b2), float(group['eps'])
-        d.step = self._t + 1
-        d.step_dev = L.ptr(self.step_dev)
-        d.lr_scale_dev = L.ptr(self.lr_scale_dev)
-        return d
-
     def _mirror_step(self):
         """torch.optim.Adam keeps the step count in state[p]['step']: mirror ours there so a state_dict round trip
         (or handing the state to torch.optim.Adam) continues the bias correction instead of restarting it."""

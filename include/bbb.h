@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define BBB_VERSION 100
+#define BBB_VERSION 101
 
 /* error codes */
 #define BBB_OK 0
@@ -59,11 +59,6 @@ extern "C" {
                                no kernel spends shared-memory bandwidth on a ReLU pass over TMA-landed tiles.  Implemented
                                by the large-batch tensor kernels only: ask bbb_linear_fwd_relu_out_supported first; a
                                call that sets it on any other path returns BBB_EUNSUPPORTED. */
-#define BBB_F_ADAM_OVERLAP 2048 /* bbb_mlp_bwd with Adam descriptors: do NOT fuse the update into the gradient write-back;
-                               run the ordinary backward kernels (gradient pointers required) and launch each layer's
-                               Adam update on a side stream as soon as that layer's backward kernel has finished, so the
-                               bandwidth-bound update of layer l overlaps the latency-bound backward of layer l - 1.  The
-                               side stream is forked from and joined back into `stream` (graph-capture safe). */
 #define BBB_F_OUT_ZEROED 256 /* y (forward) / dx (backward) is already zero-filled by the caller: kernels that
                                combine split-K partial sums with red.add skip their own memset              */
 
@@ -126,27 +121,6 @@ int bbb_linear_bwd(const float *dy, const float *dy_mask_src, const float *x, in
                    const float *gp_dev, const float *gq_dev, int64_t g_dev_stride,
                    const float *out_scale_dev, float *dx, float *grad_w_mu, float *grad_w_rho,
                    float *grad_b_mu, float *grad_b_rho, void *stream);
-
-/* The same backward with the optimiser step fused into its gradient epilogue (SURVEY 8f-1): once a CTA holds the
- * complete gradient of its block of weights it applies torch.optim.Adam's update to w_mu / w_rho / b_mu / b_rho in
- * place and never writes the gradient -- the 16 B/weight gradient round trip and the optimiser launch disappear.
- * Replaces loss.backward() + optimiser.step() at reg_task.py:72-73, class_task.py:78-79, bandits.py:49-50 for
- * single-GPU steps (with several GPUs the gradients must be all-reduced first: use bbb_linear_bwd + bbb_adam_step).
- * Only the fused tcgen05 backward implements it (BBB_F_TF32, B <= 128, rows of 16-byte multiples); otherwise the
- * call returns BBB_EUNSUPPORTED and nothing is launched.  exp_avg / exp_avg_sq: state of w_mu, w_rho, b_mu, b_rho. */
-typedef struct bbb_adam_fuse {
-  float *exp_avg[4], *exp_avg_sq[4];
-  double lr, beta1, beta2, eps;
-  uint32_t step;              /* 1-based Adam step; *step_dev is added when non-NULL (CUDA-graph replay)       */
-  const uint32_t *step_dev;
-  const float *lr_scale_dev;  /* optional device scalar multiplying lr                                        */
-} bbb_adam_fuse;
-int bbb_linear_bwd_adam(const float *dy, const float *dy_mask_src, const float *x, int64_t x_sample_stride,
-                        float *w_mu, float *w_rho, float *b_mu, float *b_rho, const float *eps_w,
-                        const float *eps_b, const bbb_rng *rng, const bbb_prior *prior, int64_t S, int64_t B,
-                        int64_t in, int64_t out, int32_t flags, float gp, float gq, const float *gp_dev,
-                        const float *gq_dev, int64_t g_dev_stride, const float *out_scale_dev, float *dx,
-                        const bbb_adam_fuse *adam, void *stream);
 
 /* ---- local-reparameterisation layer ----------------------------------------------------
  * replaces BayesianLinearLR.forward (networks.py:116-138) and compute_kl_cost (109-114).
@@ -277,10 +251,6 @@ typedef struct bbb_mlp_layer {
   const float *w_mu, *w_rho, *b_mu, *b_rho, *eps_w, *eps_b;
   int64_t in, out;
   float *y;                                       /* [S,B,out] pre-activation output (hidden layers: zero-filled)          */
-  float *w_sample;                                /* last layer only, nullable: scratch of S*out*in + 16*S floats.  When given,
-                                                     the head runs on the full-grid kernels of csrc/bbb_head2.cu (weights sampled
-                                                     once into the scratch, which the backward reuses) and done_counter must
-                                                     point to TWO zeroed words; NULL: the cluster head of bbb_head_fwd        */
   float *dz;                                      /* [S,B,out]: hidden layers zero-filled, accumulated by the layer above */
   float *g_w_mu, *g_w_rho, *g_b_mu, *g_b_rho;     /* parameter gradients, overwritten                                     */
 } bbb_mlp_layer;
@@ -294,17 +264,10 @@ int bbb_mlp_fwd(const bbb_mlp_layer *layers, int32_t n_layers, const float *x, i
  * out_scale_dev meaning, eps regenerated from the same Philox coordinates).  Reads layers[l].y (the pre-activations the
  * forward stored) and layers[n-1].dz (= d_out of bbb_mlp_fwd); layers[l].dz of the hidden layers must be zero-filled:
  * the layer above adds (dz W_s) (y > 0) into it.  Writes g_w_mu / g_w_rho / g_b_mu / g_b_rho of every layer
- * (added to with BBB_F_ACCUM).
- * adam (nullable; n_layers descriptors, see bbb_linear_bwd_adam): the optimiser's next step is applied by the backward
- * kernels themselves -- replaces loss.backward() + optimiser.step() (reg_task.py:72-73, class_task.py:78-79,
- * bandits.py:49-50) for single-GPU steps with S <= 2: a hidden layer's CTA that holds the complete gradient of its block
- * of weights updates w_mu / w_rho / b_mu / b_rho and the Adam state in place in its coalesced write-back and writes no
- * gradient (g_* of hidden layers may be NULL); the head's gradients are written and updated by one small launch.
- * sqrt and the division use the SFU approximations (1-ulp level).  Returns BBB_EUNSUPPORTED for S > 2 or BBB_F_ACCUM. */
+ * (added to with BBB_F_ACCUM). */
 int bbb_mlp_bwd(const bbb_mlp_layer *layers, int32_t n_layers, const float *x, int64_t S, int64_t B,
                 const bbb_rng *rng, const bbb_prior *prior, int32_t flags, float gp, float gq, const float *gp_dev,
-                const float *gq_dev, int64_t g_dev_stride, const float *out_scale_dev, const bbb_adam_fuse *adam,
-                void *stream);
+                const float *gq_dev, int64_t g_dev_stride, const float *out_scale_dev, void *stream);
 
 /* ELBO assembly (networks.py:205-209 / 221-225):
  * out4 = { beta mean(logq) - beta mean(logp) + nll/S, mean(logp), mean(logq), nll/S }   (kl == NULL)

@@ -135,25 +135,6 @@ class FakeLib:
             G[...] = (G + osc * val if flags & F_ACCUM else osc * val).astype(np.float32)
         return 0
 
-    def bbb_linear_bwd_adam(self, dy, mask, x, xs, wm, wr, bm, br, ew, eb, rng, prior, S, B, inn, out, flags, gp, gq,
-                            gp_dev, gq_dev, gstride, oscale, dx, adam, st):
-        """backward, then the optimiser's update of (w_mu, w_rho, b_mu, b_rho) in place; no gradient output"""
-        assert flags & F_TF32 and not flags & (F_ACCUM | F_NO_WGRAD)
-        d = adam._obj
-        gs = [np.zeros(sh, dtype=np.float32) for sh in ((out, inn), (out, inn), (out,), (out,))]
-        self.bbb_linear_bwd(dy, mask, x, xs, wm, wr, bm, br, ew, eb, rng, prior, S, B, inn, out, flags, gp, gq, gp_dev,
-                            gq_dev, gstride, oscale, dx, *[g.ctypes.data for g in gs], st)
-        self.calls[-1] = 'linear_bwd_adam'
-        t = d.step + (int(_arr(d.step_dev, C.c_uint32, 1)[0]) if d.step_dev else 0)
-        lr = d.lr * (float(_f(d.lr_scale_dev, 1)[0]) if d.lr_scale_dev else 1.0)
-        bc1, bc2 = 1 - d.beta1 ** t, 1 - d.beta2 ** t
-        for k, (ptr, g) in enumerate(zip((wm, wr, bm, br), gs)):
-            p, m, v = _f(ptr, *g.shape), _f(d.exp_avg[k], *g.shape), _f(d.exp_avg_sq[k], *g.shape)
-            m[...] = d.beta1 * m + (1 - d.beta1) * g
-            v[...] = d.beta2 * v + (1 - d.beta2) * g * g
-            p[...] = p - (lr / bc1) * m / (np.sqrt(v) / np.sqrt(bc2) + d.eps)
-        return 0
-
     # ---------------------------------------------------------------- local reparameterisation
     def bbb_lr_linear_fwd(self, x, xs, wm, wr, bm, br, ea, eb, rng, sigma_p, S, B, inn, out, flags, y, delta, kl, st):
         self.calls.append('lr_fwd')
@@ -326,7 +307,7 @@ class FakeLib:
         self.calls.append('head_fwd')
         return 0
 
-    def bbb_mlp_bwd(self, layers, n_layers, x, S, B, rng, prior, flags, gp, gq, gp_dev, gq_dev, gstride, oscale, adam, st):
+    def bbb_mlp_bwd(self, layers, n_layers, x, S, B, rng, prior, flags, gp, gq, gp_dev, gq_dev, gstride, oscale, st):
         """backward of bbb_mlp_fwd: per layer bbb_linear_bwd on the stored pre-activations; the gradient w.r.t. a hidden
         layer's pre-activation output is ADDED into its (zero-filled) dz buffer"""
         self.calls.append('mlp_bwd')
@@ -339,26 +320,9 @@ class FakeLib:
             if l > 0:
                 assert not np.any(_f(layers[l - 1].dz, S, B, t.inn)), 'fake lib: hidden dz buffers must be zeroed'
                 dx = layers[l - 1].dz
-            gptrs = (t.g_w_mu, t.g_w_rho, t.g_b_mu, t.g_b_rho)
-            shapes = ((t.out, t.inn), (t.out, t.inn), (t.out,), (t.out,))
-            if adam is not None:            # the optimiser's update replaces the gradient output (the head still writes its own)
-                assert S <= 2 and not flags & F_ACCUM
-                gs = [np.zeros(sh, dtype=np.float32) for sh in shapes]
-                if l + 1 < n_layers:
-                    gptrs = tuple(g.ctypes.data for g in gs)
             self.bbb_linear_bwd(t.dz, None, inp, xs, t.w_mu, t.w_rho, t.b_mu, t.b_rho, t.eps_w, t.eps_b, rng, prior, S, B,
-                                t.inn, t.out, fl, gp, gq, gp_dev, gq_dev, gstride, oscale, dx, *gptrs, st)
-            if adam is not None:
-                d = adam[l]
-                step = d.step + (int(_arr(d.step_dev, C.c_uint32, 1)[0]) if d.step_dev else 0)
-                lr = d.lr * (float(_f(d.lr_scale_dev, 1)[0]) if d.lr_scale_dev else 1.0)
-                bc1, bc2 = 1 - d.beta1 ** step, 1 - d.beta2 ** step
-                for k, (ptr, sh) in enumerate(zip((t.w_mu, t.w_rho, t.b_mu, t.b_rho), shapes)):
-                    g = _f(gptrs[k], *sh)
-                    p, m, v = _f(ptr, *sh), _f(d.exp_avg[k], *sh), _f(d.exp_avg_sq[k], *sh)
-                    m[...] = d.beta1 * m + (1 - d.beta1) * g
-                    v[...] = d.beta2 * v + (1 - d.beta2) * g * g
-                    p[...] = p - (lr / bc1) * m / (np.sqrt(v) / np.sqrt(bc2) + d.eps)
+                                t.inn, t.out, fl, gp, gq, gp_dev, gq_dev, gstride, oscale, dx, t.g_w_mu, t.g_w_rho,
+                                t.g_b_mu, t.g_b_rho, st)
         del self.calls[n0:]
         return 0
 

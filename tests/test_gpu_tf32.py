@@ -44,13 +44,6 @@ def test_tf32_train_step_matches_reference(name, fused):
     PC.check_train_step(c, DEV, fused=fused, rtol=1e-5, rtol_gemm=2e-2 if c.lr else RTOL_TF32, tf32=True)
 
 
-@pytest.mark.parametrize('name', BIG + DEEP_BIG)
-def test_tf32_train_step_with_full_grid_head(name, monkeypatch):
-    # the opt-in head on a full grid (csrc/bbb_head2.cu; functional.use_full_grid_head) against the same fixtures
-    monkeypatch.setattr(bnn_b200.functional, 'use_full_grid_head', True)
-    PC.check_train_step(Case(name), DEV, fused=True, rtol=1e-5, rtol_gemm=RTOL_TF32, tf32=True)
-
-
 def test_lr_tf32_backward_kernels_alone_within_bound():
     """The LR estimator's tcgen05 backward kernels against its exact fp32 kernels on the SAME stored forward state (same
     y, delta, eps, hence identical ReLU masks): every gradient within the TF32 bound of 5e-3."""

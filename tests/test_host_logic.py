@@ -31,7 +31,7 @@ def test_train_step_network_level(fake, name, fused):
 
 
 @pytest.mark.parametrize('name', ['small_cls_mix', 'small_cls_gauss', 'deep5_small_mix'])
-def test_train_step_through_the_network_level_call(fake, name):
+def test_tf32_train_step_takes_the_network_level_call_when_supported(fake, name):
     """tf32=True routes sample_elbo through ONE bbb_mlp_fwd call when bbb_mlp_supported says so (hidden widths that are
     multiples of 4, a head on top), otherwise through the per-layer calls; same results either way."""
     case = Case(name)
@@ -87,7 +87,7 @@ def test_no_cpu_fallback():
         net(c.x, sample=True)
 
 
-def test_library_exports_every_declared_symbol():
+def test_library_matches_the_header():
     """libbbb.so loads and exports every function include/bbb.h declares (no compute calls)."""
     hdr = open(os.path.join(ROOT, 'include', 'bbb.h')).read()
     declared = set(re.findall(r'\b(bbb_[a-z0-9_]+)\s*\(', hdr))
@@ -95,7 +95,7 @@ def test_library_exports_every_declared_symbol():
     lib = ctypes.CDLL(bnn_b200._lib.LIB_PATH)
     for name in declared:
         assert hasattr(lib, name), name
-    assert bnn_b200._lib.lib().bbb_version() == 100
+    assert bnn_b200._lib.lib().bbb_version() == 101
 
 
 def test_product_does_not_import_oracle():
@@ -271,41 +271,13 @@ def test_beta_may_be_a_tensor(fake):
     assert outs[0][0] == outs[1][0] and torch.allclose(outs[0][1], outs[1][1], rtol=1e-6, atol=1e-9)
 
 
-@pytest.mark.parametrize('network_level,overlap', [(True, False), (True, True), (False, False)])
-def test_fused_optimizer_step_equals_backward_then_adam(fake, network_level, overlap, monkeypatch):
-    """net.fuse_optimizer(opt): backward applies Adam inside bbb_mlp_bwd (network-level call) / bbb_linear_bwd_adam
-    (per-layer calls) and leaves .grad unset; the parameters after 2 steps equal backward + FusedAdam.step()."""
-    from bnn_b200 import functional as F
-    monkeypatch.setattr(F, 'use_network_level_call', network_level)
+def test_graphed_step_refuses_the_removed_fused_optimizer():
+    """fuse_optimizer is kept as a keyword for existing callers; asking for the removed path fails before anything is
+    allocated or captured, whatever the device"""
     c = Case('small_cls_mix')
-    res = []
-    for fuse in (False, True):
-        net = PC.build_net(c, 'cpu', tf32=True).train()
-        opt = bnn_b200.FusedAdam(net.parameters(), lr=1e-2)
-        if fuse:
-            assert net.fuse_optimizer(opt, overlap=overlap)
-        with bnn_b200.eps_mode('reference'):
-            torch.manual_seed(5)
-            for _ in range(2):
-                net.zero_grad()
-                loss = net.sample_elbo(c.x, c.y, c.beta, c.S)[0]
-                loss.backward()
-                assert all((p.grad is None) == fuse for p in net.parameters())
-                opt.step()
-        res.append([p.detach().clone() for p in net.parameters()])
-        assert ('mlp_bwd' in fake.calls) == network_level
-        if not network_level:
-            assert ('linear_bwd_adam' in fake.calls) == fuse
-    for a, b in zip(*res):
-        assert torch.allclose(a, b, rtol=1e-5, atol=1e-7), float((a - b).abs().max())
-
-
-def test_fuse_optimizer_refuses_what_the_kernel_cannot_do(fake):
-    c = Case('small_reg_mix')                      # input width 5: rows are not 16-byte multiples
-    net = PC.build_net(c, 'cpu', tf32=True)
-    assert net.fuse_optimizer(bnn_b200.FusedAdam(net.parameters())) is False and net._fused_opt is None
-    net = PC.build_net(Case('small_lr_cls'), 'cpu')
-    assert net.fuse_optimizer(bnn_b200.FusedAdam(net.parameters())) is False
+    net = PC.build_net(c, 'cpu')
+    with pytest.raises(ValueError, match='DESIGN.md §4.6'):
+        bnn_b200.GraphedTrainStep(net, bnn_b200.FusedAdam(net.parameters()), c.x, c.y, c.S, fuse_optimizer=True)
 
 
 @pytest.mark.parametrize('name', SMALL + SMALL_LR)

@@ -27,10 +27,7 @@ The posterior scales are large here (rho in [-1.5, -0.5], sigma 0.2-0.5, against
 missing eps term in one K block, batch row or sample group then moves an output by several per cent of its max.
 """
 import ctypes as C
-import os
 import re
-import subprocess
-import sys
 import zlib
 
 import numpy as np
@@ -42,8 +39,6 @@ from oracle import closed_form as CF
 from tests.fake_bbb import (FakeLib, F_SAMPLE, F_LOGPROB, F_RELU_IN, F_ACCUM, F_TF32, F_NO_DX, F_SCALE_DX, F_NO_WGRAD,
                             F_OUT_ZEROED, F_DX_PREACT, F_RELU_OUT)
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-NO_WIDE = os.environ.get('BBB_NO_WIDE') == '1'   # read once per process by the library: the child run below sets it
 
 MIX, GAUSS = ('mixture', 0.5, 1.0, float(np.exp(-6.0))), ('gaussian', 1.0)
 RTOL_Y, RTOL_G, RTOL_SUM, RTOL_TF32 = 2e-5, 5e-5, 1e-5, 5e-3
@@ -93,9 +88,7 @@ TF32_ROUNDING = {
     'tc_fwd':     {'fwd': ('rn', 'rn')},                           # bbb_linear_tc.cu: st_tile4 for both
     'tc_bwd':     {'dgrad': ('rn', 'rn'), 'wgrad': ('rn', 'rn')},
     'wide_fwd':   {'fwd': ('trunc', 'rn')},                        # bbb_wide.cu: x by TMA, w to_tf32
-    'big_fwd':    {'fwd': ('trunc', 'rn')},                        # bbb_linear_big.cu: x raw, w to_tf32
     'wide_bwd':   {'dgrad': ('trunc', 'rn'), 'wgrad': ('trunc', 'trunc')},   # big_wgrad_kernel: slabs as stored
-    'big_bwd':    {'dgrad': ('trunc', 'rn'), 'wgrad': ('trunc', 'trunc')},
     'fused_bwd':  {'dgrad': ('trunc', 'rn'), 'wgrad': ('trunc', 'trunc')},   # dz / x tiles raw, Wt to_tf32
     'lr_tc_fwd':  {'mean': ('rn', 'rn'), 'var': ('rn', 'rn')},     # bbb_lr_tc.cu: every operand to_tf32
     'lr_tc_bwd':  {'dgrad_mean': ('trunc', 'trunc'), 'dgrad_var': ('trunc', 'trunc'),
@@ -104,15 +97,13 @@ TF32_ROUNDING = {
 # Tight bounds after emulation (max-norm per tensor, beyond the slack of tf32_ambiguity and of the mixture prior's
 # conditioning, see _emu_linear_bwd): 10x the largest value observed over this table on a B200 (1000 W power limit),
 # capped at 5e-5.  The observed maxima, all in the weight-sampling wgrad where they come with the mixture prior:
-# wide_bwd / big_bwd 1.2e-5 and fused_bwd 6.4e-6 (headroom 4x and 8x under the cap).
+# wide_bwd 1.2e-5 and fused_bwd 6.4e-6 (headroom 4x and 8x under the cap).
 TIGHT = {
     'sk_fwd': 3.2e-5,       # observed 3.2e-6
     'tc_fwd': 2e-5,         # 1.8e-6
     'tc_bwd': 3.5e-5,       # 3.3e-6
     'wide_fwd': 5e-5,       # 6.6e-6
-    'big_fwd': 2e-5,        # 1.9e-6
     'wide_bwd': 5e-5,       # 1.2e-5
-    'big_bwd': 5e-5,        # 1.2e-5
     'fused_bwd': 5e-5,      # 6.4e-6
     'lr_tc_fwd': 2e-6,      # 1.7e-7
     'lr_tc_bwd': 1e-5,      # 8.4e-7
@@ -125,14 +116,12 @@ FAMILIES = {
     'head_fwd':       ('fwd', ['head_fwd_kernel']),
     'sk_fwd':         ('fwd', ['fwd_sk_kernel']),
     'wide_fwd':       ('fwd', ['wide_kernel']),
-    'big_fwd':        ('fwd', ['big_kernel']),                     # BBB_NO_WIDE=1
     'tc_fwd':         ('fwd', ['fwd_tc_kernel']),
     'narrow_fwd':     ('fwd', ['narrow_fwd_kernel']),
     'fma_fwd':        ('fwd', ['fwd_fma_kernel']),
     'head_bwd':       ('bwd', ['head_bwd_kernel']),
     'fused_bwd':      ('bwd', ['bwd_fused_kernel']),
     'wide_bwd':       ('bwd', ['wide_kernel', 'big_wgrad_kernel']),
-    'big_bwd':        ('bwd', ['big_kernel', 'big_wgrad_kernel']),  # BBB_NO_WIDE=1
     'tc_bwd':         ('bwd', ['dgrad_tc_kernel', 'wgrad_tc_kernel']),
     'narrow_bwd':     ('bwd', ['narrow_bwd_kernel']),
     'fma_bwd':        ('bwd', ['dgrad_fma_kernel', 'wgrad_fma_kernel']),
@@ -150,7 +139,7 @@ ALL_KERNELS = sorted({k for _, ks in FAMILIES.values() for k in ks} | set(EXTRA_
 DGRAD_KERNELS = {'dgrad_tc_kernel', 'dgrad_fma_kernel', 'lr_dgrad_sk_kernel', 'lr_dgrad_kernel'}
 WGRAD_KERNELS = {'wgrad_tc_kernel', 'wgrad_fma_kernel', 'thin_wgrad_kernel', 'big_wgrad_kernel', 'wgrad_combine_kernel',
                  'lr_wgrad_tc_kernel', 'lr_wgrad_kernel'}
-LARGE_BATCH = {'wide_fwd', 'big_fwd', 'wide_bwd', 'big_bwd'}
+LARGE_BATCH = {'wide_fwd', 'wide_bwd'}
 
 
 def _case(fam, S, B, inn, out, flags, **kw):
@@ -163,8 +152,7 @@ def _case(fam, S, B, inn, out, flags, **kw):
         ks = list(FAMILIES[fam][1])
         if entry in ('bwd', 'lr_bwd'):
             if flags & F_NO_DX:
-                ks = [k for k in ks if k not in DGRAD_KERNELS and not (fam in ('wide_bwd', 'big_bwd') and
-                                                                       k in ('wide_kernel', 'big_kernel'))]
+                ks = [k for k in ks if k not in DGRAD_KERNELS and not (fam == 'wide_bwd' and k == 'wide_kernel')]
             if flags & F_NO_WGRAD:
                 ks = [k for k in ks if k not in WGRAD_KERNELS]
         c['kernels'] = ks
@@ -199,10 +187,10 @@ def _fwd_cases():
     cs += [_case('sk_fwd', 2, 100, 96, 40, SL | TF | F_RELU_IN, prior=GAUSS, inject=True),
            _case('sk_fwd', 2, 100, 96, 40, TF, tag='mean'), _case('sk_fwd', 2, 100, 96, 40, SL | TF, xshared=True)]
     # large batch: TF32, B >= 384, in, out >= 32 (ragged batch tiles, RELU_OUT, log-probs counted once per tile)
-    for fam in ('wide_fwd', 'big_fwd'):
-        cs += [_case(fam, 2, 384, 64, 33, SL | TF), _case(fam, 1, 513, 96, 129, SL | TF | F_RELU_OUT, layer=1),
-               _case(fam, 3, 1030, 36, 129, SL | TF | F_RELU_IN, prior=GAUSS, sample_base=7),
-               _case(fam, 2, 513, 64, 48, TF | F_RELU_OUT, tag='mean'), _case(fam, 2, 600, 64, 64, SL | TF, inject=True)]
+    fam = 'wide_fwd'
+    cs += [_case(fam, 2, 384, 64, 33, SL | TF), _case(fam, 1, 513, 96, 129, SL | TF | F_RELU_OUT, layer=1),
+           _case(fam, 3, 1030, 36, 129, SL | TF | F_RELU_IN, prior=GAUSS, sample_base=7),
+           _case(fam, 2, 513, 64, 48, TF | F_RELU_OUT, tag='mean'), _case(fam, 2, 600, 64, 64, SL | TF, inject=True)]
     # batch-tiled TF32 forward: 128 < B < 384, or B >= 384 with out 17-31
     cs += [_case('tc_fwd', 2, 129, 64, 40, SL | TF), _case('tc_fwd', 3, 383, 36, 33, SL | TF | F_RELU_IN, layer=3),
            _case('tc_fwd', 2, 512, 64, 20, SL | TF, prior=GAUSS), _case('tc_fwd', 2, 200, 64, 40, TF, tag='mean')]
@@ -244,14 +232,14 @@ def _bwd_cases():
     cs += [_case('fused_bwd', 3, 128, 64, 129, F_SAMPLE | TF, mask=True, gp=0.3, gq=0.7),
            _case('fused_bwd', 2, 64, 36, 33, F_SAMPLE | TF | F_OUT_ZEROED, gp=0.3, gq=0.7, inject=True),
            _case('fused_bwd', 1, 7, 400, 20, F_SAMPLE | TF | F_ACCUM, mask=True, gp=0.3, gq=0.7)]
-    for fam in ('wide_bwd', 'big_bwd'):
-        m = _bwd_matrix(fam, 3, 512, 64, 96, F_SAMPLE | TF, layer=1, sample_base=6)
-        cs += [c for c in m if not (c['flags'] & F_DX_PREACT and not c['flags'] & F_RELU_IN)]
-        split_ks = FAMILIES[fam][1] + ['wgrad_combine_kernel']
-        cs += [_case(fam, 3, 512, 64, 96, F_SAMPLE | TF, gp=0.3, gq=0.7, split=1, kernels=split_ks),
-               _case(fam, 4, 600, 64, 96, F_SAMPLE | TF | F_ACCUM, gp=0.3, gq=0.7, split=1, kernels=split_ks),
-               _case(fam, 3, 512, 64, 96, F_SAMPLE | TF | F_ACCUM, gp=0.3, gq=0.7, split=-1),
-               _case(fam, 2, 1030, 36, 132, F_SAMPLE | TF | F_RELU_IN | F_DX_PREACT, gp=0.3, gq=0.7, inject=True)]
+    fam = 'wide_bwd'
+    m = _bwd_matrix(fam, 3, 512, 64, 96, F_SAMPLE | TF, layer=1, sample_base=6)
+    cs += [c for c in m if not (c['flags'] & F_DX_PREACT and not c['flags'] & F_RELU_IN)]
+    split_ks = FAMILIES[fam][1] + ['wgrad_combine_kernel']
+    cs += [_case(fam, 3, 512, 64, 96, F_SAMPLE | TF, gp=0.3, gq=0.7, split=1, kernels=split_ks),
+           _case(fam, 4, 600, 64, 96, F_SAMPLE | TF | F_ACCUM, gp=0.3, gq=0.7, split=1, kernels=split_ks),
+           _case(fam, 3, 512, 64, 96, F_SAMPLE | TF | F_ACCUM, gp=0.3, gq=0.7, split=-1),
+           _case(fam, 2, 1030, 36, 132, F_SAMPLE | TF | F_RELU_IN | F_DX_PREACT, gp=0.3, gq=0.7, inject=True)]
     # the large-batch dgrad / wgrad do not take a dy mask: a masked call goes to the batch-tiled kernels
     cs += [_case('tc_bwd', 2, 600, 64, 96, F_SAMPLE | TF, mask=True, gp=0.3, gq=0.7, tag='reroute'),
            _case('tc_bwd', 2, 600, 64, 96, F_SAMPLE | TF | F_ACCUM, mask=True, gp=0.3, gq=0.7, tag='reroute'),
@@ -392,8 +380,9 @@ def test_kernel_name_matching_is_exact():
              'void bbb::(anonymous namespace)::lr_wgrad_tc_kernel(bbb::LrArgs, float const*, int)',
              '_ZN3bbb12_GLOBAL__N_116lr_narrow_fwd_kernelEN3bbb6LrArgsEi']
     assert _matched(names) == {'lr_fwd_sk_kernel', 'lr_wgrad_tc_kernel', 'lr_narrow_fwd_kernel'}
-    assert _matched(['void bbb::fwd_sk_kernel<32, 2>(bbb::LinArgs)', '_ZN3bbb10big_kernelILb0ELb1EEEvNS_7LinArgsE']) == \
-        {'fwd_sk_kernel', 'big_kernel'}
+    assert _matched(['void bbb::fwd_sk_kernel<32, 2>(bbb::LinArgs)',
+                     '_ZN3bbb16big_wgrad_kernelILb1EEEv14CUtensorMap_stS1_NS_7LinArgsENS_9WgradPartE']) == \
+        {'fwd_sk_kernel', 'big_wgrad_kernel'}
 
 
 def test_tf32_rounding_helpers_on_bit_patterns():
@@ -1023,25 +1012,7 @@ def _run_lr(c):
 @pytest.mark.gpu
 @pytest.mark.parametrize('c', CASES, ids=_cid)
 def test_layer_call_matches_double(c):
-    if c['fam'] in ('big_fwd', 'big_bwd') and not NO_WIDE:
-        pytest.skip('first-generation large-batch kernels: run by test_large_batch_first_generation (BBB_NO_WIDE=1)')
-    if NO_WIDE and c['fam'] not in ('big_fwd', 'big_bwd'):
-        pytest.skip('BBB_NO_WIDE=1 child: only the first-generation large-batch cases')
     {'fwd': _run_fwd, 'bwd': _run_bwd, 'lr_fwd': _run_lr, 'lr_bwd': _run_lr}[c['entry']](c)
-
-
-@pytest.mark.gpu
-def test_large_batch_first_generation():
-    """BBB_NO_WIDE=1 is read once per process: the big_kernel cases run in a child pytest with it set"""
-    if NO_WIDE:
-        pytest.skip('already the child')
-    env = dict(os.environ, BBB_NO_WIDE='1')
-    r = subprocess.run([sys.executable, '-m', 'pytest', '-q', '-s', '-p', 'no:cacheprovider', '-m', 'gpu',
-                        os.path.abspath(__file__), '-k', 'big_fwd or big_bwd'], cwd=ROOT, env=env, capture_output=True,
-                       text=True, timeout=1200)
-    print(r.stdout[-20000:])
-    assert r.returncode == 0, r.stdout[-5000:] + r.stderr[-5000:]
-    assert ' passed' in r.stdout and ' failed' not in r.stdout
 
 
 @pytest.mark.parametrize('fam', sorted(TF32_ROUNDING))
@@ -1092,7 +1063,7 @@ def test_tf32_emulation_without_rounding_is_the_double(fam, monkeypatch):
 
 
 @pytest.mark.gpu
-def test_network_backward_accum_adds_what_it_otherwise_writes():
+def test_network_level_backward_accum_adds_what_it_otherwise_writes():
     """bbb_mlp_bwd with BBB_F_ACCUM (kept for every layer, bbb_mlp.cu) adds into G0 exactly the gradients the same call
     writes without it: same forward state, eps and rng.  The hidden layers' dz are summed with red.add in an order that
     is not fixed, so the two calls may differ by fp32 round-off of those sums; beyond that the bound is one rounding of
@@ -1116,10 +1087,10 @@ def test_network_backward_accum_adds_what_it_otherwise_writes():
     def backward(flags, grads):
         for dz in dxs[1:nl]:
             dz.zero_()                    # the layer above adds (dz W) (y > 0) into the hidden dz buffers
-        tab = F._mlp_layer_table(params, eps, ys, list(dxs[1:nl]) + [d_out], grads, dxs[nl])
+        tab = F._mlp_layer_table(params, eps, ys, list(dxs[1:nl]) + [d_out], grads)
         rng = eps.rng(0)
         rc, ran = _profiled(lambda: L.lib().bbb_mlp_bwd(tab, nl, L.ptr(x), S, B, C.byref(rng), C.byref(prior), flags,
-                                                        -0.3 / S, 0.3 / S, None, None, 0, L.ptr(scale), None, L.stream()))
+                                                        -0.3 / S, 0.3 / S, None, None, 0, L.ptr(scale), L.stream()))
         assert rc == 0, L.lib().bbb_last_error_string()
         return ran
 
