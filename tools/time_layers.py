@@ -1,6 +1,9 @@
 #!/usr/bin/env python
-"""Warm and cold (L2-flushed) CUDA-event timings of the layer kernels through the C ABI, one shape at a time.
-usage: python tools/time_layers.py [B S]"""
+"""Warm and cold (L2-flushed) CUDA-event timings of the layer kernels through the C ABI, one layer at a time, with the
+flags the per-layer host path (functional._net_ws_forward / _net_ws_backward) passes in TF32 mode.
+usage: python tools/time_layers.py [B S [d0 d1 ... dn]]
+The widths d0 .. dn name a network (default: the MNIST shape 784 1200 1200 10); its first layer reads the shared network
+input and hands no dx down, the others read the stored pre-activation of the layer below.  BBB_LIB selects the library."""
 import ctypes as C
 import os
 import sys
@@ -13,6 +16,7 @@ from bnn_b200 import _lib as L, functional as F  # noqa: E402
 
 B = int(sys.argv[1]) if len(sys.argv) > 1 else 128
 S = int(sys.argv[2]) if len(sys.argv) > 2 else 2
+dims = [int(d) for d in sys.argv[3:]] or [784, 1200, 1200, 10]
 dev = 'cuda'
 prior = F.make_prior([0.5, 0, -8], True)
 flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
@@ -33,7 +37,8 @@ def timeit(fn, n=30, cold=False):
     return ts[len(ts) // 2]
 
 
-for inn, out, first, last in ((784, 1200, True, False), (1200, 1200, False, False), (1200, 10, False, True)):
+for l, (inn, out) in enumerate(zip(dims[:-1], dims[1:])):
+    first = l == 0
     torch.manual_seed(0)
     wm = torch.empty(out, inn, device=dev).uniform_(-0.2, 0.2); wr = torch.empty(out, inn, device=dev).uniform_(-5, -4)
     bm = torch.empty(out, device=dev).uniform_(-0.2, 0.2); br = torch.empty(out, device=dev).uniform_(-5, -4)
@@ -62,7 +67,6 @@ for inn, out, first, last in ((784, 1200, True, False), (1200, 1200, False, Fals
     print(f'[{inn}x{out}] B={B} S={S}  fwd warm {timeit(fwd):6.1f} us  cold {timeit(fwd, cold=True):6.1f} us   '
           f'bwd warm {timeit(bwd):6.1f} us  cold {timeit(bwd, cold=True):6.1f} us', flush=True)
 
-def empty():
-    L.check(L.lib().bbb_counter_add(acc.data_ptr(), 0, st), 'x')
 cnt = torch.zeros(1, dtype=torch.int32, device=dev)
+st = torch.cuda.current_stream().cuda_stream
 print('tiny kernel (launch floor, events around one launch):', timeit(lambda: L.lib().bbb_counter_add(cnt.data_ptr(), 0, st)), 'us')
