@@ -12,7 +12,7 @@ LIB_PATH = os.environ.get('BBB_LIB') or os.path.join(_HERE, 'libbbb.so')   # BBB
 F_SAMPLE, F_LOGPROB, F_RELU_IN, F_ACCUM, F_TF32, F_NO_DX, F_SCALE_DX, F_NO_WGRAD = 1, 2, 4, 8, 16, 32, 64, 128
 F_OUT_ZEROED, F_DX_PREACT, F_RELU_OUT = 256, 512, 1024
 PRIOR_GAUSSIAN, PRIOR_MIXTURE = 0, 1
-NLL_NONE, NLL_CE, NLL_GAUSS = 0, 1, 2
+NLL_NONE, NLL_CE, NLL_GAUSS, NLL_GAUSS_HET = 0, 1, 2, 3
 
 
 class Rng(C.Structure):
@@ -59,6 +59,7 @@ _SIGS = {
     'bbb_predictive_stats': ([P, P, I64, I64, I64, I32, F32, I32, P, P, P, P, P], C.c_int),
     'bbb_nll_ce': ([P, P, I64, I64, I64, F32, P, P, P], C.c_int),
     'bbb_nll_gauss': ([P, P, F32, I64, I64, I64, F32, P, P, P], C.c_int),
+    'bbb_nll_gauss_het': ([P, P, F32, I64, I64, I64, F32, P, P, P], C.c_int),
     'bbb_head_fwd': ([P, I64, P, P, P, P, P, P, P, P, I64, I64, I64, I64, I32, I32, P, F32, F32, P, P, P, P, P, F32,
                       P, P, P, P], C.c_int),
     'bbb_mlp_supported': ([P, I32, I64, I64, I32], C.c_int),

@@ -253,6 +253,96 @@ __global__ void __launch_bounds__(PT) predictive_gauss_kernel(const float *__res
   block_add(w_sq, red, acc + A_SQERR);
 }
 
+// ---- heteroscedastic Gaussian: the mixture (1/S) sum_s N(f_s, sigma_s^2), row = [f (D) | r (D)] -------------------------
+// sigma_s = sigma_min + softplus(r_s).  Welford over f (epistemic), a running sum of sigma_s^2 (aleatoric), online LSE of
+// sum_d log N(y_d; f_s,d, sigma_s,d^2) (log predictive density).  The explicit minimum of one block per SM keeps ptxas
+// from capping the NPL = 4 instance at 64 registers, where it spilled.
+template <int NPL>
+__global__ void __launch_bounds__(PT, 1) predictive_gauss_het_kernel(const float *__restrict__ out,
+                                                                   const float *__restrict__ target, int64_t S,
+                                                                   int64_t B, int64_t D, float sigma_min,
+                                                                   float *__restrict__ mean,
+                                                                   float *__restrict__ row_stats, double *acc) {
+  __shared__ float red[kWarps];
+  const bool agg = target != nullptr && acc != nullptr;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const float log_s = logf((float)S), half_log_2pi = 0.918938533204672741780329736406f;
+  float w_n = 0.0f, w_nll = 0.0f, w_sq = 0.0f;
+  for (int64_t b = (int64_t)blockIdx.x * kWarps + warp; b < B; b += (int64_t)gridDim.x * kWarps) {
+    float yv[NPL], mu[NPL], m2[NPL], var[NPL], fc[NPL], rc[NPL], fn[NPL], rn[NPL];
+    if (target) load_row<NPL>(target + b * D, D, lane, yv);
+#pragma unroll
+    for (int j = 0; j < NPL; ++j) { mu[j] = 0.0f; m2[j] = 0.0f; var[j] = 0.0f; }
+    float lp_max = -INFINITY, lp_sum = 0.0f;
+    load_row<NPL>(out + b * 2 * D, D, lane, fc);
+    load_row<NPL>(out + b * 2 * D + D, D, lane, rc);
+    for (int64_t s = 0; s < S; ++s) {
+      if (s + 1 < S) {
+        const float *z = out + ((s + 1) * B + b) * 2 * D;
+        load_row<NPL>(z, D, lane, fn);
+        load_row<NPL>(z + D, D, lane, rn);
+      }
+      const float inv_n = 1.0f / (float)(s + 1);
+      float ll = 0.0f;
+#pragma unroll
+      for (int j = 0; j < NPL; ++j) {
+        const float d = fc[j] - mu[j];
+        mu[j] += d * inv_n;
+        m2[j] += d * (fc[j] - mu[j]);
+        const float sigma = sigma_min + fmaxf(rc[j], 0.0f) + log1pf(expf(-fabsf(rc[j])));
+        var[j] += sigma * sigma;
+        if (target && lane + 32 * j < D) {
+          const float a = (yv[j] - fc[j]) / sigma;
+          ll -= fmaf(0.5f * a, a, logf(sigma) + half_log_2pi);
+        }
+      }
+      if (target) {
+        const float l = warp_sum(ll);
+        const float m = fmaxf(lp_max, l);
+        lp_sum = lp_sum * expf(lp_max - m) + expf(l - m);
+        lp_max = m;
+      }
+#pragma unroll
+      for (int j = 0; j < NPL; ++j) { fc[j] = fn[j]; rc[j] = rn[j]; }
+    }
+    const float inv_s = 1.0f / (float)S;
+    float sqerr = 0.0f;
+    float *rs = row_stats + b * (2 * D + 1);
+#pragma unroll
+    for (int j = 0; j < NPL; ++j) {
+      const int64_t d = lane + 32 * j;
+      if (d < D) {
+        mean[b * D + d] = mu[j];
+        rs[d] = m2[j] * inv_s;
+        rs[D + d] = var[j] * inv_s;
+        if (target) { const float r = mu[j] - yv[j]; sqerr += r * r; }
+      }
+    }
+    sqerr = warp_sum(sqerr);
+    if (lane == 0) {
+      const float log_pred = target ? lp_max + logf(lp_sum) - log_s : __int_as_float(0x7fc00000);
+      rs[2 * D] = log_pred;
+      w_n += 1.0f;
+      w_nll -= log_pred;
+      w_sq += sqerr;
+    }
+  }
+  if (!agg) return;
+  block_add(w_n, red, acc + A_N);
+  block_add(w_nll, red, acc + A_NLL);
+  block_add(w_sq, red, acc + A_SQERR);
+}
+
+template <int NPL>
+cudaError_t launch_het(const float *out, const float *target, int64_t S, int64_t B, int64_t D, float sigma_min,
+                       float *mean, float *row_stats, double *acc, cudaStream_t st) {
+  const int64_t blocks = (B + kWarps - 1) / kWarps;
+  const int64_t cap = (int64_t)sm_count() * (2048 / PT);   // one resident wave
+  predictive_gauss_het_kernel<NPL><<<(int)(blocks < cap ? blocks : cap), PT, 0, st>>>(out, target, S, B, D, sigma_min,
+                                                                                      mean, row_stats, acc);
+  return cudaGetLastError();
+}
+
 template <int NPL>
 cudaError_t launch_stats(const float *out, const void *target, int64_t S, int64_t B, int64_t C, int32_t kind,
                          float sigma, int n_bins, float *mean, float *row_stats, int64_t *pred, double *acc,
@@ -279,9 +369,33 @@ cudaError_t launch_stats(const float *out, const void *target, int64_t S, int64_
 
 using namespace bbb;
 
+// kind BBB_NLL_GAUSS_HET of bbb_predictive_stats: C = 2D outputs per row, sigma = sigma_min
+static int predictive_stats_het(const float *out, const float *target, int64_t S, int64_t B, int64_t C,
+                                float sigma_min, float *mean, float *row_stats, double *acc, cudaStream_t st) {
+  BBB_CHECK_ARG(S >= 1 && B >= 0 && C >= 2 && C % 2 == 0, "bad shape (need S >= 1, B >= 0, C = 2D >= 2)");
+  BBB_CHECK_ARG(C <= 32 * 32, "more than 1024 outputs per row");
+  BBB_CHECK_ARG(sigma_min > 0.0f, "sigma_min must be > 0");
+  BBB_CHECK_ARG(!target || acc, "aggregates (acc) required with a target");
+  BBB_CHECK_ARG(B == 0 || (out && mean && row_stats), "null pointer");
+  if (B == 0) return BBB_OK;
+  const int64_t D = C / 2;
+  cudaError_t e;
+  if (D <= 32) e = launch_het<1>(out, target, S, B, D, sigma_min, mean, row_stats, acc, st);
+  else if (D <= 64) e = launch_het<2>(out, target, S, B, D, sigma_min, mean, row_stats, acc, st);
+  else if (D <= 128) e = launch_het<4>(out, target, S, B, D, sigma_min, mean, row_stats, acc, st);
+  else if (D <= 256) e = launch_het<8>(out, target, S, B, D, sigma_min, mean, row_stats, acc, st);
+  else e = launch_het<16>(out, target, S, B, D, sigma_min, mean, row_stats, acc, st);
+  BBB_CHECK_CUDA(e);
+  BBB_CHECK_LAUNCH();
+  return BBB_OK;
+}
+
 extern "C" int bbb_predictive_stats(const float *out, const void *target, int64_t S, int64_t B, int64_t C,
                                     int32_t kind, float sigma, int32_t n_bins, float *mean, float *row_stats,
                                     int64_t *pred, double *acc, void *stream) {
+  if (kind == BBB_NLL_GAUSS_HET)
+    return predictive_stats_het(out, static_cast<const float *>(target), S, B, C, sigma, mean, row_stats, acc,
+                                (cudaStream_t)stream);
   BBB_CHECK_ARG(kind == BBB_NLL_CE || kind == BBB_NLL_GAUSS, "kind must be BBB_NLL_CE or BBB_NLL_GAUSS");
   BBB_CHECK_ARG(S >= 1 && B >= 0 && C >= 1, "bad shape (need S >= 1, B >= 0, C >= 1)");
   BBB_CHECK_ARG(C <= 32 * 32, "more than 1024 classes / outputs per row");

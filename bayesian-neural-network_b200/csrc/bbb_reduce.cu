@@ -161,6 +161,35 @@ __global__ void __launch_bounds__(RT) nll_gauss_kernel(const float *__restrict__
   block_sum2_atomic(acc, 0.0f, red, nll, nullptr);
 }
 
+// Heteroscedastic Gaussian: row (s, b) of `out` is [f (D) | r (D)], sigma = sigma_min + softplus(r).  One thread per
+// (s, b, d).  With a = (y - f) / sigma every term is formed from a and 1 / sigma, never from sigma^2 or sigma^3, so the
+// value and both gradients stay finite for r in [-40, 40] and residuals of 1e3 down to sigma_min ~ 1e-6.
+__global__ void __launch_bounds__(RT) nll_gauss_het_kernel(const float *__restrict__ out,
+                                                           const float *__restrict__ target, float sigma_min,
+                                                           float cst, int64_t n, int64_t B, int64_t D,
+                                                           float grad_scale, double *nll, float *__restrict__ dout) {
+  pdl_launch_dependents();
+  pdl_wait();
+  __shared__ float red[64];
+  float acc = 0.0f;
+  for (int64_t i = (int64_t)blockIdx.x * RT + threadIdx.x; i < n; i += (int64_t)gridDim.x * RT) {
+    const int64_t row = i / D, d = i - row * D;
+    const int64_t o = row * 2 * D + d;
+    const float f = out[o], r = out[o + D];
+    const float e = expf(-fabsf(r));
+    const float sg = fmaxf(r, 0.0f) + log1pf(e);                  // softplus(r), stable for either sign
+    const float sig = r >= 0.0f ? 1.0f / (1.0f + e) : e / (1.0f + e);   // sigmoid(r) = d softplus / dr
+    const float sigma = sigma_min + sg, inv_s = 1.0f / sigma;
+    const float a = (target[(row % B) * D + d] - f) * inv_s;
+    acc += fmaf(0.5f * a, a, logf(sigma) + cst);
+    if (dout) {
+      dout[o] = -grad_scale * a * inv_s;                             // g (f - y) / sigma^2
+      dout[o + D] = grad_scale * sig * inv_s * fmaf(-a, a, 1.0f);    // g sigmoid(r) (1/sigma - (y - f)^2 / sigma^3)
+    }
+  }
+  block_sum2_atomic(acc, 0.0f, red, nll, nullptr);
+}
+
 __global__ void elbo_finalize_kernel(const double *logp, const double *logq, const double *kl, const double *nll,
                                      int S, float beta, const float *beta_dev, float *out4) {
   pdl_launch_dependents();
@@ -308,6 +337,20 @@ extern "C" int bbb_nll_gauss(const float *out, const float *target, float sigma,
   BBB_CHECK_CUDA(launch_pdl(nll_gauss_kernel, dim3(grid_for(n, RT)), dim3(RT), 0, (cudaStream_t)stream, out, target,
                             (float)(0.5 / var), (float)(1.0 / var),
                             (float)(log((double)sigma) + 0.918938533204672741780329736406), n, B * D, grad_scale, nll, dout));
+  BBB_CHECK_LAUNCH();
+  return BBB_OK;
+}
+
+extern "C" int bbb_nll_gauss_het(const float *out, const float *target, float sigma_min, int64_t S, int64_t B,
+                                 int64_t D, float grad_scale, double *nll, float *dout, void *stream) {
+  BBB_CHECK_ARG(out && target && nll, "null pointer");
+  BBB_CHECK_ARG(S >= 0 && B >= 0 && D >= 0, "negative size");
+  BBB_CHECK_ARG(D > 0 || S * B == 0, "D == 0 with S * B > 0");
+  BBB_CHECK_ARG(sigma_min > 0.0f, "sigma_min must be > 0");
+  const int64_t n = S * B * D;
+  if (n == 0) return BBB_OK;
+  BBB_CHECK_CUDA(launch_pdl(nll_gauss_het_kernel, dim3(grid_for(n, RT)), dim3(RT), 0, (cudaStream_t)stream, out, target,
+                            sigma_min, (float)0.918938533204672741780329736406, n, B, D, grad_scale, nll, dout));
   BBB_CHECK_LAUNCH();
   return BBB_OK;
 }

@@ -393,9 +393,27 @@ def mlp_forward(x2, layers, prior, S, sample=True, logprob=True, tf32=False):
 use_network_level_call = True
 
 
-def _layerwise_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, need_grad, tf32, beta_h, beta_d, out4):
+def _nll_launch(out, target, S, B, Cc, sigma, mode, likelihood, nll, d_out):
+    """The likelihood and its gradient (scaled by 1/S) on the sampled outputs [S,B,Cc]: nll += ..., d_out written.
+    The heteroscedastic likelihood reads `sigma` as sigma_min and Cc = 2D outputs per row."""
+    if likelihood == 'heteroscedastic':
+        tgt = _f32c(target)            # (held: a contiguous copy must outlive the call)
+        L.check(L.lib().bbb_nll_gauss_het(L.ptr(out), L.ptr(tgt), float(sigma), S, B, Cc // 2, 1.0 / S, L.ptr(nll),
+                                          L.ptr(d_out), L.stream()), 'bbb_nll_gauss_het')
+    elif mode == 'classification':
+        L.check(L.lib().bbb_nll_ce(L.ptr(out), L.ptr(target), S, B, Cc, 1.0 / S, L.ptr(nll), L.ptr(d_out),
+                                   L.stream()), 'bbb_nll_ce')
+    else:
+        tgt = _f32c(target)
+        L.check(L.lib().bbb_nll_gauss(L.ptr(out), L.ptr(tgt), float(sigma), S, B, Cc, 1.0 / S, L.ptr(nll),
+                                      L.ptr(d_out), L.stream()), 'bbb_nll_gauss')
+
+
+def _layerwise_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, need_grad, tf32, beta_h, beta_d, out4,
+                            likelihood='gaussian'):
     """sample_elbo's forward as one launch per layer (+ the fused head): every shape, both modes.  Returns
-    (ys: per-layer PRE-activation outputs, dxs: the backward's zero-filled dx workspace, d_out)."""
+    (ys: per-layer PRE-activation outputs, dxs: the backward's zero-filled dx workspace, d_out).  The heteroscedastic
+    likelihood has no fused head: its last layer is a plain layer call, then bbb_nll_gauss_het."""
     dev = x2.device
     # ONE zero-filled workspace (one memset per step): fp64 accumulators + the head's completion counter |
     # activations of every layer | dx of every layer above the first (the backward's split-K kernels add into them)
@@ -412,7 +430,7 @@ def _layerwise_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, n
     logp, logq, nll = acc[:S], acc[S:2 * S], acc[2 * S:]
     Cc = params[-1][0].shape[0]
     d_out = torch.empty((S, B, Cc), dtype=torch.float32, device=dev) if need_grad else None
-    if head_eligible(params[-1]):
+    if likelihood == 'gaussian' and head_eligible(params[-1]):
         # the last layer, the likelihood with its gradient and the assembly of the four scalars: one launch
         tgt = target if mode == 'classification' else _f32c(target)
         nl = len(params) - 1
@@ -423,14 +441,7 @@ def _layerwise_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, n
         ys = _net_ws_forward(x2, params, prior, S, eps, True, True, tf32, logp, logq, ys, head)
     else:
         ys = _net_ws_forward(x2, params, prior, S, eps, True, True, tf32, logp, logq, ys)
-        out = ys[-1]
-        if mode == 'classification':
-            L.check(L.lib().bbb_nll_ce(L.ptr(out), L.ptr(target), S, B, Cc, 1.0 / S, L.ptr(nll), L.ptr(d_out),
-                                       L.stream()), 'bbb_nll_ce')
-        else:
-            tgt = _f32c(target)
-            L.check(L.lib().bbb_nll_gauss(L.ptr(out), L.ptr(tgt), float(sigma), S, B, Cc, 1.0 / S, L.ptr(nll),
-                                          L.ptr(d_out), L.stream()), 'bbb_nll_gauss')
+        _nll_launch(ys[-1], target, S, B, Cc, sigma, mode, likelihood, nll, d_out)
         L.check(L.lib().bbb_elbo_finalize(L.ptr(logp), L.ptr(logq), None, L.ptr(nll), S, beta_h, L.ptr(beta_d),
                                           L.ptr(out4), L.stream()), 'bbb_elbo_finalize')
     return ys, dxs, d_out
@@ -484,10 +495,11 @@ def _mlp_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, need_gr
 class _FusedELBO(torch.autograd.Function):
     """sample_elbo (networks.py:192-209).  TF32 mode, batch <= 128: ONE C call per pass (bbb_mlp_fwd: a TMA-fed tcgen05
     kernel per hidden layer + the fused head; bbb_mlp_bwd: head + one fused wgrad/dgrad kernel per layer).  Otherwise one
-    launch per layer (+ likelihood + assembly).  Only `loss` is differentiable."""
+    launch per layer (+ likelihood + assembly).  Only `loss` is differentiable.  likelihood 'heteroscedastic' (sigma is
+    then sigma_min) always takes the per-layer calls: neither network-level call implements it."""
 
     @staticmethod
-    def forward(ctx, x2, target, beta, S, sigma, mode, prior, tf32, *flat):
+    def forward(ctx, x2, target, beta, S, sigma, mode, likelihood, prior, tf32, *flat):
         L.require_cuda(x2, target, *flat)
         x2 = _f32c(x2)
         dev = x2.device
@@ -499,14 +511,14 @@ class _FusedELBO(torch.autograd.Function):
         out4 = torch.empty(4, dtype=torch.float32, device=dev)
         beta_h, beta_d = _split_beta(beta)
         dims = [params[0][0].shape[1]] + [p[0].shape[0] for p in params]
-        use_mlp = (use_network_level_call and tf32 and mode in ('classification', 'regression') and
-                   L.mlp_supported(dims, S, B, L.F_TF32))
+        use_mlp = (likelihood == 'gaussian' and use_network_level_call and tf32 and
+                   mode in ('classification', 'regression') and L.mlp_supported(dims, S, B, L.F_TF32))
         if use_mlp:
             ys, dxs, d_out = _mlp_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, need_grad, beta_h,
                                                beta_d, out4)
         else:
             ys, dxs, d_out = _layerwise_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, need_grad, tf32,
-                                                     beta_h, beta_d, out4)
+                                                     beta_h, beta_d, out4, likelihood)
         if need_grad:
             ctx.save_for_backward(x2, d_out, *flat, *ys[:-1], *eps.tensors())
             ctx.dxs = dxs
@@ -522,7 +534,7 @@ class _FusedELBO(torch.autograd.Function):
     def backward(ctx, g_loss, *unused):
         prior, S, beta, tf32, eps, nl = ctx.cfg
         if g_loss is None:
-            return (None,) * (8 + 4 * nl)
+            return (None,) * (9 + 4 * nl)
         if getattr(ctx, 'consumed', False):
             # the split-K backward kernels ADD into the dx workspace zero-filled by the forward (BBB_F_OUT_ZEROED)
             raise RuntimeError('sample_elbo: this graph was already differentiated (retain_graph=True is not '
@@ -552,12 +564,12 @@ class _FusedELBO(torch.autograd.Function):
             _, grads = _net_ws_backward(x2, ys, d_out, params, prior, S, eps, True, tf32, -beta / S, beta / S,
                                         bd, bd, 0, scale, False, dxs=ctx.dxs)
         flat = [g for lg in grads for g in lg]
-        return (None,) * 8 + tuple(flat)
+        return (None,) * 9 + tuple(flat)
 
 
-def fused_elbo(x2, target, beta, S, sigma, mode, prior, layers, tf32=False):
+def fused_elbo(x2, target, beta, S, sigma, mode, prior, layers, tf32=False, likelihood='gaussian'):
     flat = [t for layer in layers for t in layer]
-    return _FusedELBO.apply(x2, target, beta, S, sigma, mode, prior, tf32, *flat)
+    return _FusedELBO.apply(x2, target, beta, S, sigma, mode, likelihood, prior, tf32, *flat)
 
 
 # =========================================================================================
@@ -729,10 +741,11 @@ def mlp_forward_lr(x2, layers, sigma_p, S, sample=True, calc_kl=True, tf32=False
 
 
 class _FusedELBOLR(torch.autograd.Function):
-    """sample_elbo_lr (networks.py:211-225): loss = beta * KL + NLL / S, KL evaluated once."""
+    """sample_elbo_lr (networks.py:211-225): loss = beta * KL + NLL / S, KL evaluated once.  likelihood as in
+    _FusedELBO."""
 
     @staticmethod
-    def forward(ctx, x2, target, beta, S, sigma, mode, sigma_p, tf32, *flat):
+    def forward(ctx, x2, target, beta, S, sigma, mode, likelihood, sigma_p, tf32, *flat):
         L.require_cuda(x2, target, *flat)
         x2 = _f32c(x2)
         dev = x2.device
@@ -745,13 +758,7 @@ class _FusedELBOLR(torch.autograd.Function):
         B, Cc = out.shape[1], out.shape[2]
         need_grad = any(t.requires_grad for t in flat)
         d_out = torch.empty_like(out) if need_grad else None
-        if mode == 'classification':
-            L.check(L.lib().bbb_nll_ce(L.ptr(out), L.ptr(target), S, B, Cc, 1.0 / S, L.ptr(nll), L.ptr(d_out),
-                                       L.stream()), 'bbb_nll_ce')
-        else:
-            tgt = _f32c(target)
-            L.check(L.lib().bbb_nll_gauss(L.ptr(out), L.ptr(tgt), float(sigma), S, B, Cc, 1.0 / S, L.ptr(nll),
-                                          L.ptr(d_out), L.stream()), 'bbb_nll_gauss')
+        _nll_launch(out, target, S, B, Cc, sigma, mode, likelihood, nll, d_out)
         out4 = torch.empty(4, dtype=torch.float32, device=dev)
         beta_h, beta_d = _split_beta(beta)
         L.check(L.lib().bbb_elbo_finalize(None, None, L.ptr(kl), L.ptr(nll), S, beta_h, L.ptr(beta_d), L.ptr(out4),
@@ -770,7 +777,7 @@ class _FusedELBOLR(torch.autograd.Function):
     def backward(ctx, g_loss, *unused):
         sigma_p, S, beta, eps, nl = ctx.cfg
         if g_loss is None:
-            return (None,) * (8 + 4 * nl)
+            return (None,) * (9 + 4 * nl)
         if ctx.tf32 and getattr(ctx, 'consumed', False):
             # the tcgen05 LR backward overwrites the saved delta buffers with dV (they have no other use in it)
             raise RuntimeError('sample_elbo_lr: this graph was already differentiated (retain_graph=True is not supported '
@@ -786,12 +793,12 @@ class _FusedELBOLR(torch.autograd.Function):
         _, grads = _net_lr_backward(x2, ys, deltas, d_out, params, sigma_p, S, eps, True, True, beta, ctx.beta_dev,
                                     scale, False, ctx.tf32)
         flat = [g for lg in grads for g in lg]
-        return (None,) * 8 + tuple(flat)
+        return (None,) * 9 + tuple(flat)
 
 
-def fused_elbo_lr(x2, target, beta, S, sigma, mode, sigma_p, layers, tf32=False):
+def fused_elbo_lr(x2, target, beta, S, sigma, mode, sigma_p, layers, tf32=False, likelihood='gaussian'):
     flat = [t for layer in layers for t in layer]
-    return _FusedELBOLR.apply(x2, target, beta, S, sigma, mode, float(sigma_p), tf32, *flat)
+    return _FusedELBOLR.apply(x2, target, beta, S, sigma, mode, likelihood, float(sigma_p), tf32, *flat)
 
 
 # =========================================================================================
@@ -865,6 +872,13 @@ def softmax_mean(logits):
 # posterior predictive: uncertainty and calibration of the sampled outputs (bbb_predictive_stats)
 # =========================================================================================
 PREDICTIVE_BUDGET_BYTES = 256 << 20      # bound on one chunk's fp32 activations, S * rows * sum of widths * 4 B
+PREDICTIVE_MODES = ('classification', 'regression', 'heteroscedastic')
+_PREDICTIVE_KIND = dict(classification=L.NLL_CE, regression=L.NLL_GAUSS, heteroscedastic=L.NLL_GAUSS_HET)
+
+
+def _check_predictive_mode(mode):
+    if mode not in PREDICTIVE_MODES:
+        raise ValueError(f"mode must be one of {PREDICTIVE_MODES}, got {mode!r}")
 
 
 def predictive_acc_len(mode, n_bins):
@@ -874,17 +888,20 @@ def predictive_acc_len(mode, n_bins):
 
 def _predictive_launch(out, target, mode, sigma, n_bins, mean, row_stats, pred, acc):
     S, B, Cc = out.shape
-    kind = L.NLL_CE if mode == 'classification' else L.NLL_GAUSS
+    kind = _PREDICTIVE_KIND[mode]
     L.check(L.lib().bbb_predictive_stats(L.ptr(out), L.ptr(target), S, B, Cc, kind, float(sigma), int(n_bins),
                                          L.ptr(mean), L.ptr(row_stats), L.ptr(pred), L.ptr(acc), L.stream()),
             'bbb_predictive_stats')
 
 
 def _predictive_target(target, mode, B, Cc):
-    """The target as the kernel reads it, row for row: int64 [B] labels, or float [B, D] ([B] when D = 1)."""
+    """The target as the kernel reads it, row for row: int64 [B] labels, or float [B, D] ([B] when D = 1), where D = Cc
+    except for the heteroscedastic likelihood's Cc = 2D outputs."""
     if target is None:
         return None
     L.require_cuda(target)
+    if mode == 'heteroscedastic':
+        Cc //= 2
     if mode == 'classification':
         if target.dtype != torch.int64 or tuple(target.shape) != (B,):
             raise ValueError(f'classification target must be int64 of shape ({B},), got {target.dtype} '
@@ -898,7 +915,7 @@ def _predictive_target(target, mode, B, Cc):
 
 def _predictive_outputs(B, Cc, mode, n_bins, target, device):
     k = 5 if mode == 'classification' else Cc + 1
-    mean = torch.empty((B, Cc), dtype=torch.float32, device=device)
+    mean = torch.empty((B, Cc // 2 if mode == 'heteroscedastic' else Cc), dtype=torch.float32, device=device)
     row_stats = torch.empty((B, k), dtype=torch.float32, device=device)
     pred = torch.empty(B, dtype=torch.int64, device=device) if mode == 'classification' else None
     acc = torch.zeros(predictive_acc_len(mode, n_bins), dtype=torch.float64, device=device) if target is not None \
@@ -910,12 +927,15 @@ def predictive_stats(out, target=None, mode='classification', sigma=1.0, n_bins=
     """[S,B,C] sampled outputs -> (mean [B,C], row_stats [B,K], pred [B] or None, acc or None), device tensors, one
     launch (bbb_predictive_stats; include/bbb.h gives every definition and the layout of row_stats and acc).
     mode 'classification': the outputs are logits and target int64 [B]; 'regression': a Gaussian likelihood with
-    std `sigma` and target [B,D] ([B] when D = 1).  acc (the aggregates) only with a target."""
-    if mode not in ('classification', 'regression'):
-        raise ValueError(f"mode must be 'classification' or 'regression', got {mode!r}")
+    std `sigma` and target [B,D] ([B] when D = 1); 'heteroscedastic': the outputs are [f | r] (C = 2D), the likelihood
+    N(f, (sigma + softplus(r))^2) with `sigma` as sigma_min, target as 'regression'.  acc (the aggregates) only with a
+    target."""
+    _check_predictive_mode(mode)
     L.require_cuda(out)
     z = _f32c(out)
     S, B, Cc = z.shape
+    if mode == 'heteroscedastic' and Cc % 2:
+        raise ValueError(f'heteroscedastic outputs are [f | r]: an even width, got {Cc}')
     tgt = _predictive_target(target, mode, B, Cc)
     mean, row_stats, pred, acc = _predictive_outputs(B, Cc, mode, n_bins, tgt, z.device)
     _predictive_launch(z, tgt, mode, sigma, n_bins, mean, row_stats, pred, acc)
@@ -942,9 +962,9 @@ def predictive(x2, params, S, mode, target=None, sigma=1.0, n_bins=15, chunk_row
       * local reparameterisation: the noise is per row by construction; each chunk draws its own, which equals calling
         the reference's predict chunk by chunk in order.  The call consumes one Philox step PER CHUNK.
     chunk_rows=None picks the largest row count whose activations, S * rows * sum of layer widths * 4 bytes, stay
-    under PREDICTIVE_BUDGET_BYTES, and splits the rows into chunks of equal size."""
-    if mode not in ('classification', 'regression'):
-        raise ValueError(f"mode must be 'classification' or 'regression', got {mode!r}")
+    under PREDICTIVE_BUDGET_BYTES, and splits the rows into chunks of equal size.
+    mode as in predictive_stats ('heteroscedastic': `sigma` is sigma_min)."""
+    _check_predictive_mode(mode)
     if (prior is None) == (sigma_p is None):
         raise ValueError('give exactly one of prior (weight sampling) and sigma_p (local reparameterisation)')
     L.require_cuda(x2, *[t for p in params for t in p])

@@ -11,6 +11,8 @@ from torch import nn
 from . import functional as F
 from .layers import BayesianLinear, BayesianLinearLR
 
+_HALF_LOG_2PI = 0.5 * math.log(2 * math.pi)
+
 
 @dataclass
 class PredictiveResult:
@@ -20,6 +22,8 @@ class PredictiveResult:
     confidence [B] (mean[pred]), entropy [B] (of mean), expected_entropy [B] (mean over the samples of each softmax's
     entropy: aleatoric), mutual_info [B] (entropy - expected_entropy, clamped at 0: epistemic).
     regression: mean [B,D], variance [B,D] (epistemic, over the samples; total = variance + sigma**2).
+    heteroscedastic regression: also aleatoric_variance [B,D] (the mean over the samples of sigma(x)**2; total =
+    variance + aleatoric_variance).
     log_pred [B]: log predictive density of each row's target (None without a target)."""
     mean: torch.Tensor
     pred: Optional[torch.Tensor] = None
@@ -31,6 +35,7 @@ class PredictiveResult:
     log_pred: Optional[torch.Tensor] = None
     acc: Optional[torch.Tensor] = None       # fp64 aggregates of bbb_predictive_stats (include/bbb.h)
     n_bins: int = 0
+    aleatoric_variance: Optional[torch.Tensor] = None
 
     def metrics(self):
         """The aggregates as python numbers; the one host read of a prediction.  Classification: dict(n, accuracy,
@@ -63,6 +68,11 @@ class BayesianNetwork(nn.Module):
     reinforcement_learning/bandits.py construct the net (SURVEY App. B-1); 'hidden_units' may be a list
     (or 'n_hidden' may be given) for nets deeper than the reference's fixed two hidden layers
     (BASELINE.json config 5); 'tf32' opts in to the tcgen05 kind::tf32 tensor path.
+
+    'likelihood' (regression only): 'gaussian' (default), the reference's fixed noise sigma passed to sample_elbo; or
+    'heteroscedastic', a learned per-input noise (Kendall & Gal 2017): the last layer has 2 * classes outputs [f | r],
+    the mean f and a raw scale r, and sigma(x) = sigma_min + softplus(r) with 'sigma_min' (default 1e-3) > 0.  `classes`
+    still counts the targets D; forward / sample_predict return the raw [.., 2D] outputs.
     """
 
     def __init__(self, model_params):
@@ -81,12 +91,22 @@ class BayesianNetwork(nn.Module):
         # reg_task.py / class_task.py / bandits.py run unchanged and cannot pass the key)
         self.tf32 = bool(model_params.get('tf32', os.environ.get('BBB_TF32', '0') == '1'))
         self.fused = bool(model_params.get('fused', True))
+        self.likelihood = model_params.get('likelihood', 'gaussian')
+        self.sigma_min = float(model_params.get('sigma_min', 1e-3))
+        if self.likelihood not in ('gaussian', 'heteroscedastic'):
+            raise ValueError(f"likelihood must be 'gaussian' or 'heteroscedastic', got {self.likelihood!r}")
+        if self.likelihood == 'heteroscedastic':
+            if self.mode != 'regression':
+                raise ValueError("the heteroscedastic likelihood is a regression likelihood: needs mode='regression'")
+            if not self.sigma_min > 0:
+                raise ValueError(f'sigma_min must be > 0, got {self.sigma_min}')
+        self._het = self.likelihood == 'heteroscedastic'
 
         if isinstance(self.hidden_units, (list, tuple)):
             hidden = list(self.hidden_units)
         else:
             hidden = [self.hidden_units] * int(model_params.get('n_hidden', 2))
-        dims = [self.input_shape] + hidden + [self.classes]
+        dims = [self.input_shape] + hidden + [self.classes * (2 if self._het else 1)]
         layer = BayesianLinearLR if self.local_reparam else BayesianLinear
         self.n_layers = len(dims) - 1
         for i in range(self.n_layers):
@@ -135,21 +155,30 @@ class BayesianNetwork(nn.Module):
         targets, its calibration -> PredictiveResult (device tensors; .metrics() reads the aggregates).  Eval
         semantics (sampled weights, no log-probs), no autograd, any depth, both estimators, fp32 or TF32 as the
         network is set.  Classification: the outputs are logits and target int64 [B]; regression: likelihood
-        N(y; f, sigma^2) and target [B, D] ([B] when D = 1), matched row for row.
+        N(y; f, sigma^2) and target [B, D] ([B] when D = 1), matched row for row.  Heteroscedastic likelihood: the
+        noise is the net's own sigma(x), `sigma` must stay at its default, and aleatoric_variance is filled.
         The rows are processed in chunks of chunk_rows (None: as many as keep the activations under a fixed budget,
         functional.predictive).  With weight sampling every chunk is scored by the same `samples` networks, so the
         result does not depend on chunk_rows beyond round-off, and the call consumes one Philox step, as
         sample_predict does; with local reparameterisation each chunk draws its own noise (one step per chunk)."""
         x2 = self._flat_input(x)
         params = [l.params() for l in self.layers()]
+        mode = self.mode
+        if self._het:
+            self._check_no_sigma(sigma)
+            mode, sigma = 'heteroscedastic', self.sigma_min
         with torch.no_grad():
             if self.local_reparam:
-                mean, rs, pred, acc = F.predictive(x2, params, samples, self.mode, target, sigma, n_bins, chunk_rows,
+                mean, rs, pred, acc = F.predictive(x2, params, samples, mode, target, sigma, n_bins, chunk_rows,
                                                    sigma_p=float(self.prior_init[0]), tf32=self.tf32)
             else:
-                mean, rs, pred, acc = F.predictive(x2, params, samples, self.mode, target, sigma, n_bins, chunk_rows,
+                mean, rs, pred, acc = F.predictive(x2, params, samples, mode, target, sigma, n_bins, chunk_rows,
                                                    prior=self._prior, tf32=self.tf32)
         log_pred = rs[:, -1] if target is not None else None
+        if self._het:
+            D = self.classes
+            return PredictiveResult(mean, variance=rs[:, :D], aleatoric_variance=rs[:, D:2 * D], log_pred=log_pred,
+                                    acc=acc)
         if self.mode == 'classification':
             return PredictiveResult(mean, pred, rs[:, 0], rs[:, 1], rs[:, 2], rs[:, 3], log_pred=log_pred, acc=acc,
                                     n_bins=n_bins)
@@ -190,6 +219,14 @@ class BayesianNetwork(nn.Module):
         return sum(l.kl_cost for l in self.layers())
 
     def get_nll(self, outputs, target, sigma=1.):
+        if self._het:
+            # outputs [.., 2D] = [f | r], sigma = sigma_min + softplus(r) (the stable form of bbb_nll_gauss_het)
+            self._check_no_sigma(sigma)
+            D = self.classes
+            f, r = outputs[..., :D], outputs[..., D:]
+            s = self.sigma_min + (torch.clamp(r, min=0) + torch.log1p(torch.exp(-r.abs())))
+            y = self._het_target(target, f.shape[0])
+            return (((y - f) / s) ** 2 / 2 + torch.log(s) + _HALF_LOG_2PI).sum()
         if self.mode == 'regression':
             # -Normal(outputs, sigma).log_prob(target).sum() (networks.py:185) written out -- same arithmetic and the same
             # broadcasting of target against outputs (SURVEY App. B-3) -- because the distribution object turns a python
@@ -217,6 +254,20 @@ class BayesianNetwork(nn.Module):
             return target.dim() == 2 and tuple(target.shape) == (B, self.classes) and target.is_floating_point()
         return False
 
+    def _check_no_sigma(self, sigma):
+        """The heteroscedastic net learns its noise: a fixed sigma would contradict it."""
+        if torch.is_tensor(sigma) or sigma != 1.:
+            raise ValueError('the heteroscedastic likelihood learns sigma(x): do not pass sigma (model_params '
+                             "'sigma_min' bounds it from below)")
+
+    def _het_target(self, target, B):
+        """The heteroscedastic likelihood's target, [B, D] ([B] when D = 1), matched row for row (no broadcast)."""
+        D = self.classes
+        if not (tuple(target.shape) == (B, D) or (D == 1 and tuple(target.shape) == (B,))):
+            raise ValueError(f'heteroscedastic target must have shape ({B}, {D})' + (f' or ({B},)' if D == 1 else '') +
+                             f', got {tuple(target.shape)}')
+        return target.reshape(B, D)
+
     def _flat_input(self, input):
         return input.view(-1, self.input_shape) if self.mode == 'classification' else input.reshape(-1, self.input_shape)
 
@@ -225,7 +276,13 @@ class BayesianNetwork(nn.Module):
         assert self.local_reparam == False, 'sample_elbo() method returns loss for BNNs without local reparameterisation, alternatively use sample_elbo_lr()'
         x2 = self._flat_input(input)
         params = [l.params() for l in self.layers()]
-        if self._fusable(x2, target):
+        if self._het:
+            self._check_no_sigma(sigma)
+            target = self._het_target(target, x2.shape[0])
+            if self.fused:
+                return F.fused_elbo(x2, target, beta, samples, self.sigma_min, self.mode, self._prior, params,
+                                    self.tf32, likelihood=self.likelihood)
+        elif self._fusable(x2, target):
             return F.fused_elbo(x2, target, beta, samples, sigma, self.mode, self._prior, params, self.tf32)
         outs, lps, lqs = F.mlp_forward(x2, params, self._prior, samples, True, True, self.tf32)
         negative_log_likelihood = torch.zeros(1, device=outs.device)
@@ -243,7 +300,13 @@ class BayesianNetwork(nn.Module):
         x2 = self._flat_input(input)
         params = [l.params() for l in self.layers()]
         sigma_p = float(self.prior_init[0])
-        if self._fusable(x2, target):
+        if self._het:
+            self._check_no_sigma(sigma)
+            target = self._het_target(target, x2.shape[0])
+            if self.fused:
+                return F.fused_elbo_lr(x2, target, beta, samples, self.sigma_min, self.mode, sigma_p, params,
+                                       self.tf32, likelihood=self.likelihood)
+        elif self._fusable(x2, target):
             return F.fused_elbo_lr(x2, target, beta, samples, sigma, self.mode, sigma_p, params, self.tf32)
         outs, kl = F.mlp_forward_lr(x2, params, sigma_p, samples, True, True, self.tf32)
         negative_log_likelihood = torch.zeros(1, device=outs.device)

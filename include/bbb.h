@@ -186,6 +186,11 @@ int bbb_softmax_mean(const float *logits, int64_t S, int64_t B, int64_t C, float
  *           BBB_NLL_GAUSS: likelihood N(y; f_s, sigma^2).
  *             mean [B,D] = mu = (1/S) sum_s f_s;  row_stats [B,D+1] = { epistemic variance (1/S) sum_s (f_s - mu)^2 per
  *               output (total = that + sigma^2), log predictive density LSE_s(sum_d log N(y_d; f_s,d, sigma^2)) - log S }
+ *           BBB_NLL_GAUSS_HET: heteroscedastic likelihood N(y; f_s, sigma_s^2), C = 2D even, each row [f (D) | r (D)],
+ *             sigma_s = sigma + softplus(r_s) (`sigma` is sigma_min here, see bbb_nll_gauss_het); the predictive is the
+ *             mixture (1/S) sum_s N(f_s, sigma_s^2).  mean [B,D] = mu = (1/S) sum_s f_s;  row_stats [B,2D+1] = { epistemic
+ *             variance (1/S) sum_s (f_s - mu)^2 [D], aleatoric variance (1/S) sum_s sigma_s^2 [D] (total = their sum, the
+ *             law of total variance), log predictive density LSE_s(sum_d log N(y_d; f_s,d, sigma_s,d^2)) - log S }
  *   n_bins  BBB_NLL_CE: 1..1024 confidence bins; bin m holds confidences in (m/M, (m+1)/M], i.e.
  *           m = clamp(ceil(conf M) - 1, 0, M - 1)
  *   acc     fp64 aggregates, ADDED to (required with a target, ignored without):
@@ -193,9 +198,10 @@ int bbb_softmax_mean(const float *logits, int64_t S, int64_t B, int64_t C, float
  *             the bins: the host reports them)  [2] sum -log pbar[y] / sum -lpd
  *             BBB_NLL_CE:    [3] sum correct  [4] sum Brier sum_c (pbar_c - [c = y])^2
  *                            [5 + 3m ..] bin m: count, sum confidence, sum correct      (5 + 3 n_bins doubles)
- *             BBB_NLL_GAUSS: [3] sum_d (mu_d - y_d)^2                                    (4 doubles)
+ *             BBB_NLL_GAUSS, BBB_NLL_GAUSS_HET: [3] sum_d (mu_d - y_d)^2                 (4 doubles)
  *           ECE = (1/n) sum_m |sum correct_m - sum confidence_m|.  Counts are integers, exact in fp64.
- * B == 0 is a no-op.  Bad kind or shape, n_bins out of range, sigma <= 0, a null required pointer: BBB_EINVAL. */
+ * B == 0 is a no-op.  Bad kind or shape (an odd C with BBB_NLL_GAUSS_HET), n_bins out of range, sigma <= 0, a null
+ * required pointer: BBB_EINVAL. */
 int bbb_predictive_stats(const float *out, const void *target, int64_t S, int64_t B, int64_t C, int32_t kind,
                          float sigma, int32_t n_bins, float *mean, float *row_stats, int64_t *pred, double *acc,
                          void *stream);
@@ -209,13 +215,26 @@ int bbb_nll_ce(const float *logits, const int64_t *target, int64_t S, int64_t B,
                float grad_scale, double *nll, float *dlogits, void *stream);
 int bbb_nll_gauss(const float *out, const float *target, float sigma, int64_t S, int64_t B, int64_t D,
                   float grad_scale, double *nll, float *dout, void *stream);
+/* heteroscedastic regression (a learned per-input noise, Kendall & Gal 2017): the net has 2D outputs per row,
+ * out [S,B,2D] = [f | r]: mean f = columns [0, D), raw scale r = columns [D, 2D), target [B,D];
+ *   sigma = sigma_min + softplus(r),  softplus(r) = max(r, 0) + log1p(exp(-|r|)),  sigma_min > 0
+ *   nll  += sum over (s, b, d) of (y - f)^2 / (2 sigma^2) + log sigma + log(2 pi) / 2
+ *   dout (nullable) [S,B,2D], written in full:  d/df = g (f - y) / sigma^2,
+ *                                               d/dr = g sigmoid(r) (1/sigma - (y - f)^2 / sigma^3),  g = grad_scale
+ * Finite for r in [-40, 40] and large residuals (formed from (y - f) / sigma, never from sigma^3).  Launched with
+ * programmatic dependent launch like its siblings.  Null out / target / nll, a negative size, D == 0 with S B > 0 or
+ * sigma_min <= 0: BBB_EINVAL.  No network-level call (bbb_head_fwd, bbb_mlp_fwd) implements this likelihood. */
+#define BBB_NLL_GAUSS_HET 3
+int bbb_nll_gauss_het(const float *out, const float *target, float sigma_min, int64_t S, int64_t B, int64_t D,
+                      float grad_scale, double *nll, float *dout, void *stream);
 
 /* ---- the network's head in one launch --------------------------------------------------------
  * bbb_head_fwd = bbb_linear_fwd of a narrow layer (out <= 16: the classification / regression head, networks.py:164)
  * + bbb_nll_ce / bbb_nll_gauss on its outputs + bbb_elbo_finalize, i.e. the tail of sample_elbo (networks.py:199-209)
  * from the last layer's forward to the four returned scalars.  Exact fp32, deterministic.
  *   nll_kind  BBB_NLL_NONE: plain layer forward (target, nll, dy, out4 ignored);  BBB_NLL_CE: target = int64 [B];
- *             BBB_NLL_GAUSS: target = float [B,out], sigma = likelihood std
+ *             BBB_NLL_GAUSS: target = float [B,out], sigma = likelihood std;  any other kind (BBB_NLL_GAUSS_HET
+ *             included): BBB_EINVAL
  *   y  [S,B,out] written;  dy (nullable) [S,B,out] = grad_scale * d nll / d y;  nll += sum over (s, b)
  *   logp, logq [S] += this layer's terms (BBB_F_LOGPROB); they must already hold the other layers' sums when out4 is
  *             requested, because the CTA that finishes last assembles out4 exactly as bbb_elbo_finalize does
