@@ -147,31 +147,8 @@ def plan_eps(shapes, S, device, sample=True):
 
 
 # =========================================================================================
-# weight-sampling kernels: host-side launch helpers
+# the two estimators: everything that differs between their C-ABI families
 # =========================================================================================
-def _ws_fwd(x, x_stride, p, eps, l, prior, S, B, flags, y, logp, logq):
-    wm, wr, bm, br = p
-    out, inn = wm.shape
-    ew, eb = eps.ptrs(l)
-    rng = eps.rng(l)
-    L.check(L.lib().bbb_linear_fwd(L.ptr(x), x_stride, L.ptr(wm), L.ptr(wr), L.ptr(bm), L.ptr(br), ew, eb,
-                                   C.byref(rng), C.byref(prior), S, B, inn, out, flags, L.ptr(y),
-                                   L.ptr(logp), L.ptr(logq), L.stream()), 'bbb_linear_fwd')
-
-
-def _ws_bwd(dy, mask, x, x_stride, p, eps, l, prior, S, B, flags, gp, gq, gp_dev, gq_dev, g_stride, out_scale, dx,
-            grads):
-    wm, wr, bm, br = p
-    out, inn = wm.shape
-    ew, eb = eps.ptrs(l)
-    rng = eps.rng(l)
-    L.check(L.lib().bbb_linear_bwd(L.ptr(dy), L.ptr(mask), L.ptr(x), x_stride, L.ptr(wm), L.ptr(wr), L.ptr(bm),
-                                   L.ptr(br), ew, eb, C.byref(rng), C.byref(prior), S, B, inn, out, flags,
-                                   gp, gq, L.ptr(gp_dev), L.ptr(gq_dev), g_stride, L.ptr(out_scale), L.ptr(dx),
-                                   L.ptr(grads[0]), L.ptr(grads[1]), L.ptr(grads[2]), L.ptr(grads[3]),
-                                   L.stream()), 'bbb_linear_bwd')
-
-
 def _zeroed_views(shapes, device):
     """One zero-filled buffer carved into tensors of the given shapes (a single memset for all of them): the
     split-K tensor-core kernels add partial tiles into their output with red.add (BBB_F_OUT_ZEROED)."""
@@ -185,37 +162,31 @@ def _zeroed_views(shapes, device):
     return out
 
 
+def _workspace(shapes, device, zero):
+    if zero:
+        return _zeroed_views(shapes, device)
+    return [torch.empty(sh, dtype=torch.float32, device=device) for sh in shapes]
+
+
 def head_eligible(p):
     """bbb_head_fwd's shape conditions (include/bbb.h): a narrow last layer whose rows are 16-byte multiples."""
     out, inn = p[0].shape
     return out <= 16 and inn % 4 == 0 and 4 <= inn <= 8192
 
 
-def _ws_head(x, x_stride, p, eps, l, prior, S, B, flags, y, logp, logq, mode, target, sigma, d_out, nll, beta_h,
-             beta_d, out4, done):
-    """Last layer + likelihood (+ its gradient) + ELBO assembly in one launch (bbb_head_fwd)."""
-    wm, wr, bm, br = p
-    out, inn = wm.shape
-    ew, eb = eps.ptrs(l)
-    rng = eps.rng(l)
-    kind = L.NLL_CE if mode == 'classification' else L.NLL_GAUSS
-    L.check(L.lib().bbb_head_fwd(L.ptr(x), x_stride, L.ptr(wm), L.ptr(wr), L.ptr(bm), L.ptr(br), ew, eb,
-                                 C.byref(rng), C.byref(prior), S, B, inn, out, flags, kind, L.ptr(target),
-                                 float(sigma), 1.0 / S, L.ptr(y), L.ptr(d_out), L.ptr(logp), L.ptr(logq), L.ptr(nll),
-                                 beta_h, L.ptr(beta_d), L.ptr(out4), L.ptr(done), L.stream()), 'bbb_head_fwd')
+def _dev_vec(g):
+    """The gradient of a log-prob output as the fp32 device vector a backward kernel reads (a 0-d one as [1])."""
+    if g is None:
+        return None
+    g = _f32c(g)
+    return g.reshape(1) if g.dim() == 0 else g
 
 
 def _prezero(B):
     """Only the kernels for batches of at most 128 rows combine split-K partial tiles with red.add into a zero-filled
-    output (BBB_F_OUT_ZEROED).  Above that every kernel either writes its output with plain stores or zeroes it
-    itself, so the per-step workspace (gigabytes at batch 4096) is allocated uninitialised."""
+    output (BBB_F_OUT_ZEROED).  Above that every kernel either writes its output with plain stores or zeroes it itself,
+    so the per-step workspace (gigabytes at batch 4096) is allocated uninitialised."""
     return B <= 128
-
-
-def _workspace(shapes, device, zero):
-    if zero:
-        return _zeroed_views(shapes, device)
-    return [torch.empty(sh, dtype=torch.float32, device=device) for sh in shapes]
 
 
 _relu_out_cache = {}
@@ -235,216 +206,6 @@ def _relu_out_layers(params, B, tf32):
               for l, p in enumerate(params)]
         _relu_out_cache[key] = ro
     return ro
-
-
-def _net_ws_forward(x2, params, prior, S, eps, sample, logprob, tf32, logp, logq, ys=None, head=None):
-    """All layers, all S samples.  Returns the list of outputs ys[l] = [S,B,out_l]: pre-activations, except the hidden
-    layers _relu_out_layers names (written into the zero-filled `ys` when the caller supplies them).
-    `head(inp, stride, flags, y)`, when given, runs the last layer instead of bbb_linear_fwd (the fused ELBO tail)."""
-    B = x2.shape[0]
-    ro = _relu_out_layers(params, B, tf32)
-    base = ((L.F_SAMPLE if sample else 0) | (L.F_LOGPROB if logprob else 0) | (L.F_TF32 if tf32 else 0) |
-            (L.F_OUT_ZEROED if _prezero(B) else 0))
-    if ys is None:
-        ys = _workspace([(S, B, p[0].shape[0]) for p in params], x2.device, _prezero(B))
-    inp, stride = x2, 0
-    for l, p in enumerate(params):
-        out, inn = p[0].shape
-        flags = base | (L.F_RELU_IN if l > 0 and not ro[l - 1] else 0) | (L.F_RELU_OUT if ro[l] else 0)
-        if head is not None and l == len(params) - 1:
-            head(inp, stride, flags, ys[l])
-        else:
-            _ws_fwd(inp, stride, p, eps, l, prior, S, B, flags, ys[l], logp, logq)
-        inp, stride = ys[l], B * out
-    return ys
-
-
-def _net_ws_backward(x2, ys, d_out, params, prior, S, eps, sample, tf32, gp, gq, gp_dev, gq_dev, g_stride,
-                     out_scale, need_dx0, dxs=None):
-    """Backward of _net_ws_forward.  Returns (dx0 or None, [grads per layer]).  Every layer above the first
-    hands down the gradient w.r.t. the PRE-activation output of the layer below (BBB_F_DX_PREACT: the ReLU mask
-    is applied where dx is produced), so no layer needs a separate mask pass over dy."""
-    B = x2.shape[0]
-    ro = _relu_out_layers(params, B, tf32)
-    base = (L.F_SAMPLE if sample else 0) | (L.F_TF32 if tf32 else 0) | (L.F_OUT_ZEROED if _prezero(B) else 0)
-    grads = _alloc_grads(params)
-    dy, dx0 = d_out, None
-    first = 0 if need_dx0 else 1
-    if dxs is None:
-        dxs = [None] * first + _workspace([(S, B, p[0].shape[1]) for p in params[first:]], x2.device, _prezero(B))
-    for l in reversed(range(len(params))):
-        p = params[l]
-        out, inn = p[0].shape
-        g = grads[l]
-        flags = base | (L.F_DX_PREACT if l > 0 else 0) | (L.F_RELU_IN if l > 0 and not ro[l - 1] else 0)
-        want_dx = l > 0 or need_dx0
-        dx = dxs[l] if want_dx else None
-        if not want_dx:
-            flags |= L.F_NO_DX
-        if l == 0 and need_dx0:
-            flags |= L.F_SCALE_DX
-        x_in, stride = (x2, 0) if l == 0 else (ys[l - 1], B * inn)
-        _ws_bwd(dy, None, x_in, stride, p, eps, l, prior, S, B, flags, gp, gq, gp_dev, gq_dev, g_stride, out_scale,
-                dx, g)
-        if grad_ready_hook is not None:
-            grad_ready_hook(l, g.flat)
-        dy = dx
-        if l == 0:
-            dx0 = dx
-    return dx0, grads
-
-
-# =========================================================================================
-# layer level
-# =========================================================================================
-class _BayesLinear(torch.autograd.Function):
-    """BayesianLinear.forward for one sample (networks.py:73-88) -> (y, log_prior, log_post)."""
-
-    @staticmethod
-    def forward(ctx, x, wm, wr, bm, br, prior, sample, logprob, layer_id, tf32):
-        L.require_cuda(x, wm, wr, bm, br)
-        out, inn = wm.shape
-        x2 = _f32c(x).reshape(-1, inn)
-        B = x2.shape[0]
-        p = tuple(_f32c(t) for t in (wm, wr, bm, br))
-        eps = plan_eps([((out, inn), (out,))], 1, x2.device, sample)
-        if eps.injected is not None:            # re-key as layer `layer_id`
-            eps.injected = {layer_id: eps.injected[0]}
-        acc = torch.zeros(2, dtype=torch.float64, device=x2.device)
-        y = torch.empty((1, B, out), dtype=torch.float32, device=x2.device)
-        flags = (L.F_SAMPLE if sample else 0) | (L.F_LOGPROB if logprob else 0) | (L.F_TF32 if tf32 else 0)
-        _ws_fwd(x2, 0, p, eps, layer_id, prior, 1, B, flags, y, acc[0:1], acc[1:2])
-        ctx.save_for_backward(x2, *p, *eps.tensors())
-        ctx.cfg = (prior, sample, logprob, layer_id, tf32, eps, x.shape, x.requires_grad)
-        ctx.set_materialize_grads(False)
-        lpq = acc.to(torch.float32)
-        return y.view(*x.shape[:-1], out), lpq[0], lpq[1]
-
-    @staticmethod
-    def backward(ctx, dy, dlp, dlq):
-        prior, sample, logprob, layer_id, tf32, eps, xshape, x_rg = ctx.cfg
-        x2, wm, wr, bm, br = ctx.saved_tensors[:5]
-        out, inn = wm.shape
-        B = x2.shape[0]
-        if dy is None:
-            dy = torch.zeros((B, out), dtype=torch.float32, device=x2.device)
-        dy = _f32c(dy).reshape(1, B, out)
-        g = tuple(torch.empty_like(t) for t in (wm, wr, bm, br))
-        dx = torch.empty((1, B, inn), dtype=torch.float32, device=x2.device) if x_rg else None
-        flags = (L.F_SAMPLE if sample else 0) | (L.F_TF32 if tf32 else 0) | (0 if x_rg else L.F_NO_DX)
-        gp_dev = _f32c(dlp).reshape(1) if dlp is not None else None
-        gq_dev = _f32c(dlq).reshape(1) if dlq is not None else None
-        _ws_bwd(dy, None, x2, 0, (wm, wr, bm, br), eps, layer_id, prior, 1, B, flags,
-                1.0 if gp_dev is not None else 0.0, 1.0 if gq_dev is not None else 0.0, gp_dev, gq_dev, 0, None, dx, g)
-        return (dx.view(xshape) if x_rg else None, g[0], g[1], g[2], g[3], None, None, None, None, None)
-
-
-def bayes_linear(x, wm, wr, bm, br, prior, sample, logprob, layer_id=0, tf32=False):
-    return _BayesLinear.apply(x, wm, wr, bm, br, prior, sample, logprob, layer_id, tf32)
-
-
-# =========================================================================================
-# network level, weight sampling
-# =========================================================================================
-class _MLPForward(torch.autograd.Function):
-    """S sampled forwards of the whole MLP: (x, params) -> outputs [S,B,C], log_prior [S], log_post [S]."""
-
-    @staticmethod
-    def forward(ctx, x2, prior, S, sample, logprob, tf32, *flat):
-        L.require_cuda(x2, *flat)
-        x2 = _f32c(x2)
-        params = [tuple(_f32c(t) for t in flat[i:i + 4]) for i in range(0, len(flat), 4)]
-        eps = plan_eps([(tuple(p[0].shape), (p[0].shape[0],)) for p in params], S, x2.device, sample)
-        acc = torch.zeros(2 * S, dtype=torch.float64, device=x2.device)
-        ys = _net_ws_forward(x2, params, prior, S, eps, sample, logprob, tf32, acc[:S], acc[S:])
-        ctx.save_for_backward(x2, *flat, *ys, *eps.tensors())
-        ctx.cfg = (prior, S, sample, tf32, eps, len(params), x2.requires_grad)
-        ctx.set_materialize_grads(False)
-        lpq = acc.to(torch.float32)
-        # the last layer's buffer is handed out; backward only needs the hidden pre-activations
-        return ys[-1], lpq[:S], lpq[S:]
-
-    @staticmethod
-    def backward(ctx, d_out, dlp, dlq):
-        prior, S, sample, tf32, eps, nl, x_rg = ctx.cfg
-        sv = ctx.saved_tensors
-        x2 = sv[0]
-        params = [tuple(_f32c(t) for t in sv[1 + 4 * i:5 + 4 * i]) for i in range(nl)]
-        ys = list(sv[1 + 4 * nl:1 + 5 * nl])
-        B = x2.shape[0]
-        if d_out is None:
-            d_out = torch.zeros_like(ys[-1])
-        gp_dev = _f32c(dlp) if dlp is not None else None
-        gq_dev = _f32c(dlq) if dlq is not None else None
-        dx0, grads = _net_ws_backward(x2, ys, _f32c(d_out), params, prior, S, eps, sample, tf32,
-                                      1.0 if gp_dev is not None else 0.0, 1.0 if gq_dev is not None else 0.0,
-                                      gp_dev, gq_dev, 1, None, x_rg)
-        flat = [g for lg in grads for g in lg]
-        return (dx0.sum(0) if x_rg else None, None, None, None, None, None, *flat)
-
-
-def mlp_forward(x2, layers, prior, S, sample=True, logprob=True, tf32=False):
-    flat = [t for layer in layers for t in layer]
-    return _MLPForward.apply(x2, prior, S, sample, logprob, tf32, *flat)
-
-
-# sample_elbo in TF32 mode goes through ONE C call per network pass (bbb_mlp_fwd / bbb_mlp_bwd) when the library covers
-# the network (bbb_mlp_supported); False forces the per-layer calls (A/B measurements, tools/check_mlp.py)
-use_network_level_call = True
-
-
-def _nll_launch(out, target, S, B, Cc, sigma, mode, likelihood, nll, d_out):
-    """The likelihood and its gradient (scaled by 1/S) on the sampled outputs [S,B,Cc]: nll += ..., d_out written.
-    The heteroscedastic likelihood reads `sigma` as sigma_min and Cc = 2D outputs per row."""
-    if likelihood == 'heteroscedastic':
-        tgt = _f32c(target)            # (held: a contiguous copy must outlive the call)
-        L.check(L.lib().bbb_nll_gauss_het(L.ptr(out), L.ptr(tgt), float(sigma), S, B, Cc // 2, 1.0 / S, L.ptr(nll),
-                                          L.ptr(d_out), L.stream()), 'bbb_nll_gauss_het')
-    elif mode == 'classification':
-        L.check(L.lib().bbb_nll_ce(L.ptr(out), L.ptr(target), S, B, Cc, 1.0 / S, L.ptr(nll), L.ptr(d_out),
-                                   L.stream()), 'bbb_nll_ce')
-    else:
-        tgt = _f32c(target)
-        L.check(L.lib().bbb_nll_gauss(L.ptr(out), L.ptr(tgt), float(sigma), S, B, Cc, 1.0 / S, L.ptr(nll),
-                                      L.ptr(d_out), L.stream()), 'bbb_nll_gauss')
-
-
-def _layerwise_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, need_grad, tf32, beta_h, beta_d, out4,
-                            likelihood='gaussian'):
-    """sample_elbo's forward as one launch per layer (+ the fused head): every shape, both modes.  Returns
-    (ys: per-layer PRE-activation outputs, dxs: the backward's zero-filled dx workspace, d_out).  The heteroscedastic
-    likelihood has no fused head: its last layer is a plain layer call, then bbb_nll_gauss_het."""
-    dev = x2.device
-    # ONE zero-filled workspace (one memset per step): fp64 accumulators + the head's completion counter |
-    # activations of every layer | dx of every layer above the first (the backward's split-K kernels add into them)
-    shapes = [(2 * (2 * S + 1) + 2,)] + [(S, B, p[0].shape[0]) for p in params]
-    if need_grad:
-        shapes += [(S, B, p[0].shape[1]) for p in params[1:]]
-    if _prezero(B):
-        ws = _zeroed_views(shapes, dev)
-    else:                      # large batch: only the accumulators are zeroed
-        ws = _zeroed_views(shapes[:1], dev) + _workspace(shapes[1:], dev, False)
-    acc = ws[0][:2 * (2 * S + 1)].view(torch.float64)
-    done = ws[0][2 * (2 * S + 1):]
-    ys, dxs = ws[1:1 + len(params)], ([None] + ws[1 + len(params):] if need_grad else None)
-    logp, logq, nll = acc[:S], acc[S:2 * S], acc[2 * S:]
-    Cc = params[-1][0].shape[0]
-    d_out = torch.empty((S, B, Cc), dtype=torch.float32, device=dev) if need_grad else None
-    if likelihood == 'gaussian' and head_eligible(params[-1]):
-        # the last layer, the likelihood with its gradient and the assembly of the four scalars: one launch
-        tgt = target if mode == 'classification' else _f32c(target)
-        nl = len(params) - 1
-
-        def head(inp, stride, flags, y):
-            _ws_head(inp, stride, params[nl], eps, nl, prior, S, B, flags, y, logp, logq, mode, tgt, sigma, d_out,
-                     nll, beta_h, beta_d, out4, done)
-        ys = _net_ws_forward(x2, params, prior, S, eps, True, True, tf32, logp, logq, ys, head)
-    else:
-        ys = _net_ws_forward(x2, params, prior, S, eps, True, True, tf32, logp, logq, ys)
-        _nll_launch(ys[-1], target, S, B, Cc, sigma, mode, likelihood, nll, d_out)
-        L.check(L.lib().bbb_elbo_finalize(L.ptr(logp), L.ptr(logq), None, L.ptr(nll), S, beta_h, L.ptr(beta_d),
-                                          L.ptr(out4), L.stream()), 'bbb_elbo_finalize')
-    return ys, dxs, d_out
 
 
 def _mlp_layer_table(params, eps, ys, dzs, grads):
@@ -487,158 +248,344 @@ def _mlp_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, need_gr
     rng = eps.rng(0)
     L.check(L.lib().bbb_mlp_fwd(tab, nl, L.ptr(x2), S, B, C.byref(rng), C.byref(prior),
                                 L.F_SAMPLE | L.F_LOGPROB | L.F_TF32, kind, L.ptr(tgt), float(sigma), 1.0 / S,
-                                L.ptr(d_out), L.ptr(logp), L.ptr(logq), L.ptr(nll), beta_h, L.ptr(beta_d), L.ptr(out4),
-                                L.ptr(done), L.stream()), 'bbb_mlp_fwd')
+                                L.ptr(d_out), L.ptr(logp), L.ptr(logq), L.ptr(nll), beta_h, L.ptr(beta_d),
+                                L.ptr(out4), L.ptr(done), L.stream()), 'bbb_mlp_fwd')
     return ys, ([None] + list(dzs) if need_grad else None), d_out
 
 
-class _FusedELBO(torch.autograd.Function):
-    """sample_elbo (networks.py:192-209).  TF32 mode, batch <= 128: ONE C call per pass (bbb_mlp_fwd: a TMA-fed tcgen05
-    kernel per hidden layer + the fused head; bbb_mlp_bwd: head + one fused wgrad/dgrad kernel per layer).  Otherwise one
-    launch per layer (+ likelihood + assembly).  Only `loss` is differentiable.  likelihood 'heteroscedastic' (sigma is
-    then sigma_min) always takes the per-layer calls: neither network-level call implements it."""
+# sample_elbo in TF32 mode goes through ONE C call per network pass (bbb_mlp_fwd / bbb_mlp_bwd) when the library covers
+# the network (bbb_mlp_supported); False forces the per-layer calls (A/B measurements, tools/check_mlp.py)
+use_network_level_call = True
+
+
+class _WeightSampling:
+    """Weight sampling (networks.py:48-88, 192-209): weights [out, in] sampled per sample, log prior and log posterior
+    of the sampled weights accumulated per sample (2S fp64 values), their gradient taken through the prior-gradient
+    scalars gp / gq of the backward (BBB_F_LOGPROB is a forward flag only)."""
+    __slots__ = ('prior',)
+    has_delta = False            # no per-layer buffer besides the output
+    eps_per_row = False          # one eps per weight: every input row sees the same S networks
+    reuse_error = ('sample_elbo: this graph was already differentiated (retain_graph=True is not supported by the '
+                   'fused ELBO path: its backward workspace is single-use)')
+    prezero = staticmethod(_prezero)
+    relu_out = staticmethod(_relu_out_layers)
+
+    def __init__(self, prior):
+        self.prior = prior
 
     @staticmethod
-    def forward(ctx, x2, target, beta, S, sigma, mode, likelihood, prior, tf32, *flat):
-        L.require_cuda(x2, target, *flat)
-        x2 = _f32c(x2)
-        dev = x2.device
-        params = [tuple(_f32c(t) for t in flat[i:i + 4]) for i in range(0, len(flat), 4)]
-        eps = plan_eps([(tuple(p[0].shape), (p[0].shape[0],)) for p in params], S, dev, True)
-        need_grad = any(t.requires_grad for t in flat)
-        B = x2.shape[0]
-        Cc = params[-1][0].shape[0]
-        out4 = torch.empty(4, dtype=torch.float32, device=dev)
-        beta_h, beta_d = _split_beta(beta)
-        dims = [params[0][0].shape[1]] + [p[0].shape[0] for p in params]
-        use_mlp = (likelihood == 'gaussian' and use_network_level_call and tf32 and
-                   mode in ('classification', 'regression') and L.mlp_supported(dims, S, B, L.F_TF32))
-        if use_mlp:
-            ys, dxs, d_out = _mlp_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, need_grad, beta_h,
-                                               beta_d, out4)
-        else:
-            ys, dxs, d_out = _layerwise_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, need_grad, tf32,
-                                                     beta_h, beta_d, out4, likelihood)
+    def shape(w):
+        """(in, out) of a layer from its weight tensor."""
+        out, inn = w.shape
+        return inn, out
+
+    @staticmethod
+    def eps_shapes(params, B):
+        return [(tuple(p[0].shape), (p[0].shape[0],)) for p in params]
+
+    @staticmethod
+    def acc_len(S):
+        return 2 * S
+
+    @staticmethod
+    def lp(acc, S):
+        """The log-prob accumulators the forward adds into: (log prior [S], log posterior [S])."""
+        return acc[:S], acc[S:2 * S]
+
+    @staticmethod
+    def lp_outputs(lpq, S, scalars):
+        """The log-prob outputs from the fp32 accumulators: per sample, or as two scalars when S = 1."""
+        return (lpq[0], lpq[1]) if scalars else (lpq[:S], lpq[S:])
+
+    @staticmethod
+    def grad_args(gs, logprob, scalars):
+        """(backward flags, prior-gradient arguments) from the gradients of the log-prob outputs (None: not used)."""
+        gp, gq = (_dev_vec(g) for g in gs)
+        return 0, (1.0 if gp is not None else 0.0, 1.0 if gq is not None else 0.0, gp, gq, 0 if scalars else 1)
+
+    @staticmethod
+    def elbo_grad_args(beta, beta_dev, S):
+        """loss = beta (log q - log p) / S summed over the samples + nll: gp = -beta / S, gq = beta / S."""
+        return 0, (-beta / S, beta / S, beta_dev, beta_dev, 0)
+
+    def fwd(self, x, x_stride, p, eps, l, S, B, flags, y, delta, lp):
+        wm, wr, bm, br = p
+        out, inn = wm.shape
+        ew, eb = eps.ptrs(l)
+        rng = eps.rng(l)
+        L.check(L.lib().bbb_linear_fwd(L.ptr(x), x_stride, L.ptr(wm), L.ptr(wr), L.ptr(bm), L.ptr(br), ew, eb,
+                                       C.byref(rng), C.byref(self.prior), S, B, inn, out, flags, L.ptr(y),
+                                       L.ptr(lp[0]), L.ptr(lp[1]), L.stream()), 'bbb_linear_fwd')
+
+    def bwd(self, dy, x, x_stride, p, eps, l, delta, S, B, flags, gargs, out_scale, dx, grads):
+        wm, wr, bm, br = p
+        out, inn = wm.shape
+        ew, eb = eps.ptrs(l)
+        rng = eps.rng(l)
+        gp, gq, gp_dev, gq_dev, g_stride = gargs
+        L.check(L.lib().bbb_linear_bwd(L.ptr(dy), None, L.ptr(x), x_stride, L.ptr(wm), L.ptr(wr), L.ptr(bm),
+                                       L.ptr(br), ew, eb, C.byref(rng), C.byref(self.prior), S, B, inn, out, flags,
+                                       gp, gq, L.ptr(gp_dev), L.ptr(gq_dev), g_stride, L.ptr(out_scale), L.ptr(dx),
+                                       L.ptr(grads[0]), L.ptr(grads[1]), L.ptr(grads[2]), L.ptr(grads[3]),
+                                       L.stream()), 'bbb_linear_bwd')
+
+    # ---- sample_elbo ------------------------------------------------------------------------------------------------
+    @staticmethod
+    def elbo_workspace(params, S, B, need_grad, dev):
+        """ONE zero-filled workspace (one memset per step): fp64 accumulators + the head's completion counter |
+        activations of every layer | dx of every layer above the first (the backward's split-K kernels add into them).
+        Large batches zero only the accumulators.  Returns (lp, nll, done, ys, deltas, dxs, d_out)."""
+        shapes = [(2 * (2 * S + 1) + 2,)] + [(S, B, p[0].shape[0]) for p in params]
         if need_grad:
-            ctx.save_for_backward(x2, d_out, *flat, *ys[:-1], *eps.tensors())
-            ctx.dxs = dxs
-        ctx.used_mlp = use_mlp
-        ctx.cfg = (prior, S, beta_h, tf32, eps, len(params))
-        ctx.beta_dev = beta_d
-        ctx.set_materialize_grads(False)      # no zero-filled gradients for the three non-differentiable scalars
-        loss, lp, lq, nl = out4[0:1], out4[1], out4[2], out4[3:4]
-        ctx.mark_non_differentiable(lp, lq, nl)
-        return loss, lp, lq, nl
+            shapes += [(S, B, p[0].shape[1]) for p in params[1:]]
+        if _prezero(B):
+            ws = _zeroed_views(shapes, dev)
+        else:
+            ws = _zeroed_views(shapes[:1], dev) + _workspace(shapes[1:], dev, False)
+        acc = ws[0][:2 * (2 * S + 1)].view(torch.float64)
+        done = ws[0][2 * (2 * S + 1):]
+        nl = len(params)
+        ys, dxs = ws[1:1 + nl], ([None] + ws[1 + nl:] if need_grad else None)
+        logp, logq, nll = acc[:S], acc[S:2 * S], acc[2 * S:]
+        d_out = torch.empty((S, B, params[-1][0].shape[0]), dtype=torch.float32, device=dev) if need_grad else None
+        return (logp, logq), nll, done, ys, [None] * nl, dxs, d_out
+
+    def head(self, params, eps, S, B, mode, likelihood, target, sigma, d_out, lp, nll, beta_h, beta_d, out4, done):
+        """The last layer, the likelihood with its gradient and the assembly of the four scalars in one launch
+        (bbb_head_fwd), as head(inp, stride, flags, y) for the forward loop; None when it does not apply (the
+        heteroscedastic likelihood has no fused head)."""
+        if likelihood != 'gaussian' or not head_eligible(params[-1]):
+            return None
+        nl = len(params) - 1
+        wm, wr, bm, br = params[nl]
+        out, inn = wm.shape
+        ew, eb = eps.ptrs(nl)
+        kind = L.NLL_CE if mode == 'classification' else L.NLL_GAUSS
+        tgt = target if mode == 'classification' else _f32c(target)
+
+        def head(x, x_stride, flags, y):
+            rng = eps.rng(nl)
+            L.check(L.lib().bbb_head_fwd(L.ptr(x), x_stride, L.ptr(wm), L.ptr(wr), L.ptr(bm), L.ptr(br), ew, eb,
+                                         C.byref(rng), C.byref(self.prior), S, B, inn, out, flags, kind, L.ptr(tgt),
+                                         float(sigma), 1.0 / S, L.ptr(y), L.ptr(d_out), L.ptr(lp[0]), L.ptr(lp[1]),
+                                         L.ptr(nll), beta_h, L.ptr(beta_d), L.ptr(out4), L.ptr(done), L.stream()),
+                    'bbb_head_fwd')
+        return head
 
     @staticmethod
-    def backward(ctx, g_loss, *unused):
-        prior, S, beta, tf32, eps, nl = ctx.cfg
-        if g_loss is None:
-            return (None,) * (9 + 4 * nl)
-        if getattr(ctx, 'consumed', False):
-            # the split-K backward kernels ADD into the dx workspace zero-filled by the forward (BBB_F_OUT_ZEROED)
-            raise RuntimeError('sample_elbo: this graph was already differentiated (retain_graph=True is not '
-                               'supported by the fused ELBO path: its backward workspace is single-use)')
-        ctx.consumed = True
-        sv = ctx.saved_tensors
-        x2, d_out = sv[0], sv[1]
-        params = [tuple(_f32c(t) for t in sv[2 + 4 * i:6 + 4 * i]) for i in range(nl)]
-        ys = list(sv[2 + 4 * nl:2 + 4 * nl + nl - 1]) + [None]
-        scale = _f32c(g_loss).reshape(1)
-        bd = ctx.beta_dev
-        if ctx.used_mlp:
-            # ONE C call for the whole backward (bbb_mlp_bwd): ys are the stored pre-activations, ctx.dxs[l + 1] the
-            # zero-filled gradient w.r.t. hidden layer l's pre-activation output
-            grads = _alloc_grads(params)
-            B = x2.shape[0]
-            dzs = list(ctx.dxs[1:nl]) + [d_out]
-            tab = _mlp_layer_table(params, eps, ys, dzs, grads)
-            rng = eps.rng(0)
-            L.check(L.lib().bbb_mlp_bwd(tab, nl, L.ptr(x2), S, B, C.byref(rng), C.byref(prior), L.F_SAMPLE | L.F_TF32,
-                                        -beta / S, beta / S, L.ptr(bd), L.ptr(bd), 0, L.ptr(scale), L.stream()),
-                    'bbb_mlp_bwd')
-            if grad_ready_hook is not None:
-                for l in reversed(range(nl)):
-                    grad_ready_hook(l, grads[l].flat)
-        else:
-            _, grads = _net_ws_backward(x2, ys, d_out, params, prior, S, eps, True, tf32, -beta / S, beta / S,
-                                        bd, bd, 0, scale, False, dxs=ctx.dxs)
-        flat = [g for lg in grads for g in lg]
-        return (None,) * 9 + tuple(flat)
+    def finalize(lp, nll, S, beta_h, beta_d, out4):
+        L.check(L.lib().bbb_elbo_finalize(L.ptr(lp[0]), L.ptr(lp[1]), None, L.ptr(nll), S, beta_h, L.ptr(beta_d),
+                                          L.ptr(out4), L.stream()), 'bbb_elbo_finalize')
+
+    @staticmethod
+    def elbo_outputs(out4):
+        """(loss [1], log_prior, log_variational_posterior, negative_log_likelihood [1])"""
+        return out4[0:1], out4[1], out4[2], out4[3:4]
+
+    @staticmethod
+    def single_use(tf32):
+        # the split-K backward kernels ADD into the dx workspace zero-filled by the forward (BBB_F_OUT_ZEROED)
+        return True
+
+    @staticmethod
+    def network_call(params, S, B, mode, likelihood, tf32):
+        """Does sample_elbo run as ONE C call per pass (bbb_mlp_fwd / bbb_mlp_bwd: TMA-fed tcgen05 kernels for the
+        hidden layers + the fused head)?  Neither call implements the heteroscedastic likelihood."""
+        dims = [params[0][0].shape[1]] + [p[0].shape[0] for p in params]
+        return (likelihood == 'gaussian' and use_network_level_call and tf32 and
+                mode in ('classification', 'regression') and L.mlp_supported(dims, S, B, L.F_TF32))
+
+    def network_forward(self, x2, target, params, eps, S, B, sigma, mode, need_grad, beta_h, beta_d, out4):
+        return _mlp_forward_call(x2, target, params, eps, self.prior, S, B, sigma, mode, need_grad, beta_h, beta_d,
+                                 out4)
+
+    def network_backward(self, x2, ys, dxs, d_out, params, S, eps, gargs, scale):
+        """ONE C call for the whole backward (bbb_mlp_bwd): ys are the stored hidden pre-activations, dxs[l + 1] the
+        zero-filled gradient w.r.t. hidden layer l's pre-activation output."""
+        nl = len(params)
+        grads = _alloc_grads(params)
+        tab = _mlp_layer_table(params, eps, list(ys) + [None], list(dxs[1:nl]) + [d_out], grads)
+        rng = eps.rng(0)
+        gp, gq, gp_dev, gq_dev, g_stride = gargs
+        L.check(L.lib().bbb_mlp_bwd(tab, nl, L.ptr(x2), S, x2.shape[0], C.byref(rng), C.byref(self.prior),
+                                    L.F_SAMPLE | L.F_TF32, gp, gq, L.ptr(gp_dev), L.ptr(gq_dev), g_stride,
+                                    L.ptr(scale), L.stream()), 'bbb_mlp_bwd')
+        if grad_ready_hook is not None:
+            for l in reversed(range(nl)):
+                grad_ready_hook(l, grads[l].flat)
+        return grads
 
 
-def fused_elbo(x2, target, beta, S, sigma, mode, prior, layers, tf32=False, likelihood='gaussian'):
-    flat = [t for layer in layers for t in layer]
-    return _FusedELBO.apply(x2, target, beta, S, sigma, mode, likelihood, prior, tf32, *flat)
+class _LocalReparam:
+    """Local reparameterisation (networks.py:90-138, 211-225): weights [in, out], the pre-activation sampled per row
+    from its mean x mu and variance delta = x^2 sigma^2 (kept per layer for the backward), one closed-form KL for the
+    whole call, its gradient taken through BBB_F_LOGPROB in the backward."""
+    __slots__ = ('sigma_p',)
+    has_delta = True
+    eps_per_row = True           # the noise is drawn per input row: a chunked pass draws it chunk by chunk
+    reuse_error = ('sample_elbo_lr: this graph was already differentiated (retain_graph=True is not supported by the '
+                   'TF32 local-reparameterisation path: its saved state is single-use)')
+
+    def __init__(self, sigma_p):
+        self.sigma_p = float(sigma_p)
+
+    @staticmethod
+    def shape(w):
+        return tuple(w.shape)
+
+    @staticmethod
+    def eps_shapes(params, B):
+        return [((B, p[0].shape[1]), (p[0].shape[1],)) for p in params]
+
+    @staticmethod
+    def prezero(B):
+        # the tensor-core kernels add their split-K partial sums of x mu and x^2 sigma^2 into y and delta (and of dx)
+        # before the epilogue turns them into the outputs, at every batch size
+        return True
+
+    @staticmethod
+    def relu_out(params, B, tf32):
+        return [False] * len(params)
+
+    @staticmethod
+    def acc_len(S):
+        return 1
+
+    @staticmethod
+    def lp(acc, S):
+        """The KL accumulator the forward adds into (evaluated once per call, not per sample: SURVEY B-8)."""
+        return (acc,)
+
+    @staticmethod
+    def lp_outputs(lpq, S, scalars):
+        return (lpq[0],)
+
+    @staticmethod
+    def grad_args(gs, logprob, scalars):
+        use_kl = logprob and gs[0] is not None
+        return (L.F_LOGPROB if use_kl else 0), (1.0, _dev_vec(gs[0]) if use_kl else None)
+
+    @staticmethod
+    def elbo_grad_args(beta, beta_dev, S):
+        """loss = beta KL + nll"""
+        return L.F_LOGPROB, (beta, beta_dev)
+
+    def fwd(self, x, x_stride, p, eps, l, S, B, flags, y, delta, lp):
+        wm, wr, bm, br = p
+        inn, out = wm.shape
+        ea, eb = eps.ptrs(l)
+        rng = eps.rng(l)
+        L.check(L.lib().bbb_lr_linear_fwd(L.ptr(x), x_stride, L.ptr(wm), L.ptr(wr), L.ptr(bm), L.ptr(br), ea, eb,
+                                          C.byref(rng), self.sigma_p, S, B, inn, out, flags, L.ptr(y), L.ptr(delta),
+                                          L.ptr(lp[0]), L.stream()), 'bbb_lr_linear_fwd')
+
+    def bwd(self, dy, x, x_stride, p, eps, l, delta, S, B, flags, gargs, out_scale, dx, grads):
+        """In TF32 mode the kernels overwrite the saved delta with dV (it has no other use in the backward)."""
+        wm, wr, bm, br = p
+        inn, out = wm.shape
+        ea, eb = eps.ptrs(l)
+        rng = eps.rng(l)
+        g_kl, g_kl_dev = gargs
+        L.check(L.lib().bbb_lr_linear_bwd(L.ptr(dy), None, L.ptr(x), x_stride, L.ptr(wm), L.ptr(wr), L.ptr(bm),
+                                          L.ptr(br), ea, eb, C.byref(rng), L.ptr(delta), self.sigma_p, S, B, inn, out,
+                                          flags, g_kl, L.ptr(g_kl_dev), L.ptr(out_scale), L.ptr(dx), L.ptr(grads[0]),
+                                          L.ptr(grads[1]), L.ptr(grads[2]), L.ptr(grads[3]), L.stream()),
+                'bbb_lr_linear_bwd')
+
+    # ---- sample_elbo_lr ---------------------------------------------------------------------------------------------
+    def elbo_workspace(self, params, S, B, need_grad, dev):
+        """Returns (lp, nll, done, ys, deltas, dxs, d_out); the backward allocates its own dx buffers."""
+        acc = torch.zeros(2, dtype=torch.float64, device=dev)
+        kl, nll = acc[0:1], acc[1:2]
+        ys, deltas = _activations(self, params, S, B, True, dev)
+        d_out = torch.empty_like(ys[-1]) if need_grad else None
+        return (kl,), nll, None, ys, deltas, None, d_out
+
+    @staticmethod
+    def head(*args):
+        return None
+
+    @staticmethod
+    def finalize(lp, nll, S, beta_h, beta_d, out4):
+        L.check(L.lib().bbb_elbo_finalize(None, None, L.ptr(lp[0]), L.ptr(nll), S, beta_h, L.ptr(beta_d), L.ptr(out4),
+                                          L.stream()), 'bbb_elbo_finalize')
+
+    @staticmethod
+    def elbo_outputs(out4):
+        """(loss [1], kl, negative_log_likelihood [1])"""
+        return out4[0:1], out4[1], out4[2:3]
+
+    @staticmethod
+    def single_use(tf32):
+        # the tcgen05 LR backward overwrites the saved delta buffers with dV
+        return tf32
+
+    @staticmethod
+    def network_call(params, S, B, mode, likelihood, tf32):
+        return False
 
 
 # =========================================================================================
-# local reparameterisation
+# one network pass, forward and backward, for either estimator
 # =========================================================================================
-def _lr_fwd(x, x_stride, p, eps, l, sigma_p, S, B, flags, y, delta, kl):
-    wm, wr, bm, br = p
-    inn, out = wm.shape
-    ea, eb = eps.ptrs(l)
-    rng = eps.rng(l)
-    L.check(L.lib().bbb_lr_linear_fwd(L.ptr(x), x_stride, L.ptr(wm), L.ptr(wr), L.ptr(bm), L.ptr(br), ea, eb,
-                                      C.byref(rng), sigma_p, S, B, inn, out, flags, L.ptr(y), L.ptr(delta),
-                                      L.ptr(kl), L.stream()), 'bbb_lr_linear_fwd')
+def _activations(est, params, S, B, sample, dev):
+    """Every layer's output [S,B,out] (and delta, when the estimator keeps one and the call samples): one buffer,
+    zero-filled when the estimator's kernels add into it."""
+    shapes = [(S, B, est.shape(p[0])[1]) for p in params]
+    bufs = _workspace(shapes * (2 if sample and est.has_delta else 1), dev, est.prezero(B))
+    n = len(params)
+    return bufs[:n], (bufs[n:] or [None] * n)
 
 
-def _lr_bwd(dy, mask, x, x_stride, p, eps, l, delta, sigma_p, S, B, flags, g_kl, g_kl_dev, out_scale, dx, grads):
-    wm, wr, bm, br = p
-    inn, out = wm.shape
-    ea, eb = eps.ptrs(l)
-    rng = eps.rng(l)
-    L.check(L.lib().bbb_lr_linear_bwd(L.ptr(dy), L.ptr(mask), L.ptr(x), x_stride, L.ptr(wm), L.ptr(wr), L.ptr(bm),
-                                      L.ptr(br), ea, eb, C.byref(rng), L.ptr(delta), sigma_p, S, B, inn, out, flags,
-                                      g_kl, L.ptr(g_kl_dev), L.ptr(out_scale), L.ptr(dx), L.ptr(grads[0]),
-                                      L.ptr(grads[1]), L.ptr(grads[2]), L.ptr(grads[3]), L.stream()),
-            'bbb_lr_linear_bwd')
-
-
-def _net_lr_forward(x2, params, sigma_p, S, eps, sample, calc_kl, kl, tf32=False):
+def _forward(est, x2, params, S, eps, sample, logprob, tf32, lp, ys=None, deltas=None, head=None):
+    """All layers, all S samples.  Returns (ys, deltas): ys[l] = [S,B,out_l] pre-activations, except the hidden
+    layers est.relu_out names.  `ys`, `deltas` when the caller supplies them; `head(inp, stride, flags, y)`, when
+    given, runs the last layer instead of the layer call (the fused ELBO tail)."""
     B = x2.shape[0]
-    base = ((L.F_SAMPLE if sample else 0) | (L.F_LOGPROB if calc_kl else 0) | (L.F_TF32 if tf32 else 0) |
-            L.F_OUT_ZEROED)
-    # one zero-filled buffer for every layer's y and delta: the tensor-core kernels add their split-K partial sums
-    # of x mu and x^2 sigma^2 into them before the epilogue turns them into the outputs
-    shapes = [(S, B, p[0].shape[1]) for p in params]
-    bufs = _zeroed_views(shapes + (shapes if sample else []), x2.device)
-    ys, deltas = bufs[:len(params)], (bufs[len(params):] if sample else [None] * len(params))
+    ro = est.relu_out(params, B, tf32)
+    base = ((L.F_SAMPLE if sample else 0) | (L.F_LOGPROB if logprob else 0) | (L.F_TF32 if tf32 else 0) |
+            (L.F_OUT_ZEROED if est.prezero(B) else 0))
+    if ys is None:
+        ys, deltas = _activations(est, params, S, B, sample, x2.device)
     inp, stride = x2, 0
     for l, p in enumerate(params):
-        inn, out = p[0].shape
-        _lr_fwd(inp, stride, p, eps, l, sigma_p, S, B, base | (L.F_RELU_IN if l > 0 else 0), ys[l], deltas[l], kl)
-        inp, stride = ys[l], B * out
+        flags = base | (L.F_RELU_IN if l > 0 and not ro[l - 1] else 0) | (L.F_RELU_OUT if ro[l] else 0)
+        if head is not None and l == len(params) - 1:
+            head(inp, stride, flags, ys[l])
+        else:
+            est.fwd(inp, stride, p, eps, l, S, B, flags, ys[l], deltas[l], lp)
+        inp, stride = ys[l], B * est.shape(p[0])[1]
     return ys, deltas
 
 
-def _net_lr_backward(x2, ys, deltas, d_out, params, sigma_p, S, eps, sample, calc_kl, g_kl, g_kl_dev, out_scale,
-                     need_dx0, tf32=False):
-    """Backward of _net_lr_forward.  As in the weight-sampling path every layer above the first hands down the
-    gradient w.r.t. the pre-activation output of the layer below (BBB_F_DX_PREACT).  In TF32 mode the kernels
-    overwrite the saved delta buffers with dV (they have no other use in the backward)."""
+def _backward(est, x2, ys, deltas, d_out, params, S, eps, sample, tf32, pg, out_scale, need_dx0, dxs=None):
+    """Backward of _forward; pg = (flags, arguments) of the prior gradient (est.grad_args / est.elbo_grad_args).
+    Returns (dx0 or None, [grads per layer]).  Every layer above the first hands down the gradient w.r.t. the
+    PRE-activation output of the layer below (BBB_F_DX_PREACT: the ReLU mask is applied where dx is produced), so no
+    layer needs a separate mask pass over dy."""
     B = x2.shape[0]
-    base = ((L.F_SAMPLE if sample else 0) | (L.F_LOGPROB if calc_kl else 0) | (L.F_TF32 if tf32 else 0) |
-            L.F_OUT_ZEROED)
+    ro = est.relu_out(params, B, tf32)
+    gflags, gargs = pg
+    base = ((L.F_SAMPLE if sample else 0) | (L.F_TF32 if tf32 else 0) | (L.F_OUT_ZEROED if est.prezero(B) else 0) |
+            gflags)
     grads = _alloc_grads(params)
     dy, dx0 = d_out, None
     first = 0 if need_dx0 else 1
-    dxs = [None] * first + _zeroed_views([(S, B, p[0].shape[0]) for p in params[first:]], x2.device)
+    if dxs is None:
+        dxs = [None] * first + _workspace([(S, B, est.shape(p[0])[0]) for p in params[first:]], x2.device,
+                                          est.prezero(B))
     for l in reversed(range(len(params))):
         p = params[l]
-        inn, out = p[0].shape
         g = grads[l]
-        flags = base | ((L.F_RELU_IN | L.F_DX_PREACT) if l > 0 else 0)
+        flags = base | (L.F_DX_PREACT if l > 0 else 0) | (L.F_RELU_IN if l > 0 and not ro[l - 1] else 0)
         want_dx = l > 0 or need_dx0
         dx = dxs[l] if want_dx else None
         if not want_dx:
             flags |= L.F_NO_DX
         if l == 0 and need_dx0:
             flags |= L.F_SCALE_DX
-        x_in, stride = (x2, 0) if l == 0 else (ys[l - 1], B * inn)
-        _lr_bwd(dy, None, x_in, stride, p, eps, l, deltas[l], sigma_p, S, B, flags, g_kl, g_kl_dev, out_scale, dx, g)
+        x_in, stride = (x2, 0) if l == 0 else (ys[l - 1], B * est.shape(p[0])[0])
+        est.bwd(dy, x_in, stride, p, eps, l, deltas[l], S, B, flags, gargs, out_scale, dx, g)
         if grad_ready_hook is not None:
             grad_ready_hook(l, g.flat)
         dy = dx
@@ -647,158 +594,221 @@ def _net_lr_backward(x2, ys, deltas, d_out, params, sigma_p, S, eps, sample, cal
     return dx0, grads
 
 
-class _LRLinear(torch.autograd.Function):
-    """BayesianLinearLR.forward for one sample (networks.py:116-138) -> (y, kl)."""
+def _params(flat):
+    return [tuple(_f32c(t) for t in flat[i:i + 4]) for i in range(0, len(flat), 4)]
+
+
+def _save(ctx, **groups):
+    """ctx.save_for_backward of named groups, each a tensor (or None) or a list of them; _saved(ctx) returns them by
+    name."""
+    layout, tensors = [], []
+    for name, g in groups.items():
+        is_list = isinstance(g, (list, tuple))
+        layout.append((name, len(g) if is_list else None))
+        tensors += g if is_list else [g]
+    ctx.save_for_backward(*tensors)
+    ctx.saved_layout = layout
+
+
+def _saved(ctx):
+    sv, out, i = ctx.saved_tensors, {}, 0
+    for name, n in ctx.saved_layout:
+        out[name] = sv[i] if n is None else list(sv[i:i + n])
+        i += 1 if n is None else n
+    return out
+
+
+# =========================================================================================
+# layer level: one sample of one layer
+# =========================================================================================
+class _Linear(torch.autograd.Function):
+    """BayesianLinear.forward (networks.py:73-88) -> (y, log_prior, log_post), BayesianLinearLR.forward
+    (networks.py:116-138) -> (y, kl), for one sample."""
 
     @staticmethod
-    def forward(ctx, x, wm, wr, bm, br, sigma_p, sample, calc_kl, layer_id):
+    def forward(ctx, est, x, wm, wr, bm, br, sample, logprob, layer_id, tf32):
         L.require_cuda(x, wm, wr, bm, br)
-        inn, out = wm.shape
+        inn, out = est.shape(wm)
         x2 = _f32c(x).reshape(-1, inn)
         B = x2.shape[0]
         p = tuple(_f32c(t) for t in (wm, wr, bm, br))
-        eps = plan_eps([((B, out), (out,))], 1, x2.device, sample)
-        if eps.injected is not None:
+        eps = plan_eps(est.eps_shapes([p], B), 1, x2.device, sample)
+        if eps.injected is not None:            # re-key as layer `layer_id`
             eps.injected = {layer_id: eps.injected[0]}
-        kl = torch.zeros(1, dtype=torch.float64, device=x2.device)
+        acc = torch.zeros(est.acc_len(1), dtype=torch.float64, device=x2.device)
         y = torch.empty((1, B, out), dtype=torch.float32, device=x2.device)
-        delta = torch.empty_like(y) if sample else None
-        flags = (L.F_SAMPLE if sample else 0) | (L.F_LOGPROB if calc_kl else 0)
-        _lr_fwd(x2, 0, p, eps, layer_id, sigma_p, 1, B, flags, y, delta, kl)
-        saved = [x2, *p] + ([delta] if sample else []) + eps.tensors()
-        ctx.save_for_backward(*saved)
-        ctx.cfg = (sigma_p, sample, calc_kl, layer_id, eps, x.shape, x.requires_grad)
+        delta = torch.empty_like(y) if sample and est.has_delta else None
+        flags = (L.F_SAMPLE if sample else 0) | (L.F_LOGPROB if logprob else 0) | (L.F_TF32 if tf32 else 0)
+        est.fwd(x2, 0, p, eps, layer_id, 1, B, flags, y, delta, est.lp(acc, 1))
+        _save(ctx, x2=x2, p=p, delta=delta, eps=eps.tensors())
+        ctx.est, ctx.sample, ctx.logprob, ctx.layer_id, ctx.tf32, ctx.eps = est, sample, logprob, layer_id, tf32, eps
+        ctx.xshape, ctx.x_rg = x.shape, x.requires_grad
         ctx.set_materialize_grads(False)
-        return y.view(*x.shape[:-1], out), kl.to(torch.float32)[0]
+        lpq = acc.to(torch.float32)
+        return (y.view(*x.shape[:-1], out), *est.lp_outputs(lpq, 1, True))
 
     @staticmethod
-    def backward(ctx, dy, dkl):
-        sigma_p, sample, calc_kl, layer_id, eps, xshape, x_rg = ctx.cfg
-        sv = ctx.saved_tensors
-        x2, wm, wr, bm, br = sv[:5]
-        delta = sv[5] if sample else None
-        inn, out = wm.shape
+    def backward(ctx, dy, *dlp):
+        est, s = ctx.est, _saved(ctx)
+        x2, p = s['x2'], tuple(s['p'])
+        inn, out = est.shape(p[0])
         B = x2.shape[0]
         if dy is None:
             dy = torch.zeros((B, out), dtype=torch.float32, device=x2.device)
         dy = _f32c(dy).reshape(1, B, out)
-        g = tuple(torch.empty_like(t) for t in (wm, wr, bm, br))
-        dx = torch.empty((1, B, inn), dtype=torch.float32, device=x2.device) if x_rg else None
-        use_kl = calc_kl and dkl is not None
-        flags = (L.F_SAMPLE if sample else 0) | (L.F_LOGPROB if use_kl else 0) | (0 if x_rg else L.F_NO_DX)
-        g_kl_dev = _f32c(dkl).reshape(1) if use_kl else None
-        _lr_bwd(dy, None, x2, 0, (wm, wr, bm, br), eps, layer_id, delta, sigma_p, 1, B, flags, 1.0, g_kl_dev, None,
-                dx, g)
-        return (dx.view(xshape) if x_rg else None, g[0], g[1], g[2], g[3], None, None, None, None)
+        g = tuple(torch.empty_like(t) for t in p)
+        dx = torch.empty((1, B, inn), dtype=torch.float32, device=x2.device) if ctx.x_rg else None
+        gflags, gargs = est.grad_args(dlp, ctx.logprob, True)
+        flags = ((L.F_SAMPLE if ctx.sample else 0) | (L.F_TF32 if ctx.tf32 else 0) | (0 if ctx.x_rg else L.F_NO_DX) |
+                 gflags)
+        est.bwd(dy, x2, 0, p, ctx.eps, ctx.layer_id, s['delta'], 1, B, flags, gargs, None, dx, g)
+        return (None, dx.view(ctx.xshape) if ctx.x_rg else None, *g, None, None, None, None)
+
+
+def bayes_linear(x, wm, wr, bm, br, prior, sample, logprob, layer_id=0, tf32=False):
+    return _Linear.apply(_WeightSampling(prior), x, wm, wr, bm, br, sample, logprob, layer_id, tf32)
 
 
 def lr_linear(x, wm, wr, bm, br, sigma_p, sample, calc_kl, layer_id=0):
-    return _LRLinear.apply(x, wm, wr, bm, br, float(sigma_p), sample, calc_kl, layer_id)
+    return _Linear.apply(_LocalReparam(sigma_p), x, wm, wr, bm, br, sample, calc_kl, layer_id, False)
 
 
-def _lr_eps_shapes(params, B):
-    return [((B, p[0].shape[1]), (p[0].shape[1],)) for p in params]
-
-
-class _MLPForwardLR(torch.autograd.Function):
-    """S sampled forwards with LR layers -> outputs [S,B,C], kl [] (computed once, SURVEY B-8)."""
+# =========================================================================================
+# network level: S sampled forwards of the whole MLP, differentiable outputs
+# =========================================================================================
+class _NetworkForward(torch.autograd.Function):
+    """(x, params) -> outputs [S,B,C] and the log-prob outputs: log_prior [S], log_post [S] (weight sampling), or kl []
+    (local reparameterisation, computed once: SURVEY B-8)."""
 
     @staticmethod
-    def forward(ctx, x2, sigma_p, S, sample, calc_kl, tf32, *flat):
+    def forward(ctx, est, x2, S, sample, logprob, tf32, *flat):
         L.require_cuda(x2, *flat)
         x2 = _f32c(x2)
-        params = [tuple(_f32c(t) for t in flat[i:i + 4]) for i in range(0, len(flat), 4)]
-        eps = plan_eps(_lr_eps_shapes(params, x2.shape[0]), S, x2.device, sample)
-        kl = torch.zeros(1, dtype=torch.float64, device=x2.device)
-        ys, deltas = _net_lr_forward(x2, params, sigma_p, S, eps, sample, calc_kl, kl, tf32)
-        ctx.save_for_backward(x2, *flat, *ys, *[d for d in deltas if d is not None], *eps.tensors())
-        ctx.cfg = (sigma_p, S, sample, calc_kl, eps, len(params), x2.requires_grad)
-        ctx.tf32 = tf32
+        params = _params(flat)
+        eps = plan_eps(est.eps_shapes(params, x2.shape[0]), S, x2.device, sample)
+        acc = torch.zeros(est.acc_len(S), dtype=torch.float64, device=x2.device)
+        ys, deltas = _forward(est, x2, params, S, eps, sample, logprob, tf32, est.lp(acc, S))
+        _save(ctx, x2=x2, flat=flat, ys=ys, deltas=deltas, eps=eps.tensors())
+        ctx.est, ctx.S, ctx.sample, ctx.logprob, ctx.tf32, ctx.eps = est, S, sample, logprob, tf32, eps
+        ctx.x_rg = x2.requires_grad
         ctx.set_materialize_grads(False)
-        return ys[-1], kl.to(torch.float32)[0]
+        # the last layer's buffer is handed out; backward only needs the hidden pre-activations
+        return (ys[-1], *est.lp_outputs(acc.to(torch.float32), S, False))
 
     @staticmethod
-    def backward(ctx, d_out, dkl):
-        sigma_p, S, sample, calc_kl, eps, nl, x_rg = ctx.cfg
-        sv = ctx.saved_tensors
-        x2 = sv[0]
-        params = [tuple(_f32c(t) for t in sv[1 + 4 * i:5 + 4 * i]) for i in range(nl)]
-        ys = list(sv[1 + 4 * nl:1 + 5 * nl])
-        deltas = list(sv[1 + 5 * nl:1 + 6 * nl]) if sample else [None] * nl
+    def backward(ctx, d_out, *dlp):
+        est, s = ctx.est, _saved(ctx)
+        params = _params(s['flat'])
         if d_out is None:
-            d_out = torch.zeros_like(ys[-1])
-        use_kl = calc_kl and dkl is not None
-        g_kl_dev = _f32c(dkl).reshape(1) if use_kl else None
-        dx0, grads = _net_lr_backward(x2, ys, deltas, _f32c(d_out), params, sigma_p, S, eps, sample, use_kl, 1.0,
-                                      g_kl_dev, None, x_rg, ctx.tf32)
+            d_out = torch.zeros_like(s['ys'][-1])
+        pg = est.grad_args(dlp, ctx.logprob, False)
+        dx0, grads = _backward(est, s['x2'], s['ys'], s['deltas'], _f32c(d_out), params, ctx.S, ctx.eps, ctx.sample,
+                               ctx.tf32, pg, None, ctx.x_rg)
         flat = [g for lg in grads for g in lg]
-        return (dx0.sum(0) if x_rg else None, None, None, None, None, None, *flat)
+        return (None, dx0.sum(0) if ctx.x_rg else None, None, None, None, None, *flat)
+
+
+def _network_forward(est, x2, layers, S, sample, logprob, tf32):
+    return _NetworkForward.apply(est, x2, S, sample, logprob, tf32, *[t for layer in layers for t in layer])
+
+
+def mlp_forward(x2, layers, prior, S, sample=True, logprob=True, tf32=False):
+    return _network_forward(_WeightSampling(prior), x2, layers, S, sample, logprob, tf32)
 
 
 def mlp_forward_lr(x2, layers, sigma_p, S, sample=True, calc_kl=True, tf32=False):
-    flat = [t for layer in layers for t in layer]
-    return _MLPForwardLR.apply(x2, float(sigma_p), S, sample, calc_kl, tf32, *flat)
+    return _network_forward(_LocalReparam(sigma_p), x2, layers, S, sample, calc_kl, tf32)
 
 
-class _FusedELBOLR(torch.autograd.Function):
-    """sample_elbo_lr (networks.py:211-225): loss = beta * KL + NLL / S, KL evaluated once.  likelihood as in
-    _FusedELBO."""
+# =========================================================================================
+# fused ELBO: the network pass + likelihood + ELBO assembly, loss only differentiable
+# =========================================================================================
+def _nll_launch(out, target, S, B, Cc, sigma, mode, likelihood, nll, d_out):
+    """The likelihood and its gradient (scaled by 1/S) on the sampled outputs [S,B,Cc]: nll += ..., d_out written.
+    The heteroscedastic likelihood reads `sigma` as sigma_min and Cc = 2D outputs per row."""
+    if likelihood == 'heteroscedastic':
+        tgt = _f32c(target)            # (held: a contiguous copy must outlive the call)
+        L.check(L.lib().bbb_nll_gauss_het(L.ptr(out), L.ptr(tgt), float(sigma), S, B, Cc // 2, 1.0 / S, L.ptr(nll),
+                                          L.ptr(d_out), L.stream()), 'bbb_nll_gauss_het')
+    elif mode == 'classification':
+        L.check(L.lib().bbb_nll_ce(L.ptr(out), L.ptr(target), S, B, Cc, 1.0 / S, L.ptr(nll), L.ptr(d_out),
+                                   L.stream()), 'bbb_nll_ce')
+    else:
+        tgt = _f32c(target)
+        L.check(L.lib().bbb_nll_gauss(L.ptr(out), L.ptr(tgt), float(sigma), S, B, Cc, 1.0 / S, L.ptr(nll),
+                                      L.ptr(d_out), L.stream()), 'bbb_nll_gauss')
+
+
+class _ELBO(torch.autograd.Function):
+    """sample_elbo (networks.py:192-209) and sample_elbo_lr (networks.py:211-225): one launch per layer, then the
+    likelihood and the assembly of the ELBO, or the estimator's fused tail: the head (last layer + likelihood +
+    assembly in one launch) or ONE C call per pass (weight sampling, TF32, batch <= 128).  Only `loss` is
+    differentiable.  likelihood 'heteroscedastic' (sigma is then sigma_min) always takes the per-layer calls."""
 
     @staticmethod
-    def forward(ctx, x2, target, beta, S, sigma, mode, likelihood, sigma_p, tf32, *flat):
+    def forward(ctx, est, x2, target, beta, S, sigma, mode, likelihood, tf32, *flat):
         L.require_cuda(x2, target, *flat)
         x2 = _f32c(x2)
         dev = x2.device
-        params = [tuple(_f32c(t) for t in flat[i:i + 4]) for i in range(0, len(flat), 4)]
-        eps = plan_eps(_lr_eps_shapes(params, x2.shape[0]), S, dev, True)
-        acc = torch.zeros(2, dtype=torch.float64, device=dev)
-        kl, nll = acc[0:1], acc[1:2]
-        ys, deltas = _net_lr_forward(x2, params, sigma_p, S, eps, True, True, kl, tf32)
-        out = ys[-1]
-        B, Cc = out.shape[1], out.shape[2]
+        params = _params(flat)
+        B = x2.shape[0]
+        eps = plan_eps(est.eps_shapes(params, B), S, dev, True)
         need_grad = any(t.requires_grad for t in flat)
-        d_out = torch.empty_like(out) if need_grad else None
-        _nll_launch(out, target, S, B, Cc, sigma, mode, likelihood, nll, d_out)
         out4 = torch.empty(4, dtype=torch.float32, device=dev)
         beta_h, beta_d = _split_beta(beta)
-        L.check(L.lib().bbb_elbo_finalize(None, None, L.ptr(kl), L.ptr(nll), S, beta_h, L.ptr(beta_d), L.ptr(out4),
-                                          L.stream()), 'bbb_elbo_finalize')
+        ctx.used_network_call = est.network_call(params, S, B, mode, likelihood, tf32)
+        if ctx.used_network_call:
+            ys, dxs, d_out = est.network_forward(x2, target, params, eps, S, B, sigma, mode, need_grad, beta_h, beta_d,
+                                                 out4)
+            deltas = [None] * len(params)
+        else:
+            lp, nll, done, ys, deltas, dxs, d_out = est.elbo_workspace(params, S, B, need_grad, dev)
+            head = est.head(params, eps, S, B, mode, likelihood, target, sigma, d_out, lp, nll, beta_h, beta_d, out4,
+                            done)
+            _forward(est, x2, params, S, eps, True, True, tf32, lp, ys, deltas, head)
+            if head is None:
+                _nll_launch(ys[-1], target, S, B, ys[-1].shape[2], sigma, mode, likelihood, nll, d_out)
+                est.finalize(lp, nll, S, beta_h, beta_d, out4)
         if need_grad:
-            ctx.save_for_backward(x2, d_out, *flat, *ys[:-1], *deltas, *eps.tensors())
-        ctx.cfg = (sigma_p, S, beta_h, eps, len(params))
-        ctx.tf32 = tf32
-        ctx.set_materialize_grads(False)
-        ctx.beta_dev = beta_d
-        loss, klm, nl = out4[0:1], out4[1], out4[2:3]
-        ctx.mark_non_differentiable(klm, nl)
-        return loss, klm, nl
+            _save(ctx, x2=x2, d_out=d_out, flat=flat, ys=ys[:-1], deltas=deltas, eps=eps.tensors())
+            ctx.dxs = dxs
+        ctx.est, ctx.S, ctx.beta, ctx.beta_dev, ctx.tf32, ctx.eps = est, S, beta_h, beta_d, tf32, eps
+        ctx.n_flat = len(flat)
+        ctx.set_materialize_grads(False)      # no zero-filled gradients for the non-differentiable scalars
+        outs = est.elbo_outputs(out4)
+        ctx.mark_non_differentiable(*outs[1:])
+        return outs
 
     @staticmethod
     def backward(ctx, g_loss, *unused):
-        sigma_p, S, beta, eps, nl = ctx.cfg
+        est = ctx.est
         if g_loss is None:
-            return (None,) * (9 + 4 * nl)
-        if ctx.tf32 and getattr(ctx, 'consumed', False):
-            # the tcgen05 LR backward overwrites the saved delta buffers with dV (they have no other use in it)
-            raise RuntimeError('sample_elbo_lr: this graph was already differentiated (retain_graph=True is not supported '
-                               'by the TF32 local-reparameterisation path: its saved state is single-use)')
+            return (None,) * (9 + ctx.n_flat)
+        if est.single_use(ctx.tf32) and getattr(ctx, 'consumed', False):
+            raise RuntimeError(est.reuse_error)
         ctx.consumed = True
-        sv = ctx.saved_tensors
-        x2, d_out = sv[0], sv[1]
-        params = [tuple(_f32c(t) for t in sv[2 + 4 * i:6 + 4 * i]) for i in range(nl)]
-        o = 2 + 4 * nl
-        ys = list(sv[o:o + nl - 1]) + [None]
-        deltas = list(sv[o + nl - 1:o + 2 * nl - 1])
+        s = _saved(ctx)
+        params = _params(s['flat'])
         scale = _f32c(g_loss).reshape(1)
-        _, grads = _net_lr_backward(x2, ys, deltas, d_out, params, sigma_p, S, eps, True, True, beta, ctx.beta_dev,
-                                    scale, False, ctx.tf32)
-        flat = [g for lg in grads for g in lg]
-        return (None,) * 9 + tuple(flat)
+        pg = est.elbo_grad_args(ctx.beta, ctx.beta_dev, ctx.S)
+        if ctx.used_network_call:
+            grads = est.network_backward(s['x2'], s['ys'], ctx.dxs, s['d_out'], params, ctx.S, ctx.eps, pg[1], scale)
+        else:
+            _, grads = _backward(est, s['x2'], s['ys'], s['deltas'], s['d_out'], params, ctx.S, ctx.eps, True,
+                                 ctx.tf32, pg, scale, False, dxs=ctx.dxs)
+        return (None,) * 9 + tuple(g for lg in grads for g in lg)
+
+
+def _elbo(est, x2, target, beta, S, sigma, mode, layers, tf32, likelihood):
+    return _ELBO.apply(est, x2, target, beta, S, sigma, mode, likelihood, tf32, *[t for layer in layers for t in layer])
+
+
+def fused_elbo(x2, target, beta, S, sigma, mode, prior, layers, tf32=False, likelihood='gaussian'):
+    return _elbo(_WeightSampling(prior), x2, target, beta, S, sigma, mode, layers, tf32, likelihood)
 
 
 def fused_elbo_lr(x2, target, beta, S, sigma, mode, sigma_p, layers, tf32=False, likelihood='gaussian'):
-    flat = [t for layer in layers for t in layer]
-    return _FusedELBOLR.apply(x2, target, beta, S, sigma, mode, likelihood, float(sigma_p), tf32, *flat)
+    return _elbo(_LocalReparam(sigma_p), x2, target, beta, S, sigma, mode, layers, tf32, likelihood)
 
 
 # =========================================================================================
@@ -967,38 +977,38 @@ def predictive(x2, params, S, mode, target=None, sigma=1.0, n_bins=15, chunk_row
     _check_predictive_mode(mode)
     if (prior is None) == (sigma_p is None):
         raise ValueError('give exactly one of prior (weight sampling) and sigma_p (local reparameterisation)')
+    est = _WeightSampling(prior) if sigma_p is None else _LocalReparam(sigma_p)
+    return _predictive(est, x2, params, S, mode, target, sigma, n_bins, chunk_rows, tf32)
+
+
+def _predictive(est, x2, params, S, mode, target, sigma, n_bins, chunk_rows, tf32):
     L.require_cuda(x2, *[t for p in params for t in p])
     x2 = _f32c(x2)
     dev = x2.device
     B = x2.shape[0]
     params = [tuple(_f32c(t) for t in p) for p in params]
-    lr = sigma_p is not None
-    widths = [p[0].shape[1] if lr else p[0].shape[0] for p in params]
+    widths = [est.shape(p[0])[1] for p in params]
     Cc = widths[-1]
     tgt = _predictive_target(target, mode, B, Cc)
     mean, row_stats, pred, acc = _predictive_outputs(B, Cc, mode, n_bins, tgt, dev)
     if B == 0:
         return mean, row_stats, pred, acc
     if chunk_rows is None:
-        # (the local-reparameterisation forward also keeps a delta buffer per layer)
-        n_chunks = -(-B // predictive_chunk_rows(S, widths * (2 if lr else 1)))
+        # (counting the delta buffer of each layer, where the estimator keeps one)
+        n_chunks = -(-B // predictive_chunk_rows(S, widths * (2 if est.has_delta else 1)))
         chunk_rows = -(-B // n_chunks)
     chunk_rows = int(chunk_rows)
     if chunk_rows < 1:
         raise ValueError(f'chunk_rows must be >= 1, got {chunk_rows}')
-    if not lr:
-        eps = plan_eps([(tuple(p[0].shape), (p[0].shape[0],)) for p in params], S, dev, True)
+    eps = None if est.eps_per_row else plan_eps(est.eps_shapes(params, B), S, dev, True)
     scratch = torch.zeros(2 * S, dtype=torch.float64, device=dev)    # log-prob slots the forward does not fill
     for r0 in range(0, B, chunk_rows):
         r1 = min(B, r0 + chunk_rows)
         xc = x2[r0:r1]
         if xc.data_ptr() % 16:     # keep the 16-byte row loads (and so the kernel family) of an unchunked call
             xc = xc.clone()
-        if lr:
-            eps = plan_eps(_lr_eps_shapes(params, r1 - r0), S, dev, True)
-            ys, _ = _net_lr_forward(xc, params, float(sigma_p), S, eps, True, False, scratch[:1], tf32)
-        else:
-            ys = _net_ws_forward(xc, params, prior, S, eps, True, False, tf32, scratch[:S], scratch[S:])
+        ec = eps if eps is not None else plan_eps(est.eps_shapes(params, r1 - r0), S, dev, True)
+        ys, _ = _forward(est, xc, params, S, ec, True, False, tf32, est.lp(scratch, S))
         _predictive_launch(ys[-1], None if tgt is None else tgt[r0:r1], mode, sigma, n_bins, mean[r0:r1],
                            row_stats[r0:r1], None if pred is None else pred[r0:r1], acc)
         del ys                     # free this chunk's activations before the next chunk allocates its own

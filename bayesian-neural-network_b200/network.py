@@ -118,6 +118,7 @@ class BayesianNetwork(nn.Module):
             if i + 1 < self.n_layers:
                 setattr(self, f'l{i + 1}_act', nn.ReLU())
         self._prior = None if self.local_reparam else F.make_prior(self.prior_init, self.mixture_prior)
+        self._est = F._LocalReparam(self.prior_init[0]) if self.local_reparam else F._WeightSampling(self._prior)
 
     def layers(self):
         return [getattr(self, f'l{i + 1}') for i in range(self.n_layers)]
@@ -140,11 +141,7 @@ class BayesianNetwork(nn.Module):
         x2 = self._flat_input(x)
         params = [l.params() for l in self.layers()]
         with torch.no_grad():
-            if self.local_reparam:
-                outs, _ = F.mlp_forward_lr(x2, params, float(self.prior_init[0]), samples, True, False, self.tf32)
-            else:
-                outs, _, _ = F.mlp_forward(x2, params, self._prior, samples, True, False, self.tf32)
-        return outs
+            return F._network_forward(self._est, x2, params, samples, True, False, self.tf32)[0]
 
     def predict_proba(self, x, samples):
         """BNN_Classification.predict (class_task.py:81-87): softmax of every sampled forward, averaged."""
@@ -167,13 +164,10 @@ class BayesianNetwork(nn.Module):
         if self._het:
             self._check_no_sigma(sigma)
             mode, sigma = 'heteroscedastic', self.sigma_min
+        F._check_predictive_mode(mode)
         with torch.no_grad():
-            if self.local_reparam:
-                mean, rs, pred, acc = F.predictive(x2, params, samples, mode, target, sigma, n_bins, chunk_rows,
-                                                   sigma_p=float(self.prior_init[0]), tf32=self.tf32)
-            else:
-                mean, rs, pred, acc = F.predictive(x2, params, samples, mode, target, sigma, n_bins, chunk_rows,
-                                                   prior=self._prior, tf32=self.tf32)
+            mean, rs, pred, acc = F._predictive(self._est, x2, params, samples, mode, target, sigma, n_bins, chunk_rows,
+                                                self.tf32)
         log_pred = rs[:, -1] if target is not None else None
         if self._het:
             D = self.classes
@@ -271,23 +265,33 @@ class BayesianNetwork(nn.Module):
     def _flat_input(self, input):
         return input.view(-1, self.input_shape) if self.mode == 'classification' else input.reshape(-1, self.input_shape)
 
-    def sample_elbo(self, input, target, beta, samples, sigma=1.):
-        ''' Sample ELBO for BNN w/o Local Reparameterisation (networks.py:192-209) '''
-        assert self.local_reparam == False, 'sample_elbo() method returns loss for BNNs without local reparameterisation, alternatively use sample_elbo_lr()'
+    def _sample_elbo(self, input, target, beta, samples, sigma):
+        """The body both sample_elbo methods share -> (the fused path's result, None, None), or (None, the sampled
+        forward's log-prob outputs, the NLL summed over the samples) for the caller to assemble."""
         x2 = self._flat_input(input)
         params = [l.params() for l in self.layers()]
         if self._het:
             self._check_no_sigma(sigma)
             target = self._het_target(target, x2.shape[0])
             if self.fused:
-                return F.fused_elbo(x2, target, beta, samples, self.sigma_min, self.mode, self._prior, params,
-                                    self.tf32, likelihood=self.likelihood)
+                return F._elbo(self._est, x2, target, beta, samples, self.sigma_min, self.mode, params, self.tf32,
+                               self.likelihood), None, None
         elif self._fusable(x2, target):
-            return F.fused_elbo(x2, target, beta, samples, sigma, self.mode, self._prior, params, self.tf32)
-        outs, lps, lqs = F.mlp_forward(x2, params, self._prior, samples, True, True, self.tf32)
+            return F._elbo(self._est, x2, target, beta, samples, sigma, self.mode, params, self.tf32, 'gaussian'), \
+                None, None
+        outs, *lp = F._network_forward(self._est, x2, params, samples, True, True, self.tf32)
         negative_log_likelihood = torch.zeros(1, device=outs.device)
         for i in range(samples):
             negative_log_likelihood = negative_log_likelihood + self.get_nll(outs[i], target, sigma)
+        return None, lp, negative_log_likelihood
+
+    def sample_elbo(self, input, target, beta, samples, sigma=1.):
+        ''' Sample ELBO for BNN w/o Local Reparameterisation (networks.py:192-209) '''
+        assert self.local_reparam == False, 'sample_elbo() method returns loss for BNNs without local reparameterisation, alternatively use sample_elbo_lr()'
+        fused, lp, negative_log_likelihood = self._sample_elbo(input, target, beta, samples, sigma)
+        if fused is not None:
+            return fused
+        lps, lqs = lp
         log_prior = beta * lps.mean()
         log_variational_posterior = beta * lqs.mean()
         negative_log_likelihood = negative_log_likelihood / samples
@@ -297,21 +301,10 @@ class BayesianNetwork(nn.Module):
     def sample_elbo_lr(self, input, target, beta, samples, sigma=1.):
         ''' Sample ELBO for BNN w/ Local Reparameterisation (networks.py:211-225) '''
         assert self.local_reparam == True, 'sample_elbo_lr() method returns loss for BNNs with local reparameterisation, alternatively use sample_elbo()'
-        x2 = self._flat_input(input)
-        params = [l.params() for l in self.layers()]
-        sigma_p = float(self.prior_init[0])
-        if self._het:
-            self._check_no_sigma(sigma)
-            target = self._het_target(target, x2.shape[0])
-            if self.fused:
-                return F.fused_elbo_lr(x2, target, beta, samples, self.sigma_min, self.mode, sigma_p, params,
-                                       self.tf32, likelihood=self.likelihood)
-        elif self._fusable(x2, target):
-            return F.fused_elbo_lr(x2, target, beta, samples, sigma, self.mode, sigma_p, params, self.tf32)
-        outs, kl = F.mlp_forward_lr(x2, params, sigma_p, samples, True, True, self.tf32)
-        negative_log_likelihood = torch.zeros(1, device=outs.device)
-        for i in range(samples):
-            negative_log_likelihood = negative_log_likelihood + self.get_nll(outs[i], target, sigma)
+        fused, lp, negative_log_likelihood = self._sample_elbo(input, target, beta, samples, sigma)
+        if fused is not None:
+            return fused
+        kl, = lp
         negative_log_likelihood = negative_log_likelihood / samples
         loss = beta * kl + negative_log_likelihood
         return loss, kl, negative_log_likelihood

@@ -56,13 +56,14 @@ def test_lr_tf32_backward_kernels_alone_within_bound():
     x = torch.rand(B, dims[0], device=DEV)
     d_out = torch.randn(S, B, dims[-1], device=DEV) / B
     R.manual_seed(7, 0)
-    eps = F.plan_eps([((B, p[0].shape[1]), (p[0].shape[1],)) for p in params], S, x.device, True)
+    est = F._LocalReparam(1.0)
+    eps = F.plan_eps(est.eps_shapes(params, B), S, x.device, True)
     kl = torch.zeros(1, dtype=torch.float64, device=DEV)
-    ys, deltas = F._net_lr_forward(x, params, 1.0, S, eps, True, True, kl, True)
+    ys, deltas = F._forward(est, x, params, S, eps, True, True, True, (kl,))
     got = {}
     for tf32 in (False, True):
-        _, grads = F._net_lr_backward(x, [t.clone() for t in ys], [t.clone() for t in deltas], d_out.clone(), params,
-                                      1.0, S, eps, True, True, 0.1, None, None, False, tf32)
+        _, grads = F._backward(est, x, [t.clone() for t in ys], [t.clone() for t in deltas], d_out.clone(), params, S,
+                               eps, True, tf32, est.elbo_grad_args(0.1, None, S), None, False)
         got[tf32] = [[g.clone() for g in lg] for lg in grads]
     for la, lb in zip(got[True], got[False]):
         for a, b in zip(la, lb):

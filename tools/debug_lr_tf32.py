@@ -27,16 +27,28 @@ def rel(a, b):
     return float((a.double() - b.double()).abs().max() / b.double().abs().max())
 
 
+def run(est, params, tf32, beta):
+    """forward + backward of one estimator with the same Philox eps -> (ys, deltas, grads, log-prob accumulators)"""
+    R.manual_seed(7, 0)
+    eps = F.plan_eps(est.eps_shapes(params, B), S, x.device, True)
+    acc = torch.zeros(est.acc_len(S), dtype=torch.float64, device=dev)
+    ys, deltas = F._forward(est, x, params, S, eps, True, True, tf32, est.lp(acc, S))
+    ys, deltas = [t.clone() for t in ys], [None if t is None else t.clone() for t in deltas]
+    _, grads = backward(est, params, eps, ys, deltas, tf32, beta)
+    return ys, deltas, grads, acc
+
+
+def backward(est, params, eps, ys, deltas, tf32, beta):
+    _, grads = F._backward(est, x, [t.clone() for t in ys], [None if t is None else t.clone() for t in deltas],
+                           d_out.clone(), params, S, eps, True, tf32, est.elbo_grad_args(beta, None, S), None, False)
+    return None, [[g.clone() for g in lg] for lg in grads]
+
+
+lr = F._LocalReparam(1.0)
 res = {}
 for tf32 in (False, True):
-    R.manual_seed(7, 0)
-    eps = F.plan_eps([((B, p[0].shape[1]), (p[0].shape[1],)) for p in params], S, x.device, True)
-    kl = torch.zeros(1, dtype=torch.float64, device=dev)
-    ys, deltas = F._net_lr_forward(x, params, 1.0, S, eps, True, True, kl, tf32)
-    ys, deltas = [t.clone() for t in ys], [t.clone() for t in deltas]
-    _, grads = F._net_lr_backward(x, [t.clone() for t in ys], [t.clone() for t in deltas], d_out.clone(), params, 1.0, S, eps,
-                                  True, True, 0.1, None, None, False, tf32)
-    res[tf32] = (ys, deltas, [[g.clone() for g in lg] for lg in grads], float(kl))
+    ys, deltas, grads, kl = run(lr, params, tf32, 0.1)
+    res[tf32] = (ys, deltas, grads, float(kl))
 (y0, d0, g0, k0), (y1, d1, g1, k1) = res[False], res[True]
 print('kl', k0, k1)
 for l in range(len(params)):
@@ -45,12 +57,8 @@ for l in range(len(params)):
 
 # ---- backward kernels alone: both modes on the SAME stored forward (the TF32 one), so the ReLU masks are identical ----
 R.manual_seed(7, 0)
-eps = F.plan_eps([((B, p[0].shape[1]), (p[0].shape[1],)) for p in params], S, x.device, True)
-gb = {}
-for tf32 in (False, True):
-    _, grads = F._net_lr_backward(x, [t.clone() for t in y1], [t.clone() for t in d1], d_out.clone(), params, 1.0, S, eps,
-                                  True, True, 0.1, None, None, False, tf32)
-    gb[tf32] = [[g.clone() for g in lg] for lg in grads]
+eps = F.plan_eps(lr.eps_shapes(params, B), S, x.device, True)
+gb = {tf32: backward(lr, params, eps, y1, d1, tf32, 0.1)[1] for tf32 in (False, True)}
 print('backward kernels on identical forward state:')
 for l in range(len(params)):
     print(f'layer {l}: ' + '  '.join(f'{n} {rel(a, b):.2e}' for n, a, b in zip(('g_w_mu', 'g_w_rho', 'g_b_mu', 'g_b_rho'), gb[True][l], gb[False][l])))
@@ -58,17 +66,12 @@ flips = [float(((a > 0) != (b > 0)).float().mean()) for a, b in zip(y1[:-1], y0[
 print('fraction of hidden units whose ReLU mask differs between the two forwards:', flips)
 
 # ---- the same experiment on the weight-sampling estimator (same shapes, [out, in] weights) --------------------------
-prior = F.make_prior([0.5, 0, -8], True)
+ws = F._WeightSampling(F.make_prior([0.5, 0, -8], True))
 wparams = [tuple(t.t().contiguous() if t.dim() == 2 else t for t in p) for p in params]
 wres = {}
 for tf32 in (False, True):
-    R.manual_seed(7, 0)
-    eps = F.plan_eps([(tuple(p[0].shape), (p[0].shape[0],)) for p in wparams], S, x.device, True)
-    acc = torch.zeros(2 * S, dtype=torch.float64, device=dev)
-    ys = [t.clone() for t in F._net_ws_forward(x, wparams, prior, S, eps, True, True, tf32, acc[:S], acc[S:])]
-    _, grads = F._net_ws_backward(x, [t.clone() for t in ys], d_out.clone(), wparams, prior, S, eps, True, tf32, 0.0, 0.0,
-                                  None, None, 0, None, False)
-    wres[tf32] = (ys, [[g.clone() for g in lg] for lg in grads])
+    ys, _, grads, _ = run(ws, wparams, tf32, 0.0)
+    wres[tf32] = (ys, grads)
 print('weight-sampling estimator, fp32 kernels vs tcgen05 kernels:')
 for l in range(len(wparams)):
     print(f'layer {l}: y {rel(wres[True][0][l], wres[False][0][l]):.2e}  '

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Warm and cold (L2-flushed) CUDA-event timings of the layer kernels through the C ABI, one layer at a time, with the
-flags the per-layer host path (functional._net_ws_forward / _net_ws_backward) passes in TF32 mode.
+flags the per-layer host path (functional._forward / _backward with weight sampling) passes in TF32 mode.
 usage: python tools/time_layers.py [B S [d0 d1 ... dn]]
 The widths d0 .. dn name a network (default: the MNIST shape 784 1200 1200 10); its first layer reads the shared network
 input and hands no dx down, the others read the stored pre-activation of the layer below.  BBB_LIB selects the library."""
