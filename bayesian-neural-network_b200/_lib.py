@@ -39,6 +39,15 @@ class MlpLayer(C.Structure):
                 ('g_w_mu', C.c_void_p), ('g_w_rho', C.c_void_p), ('g_b_mu', C.c_void_p), ('g_b_rho', C.c_void_p)]
 
 
+class GaussPriorTensor(C.Structure):
+    """struct bbb_gauss_prior_tensor: one weight or bias tensor of a per-weight Gaussian prior call"""
+    _fields_ = [('mu', C.c_void_p), ('rho', C.c_void_p), ('prior_mu', C.c_void_p), ('prior_rho', C.c_void_p),
+                ('eps', C.c_void_p), ('grad_mu', C.c_void_p), ('grad_rho', C.c_void_p), ('n', C.c_int64),
+                ('tensor_id', C.c_uint32)]
+
+
+GAUSS_PRIOR_MAX_TENSORS = 64
+
 P, I64, I32, F32, F64, U32, U64 = C.c_void_p, C.c_int64, C.c_int32, C.c_float, C.c_double, C.c_uint32, C.c_uint64
 _SIGS = {
     'bbb_version': ([], C.c_int),
@@ -52,6 +61,10 @@ _SIGS = {
                            P, P, P, P, P, P], C.c_int),
     'bbb_logprob_reduce': ([P, P, P, U64, U32, U32, U32, P, I64, I32, P, P, P, P], C.c_int),
     'bbb_kl_gauss': ([P, P, F32, I64, P, P], C.c_int),
+    'bbb_gauss_prior_logprob': ([P, I32, I64, P, P, P, P], C.c_int),
+    'bbb_gauss_prior_logprob_bwd': ([P, I32, I64, P, F32, F32, P, P, I64, P, P], C.c_int),
+    'bbb_gauss_prior_kl': ([P, I32, P, P], C.c_int),
+    'bbb_gauss_prior_kl_bwd': ([P, I32, F32, P, P, P], C.c_int),
     'bbb_philox_fill_normal': ([P, I64, U64, U32, U32, U32, P], C.c_int),
     'bbb_snr': ([P, P, I64, P, P], C.c_int),
     'bbb_snr_prune': ([P, P, I64, F32, P, P], C.c_int),

@@ -4,6 +4,9 @@
 // Roofline: HBM.  bbb_logprob_reduce reads 8 B/weight (mu, rho; +4 with injected eps, +4 when W is
 // written) and does ~60 flops + Philox per weight; bbb_kl_gauss reads 8 B/weight.  Loads are 16-byte
 // vectors, four independent vectors in flight per thread, grid = a multiple of the 148 SMs.
+// bbb_gauss_prior_logprob / bbb_gauss_prior_kl (per-weight priors) read 16 B/parameter (mu, rho, prior mu, prior rho;
+// +4 S with injected eps), the log-prob call once per group of 8 samples (one group for S <= 8); their backward calls
+// read the same 16 B and read-modify-write both gradients: 32 B/parameter (+4 S injected).
 #include <stdarg.h>
 
 #include <atomic>
@@ -255,7 +258,231 @@ __global__ void __launch_bounds__(128) softmax_mean_kernel(const float *__restri
   }
 }
 
+// ---- per-weight Gaussian priors p = N(m, sp^2), sp = softplus(r) (bbb_gauss_prior_*) ------------------------------------
+// One launch streams every tensor of a network: the table travels by value in the kernel parameters (4.4 KB, the
+// large-parameter launch of CUDA 12.1+), each thread takes quads (4 consecutive elements) of each tensor in turn with
+// a grid stride.  A tensor whose pointers are 16-byte aligned (and, with injected eps, whose n is a multiple of 4, so
+// every eps row is) uses float4 loads; otherwise, and for the n % 4 tail, scalar loads of the valid elements.
+// Every term is formed from (w - m)/sp, (mu - m)/sp and sigma/sp, so sigma, sp ~ 1e-5 stay finite.
+constexpr int kGpMax = BBB_GAUSS_PRIOR_MAX_TENSORS;
+constexpr int kGpS = 8;   // samples per CTA row of the log-prob kernel: their partial sums live in registers
+struct GpTable {
+  const float *mu[kGpMax], *rho[kGpMax], *pm[kGpMax], *pr[kGpMax], *eps[kGpMax];
+  float *gm[kGpMax], *gr[kGpMax];
+  int64_t n[kGpMax];
+  uint32_t id[kGpMax];
+  bool vec[kGpMax];
+  int nt;
+};
+
+__device__ __forceinline__ void ld4_rw(const float *p, int64_t i, int valid, bool vec, float v[4]) {
+  if (vec && valid == 4) {
+    const float4 t = *reinterpret_cast<const float4 *>(p + i);
+    v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
+  } else {
+#pragma unroll
+    for (int j = 0; j < 4; ++j) v[j] = j < valid ? p[i + j] : 0.0f;
+  }
+}
+__device__ __forceinline__ void st4(float *p, int64_t i, int valid, bool vec, const float v[4]) {
+  if (vec && valid == 4) {
+    *reinterpret_cast<float4 *>(p + i) = make_float4(v[0], v[1], v[2], v[3]);
+  } else {
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+      if (j < valid) p[i + j] = v[j];
+  }
+}
+// the eps of the 4 elements of quad q, sample `smp` (index s of the call): injected row s, or Philox exactly as the
+// layer kernels draw it (the linear-index quad mapping of logprob_reduce_kernel)
+__device__ __forceinline__ void gp_eps(const GpTable &t, int k, const RngDev &rng, int64_t s, int64_t q, int valid,
+                                       float e[4]) {
+  if (t.eps[k]) ld4(t.eps[k] + s * t.n[k], q << 2, valid, t.vec[k], e);
+  else philox_normal4(rng, t.id[k], rng.sample_base + (uint32_t)s, (uint32_t)q, e);
+}
+
+// logp[s] += sum log N(w_s; m, sp^2), logq[s] += sum log N(w_s; mu, sigma^2) for the kGpS samples of blockIdx.y
+__global__ void __launch_bounds__(RT, 2) gauss_prior_logprob_kernel(const GpTable t, int64_t S, RngDev rng, double *logp,
+                                                                 double *logq) {
+  pdl_launch_dependents();
+  pdl_wait();
+  __shared__ float red[64];
+  rng_resolve(rng);
+  const int64_t s0 = (int64_t)blockIdx.y * kGpS;
+  const int ns = (int)(S - s0 < kGpS ? S - s0 : kGpS);
+  float lp[kGpS], lq[kGpS];
+#pragma unroll
+  for (int j = 0; j < kGpS; ++j) lp[j] = lq[j] = 0.0f;
+  const int64_t stride = (int64_t)gridDim.x * RT;
+  for (int k = 0; k < t.nt; ++k) {
+    const int64_t n = t.n[k], nq = (n + 3) >> 2;
+    for (int64_t q = (int64_t)blockIdx.x * RT + threadIdx.x; q < nq; q += stride) {
+      const int valid = (int)(n - (q << 2) < 4 ? n - (q << 2) : 4);
+      float m[4], r[4], pm[4], pr[4];
+      ld4(t.mu[k], q << 2, valid, t.vec[k], m);
+      ld4(t.rho[k], q << 2, valid, t.vec[k], r);
+      ld4(t.pm[k], q << 2, valid, t.vec[k], pm);
+      ld4(t.pr[k], q << 2, valid, t.vec[k], pr);
+      // cp, cq: the sample-independent parts of the quad's log p and log q, -sum (log sp + log(2 pi)/2) and
+      // -sum (log sigma + log(2 pi)/2)
+      float sg[4], isp[4], cp = 0.0f, cq = 0.0f;
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        sg[j] = softplus_f(r[j]);
+        const float sp = softplus_f(pr[j]);
+        isp[j] = 1.0f / sp;
+        if (j < valid) {
+          cp -= kHalfLog2Pi + logf(sp);
+          cq -= kHalfLog2Pi + logf(sg[j]);
+        }
+      }
+#pragma unroll
+      for (int js = 0; js < kGpS; ++js) {
+        if (js < ns) {
+          float e[4];
+          gp_eps(t, k, rng, s0 + js, q, valid, e);
+          float ap = 0.0f, aq = 0.0f;
+#pragma unroll
+          for (int j = 0; j < 4; ++j) {
+            if (j < valid) {
+              const float w = __fadd_rn(m[j], __fmul_rn(sg[j], e[j]));
+              const float a = (w - pm[j]) * isp[j];
+              ap = fmaf(a, a, ap);
+              aq = fmaf(e[j], e[j], aq);
+            }
+          }
+          lp[js] += fmaf(-0.5f, ap, cp);
+          lq[js] += fmaf(-0.5f, aq, cq);
+        }
+      }
+    }
+  }
+#pragma unroll
+  for (int js = 0; js < kGpS; ++js)
+    if (js < ns) block_sum2_atomic(lp[js], lq[js], red, logp + s0 + js, logq + s0 + js);
+}
+
+// grad_mu += c sum_s gp_s (-(w_s - m)/sp^2),  grad_rho += c sigmoid(rho) sum_s [gp_s (-(w_s - m)/sp^2) eps_s - gq_s/sigma]
+__global__ void __launch_bounds__(RT) gauss_prior_logprob_bwd_kernel(const GpTable t, int64_t S, RngDev rng, float gp,
+                                                                     float gq, const float *gp_dev,
+                                                                     const float *gq_dev, int64_t gstride,
+                                                                     const float *out_scale_dev) {
+  pdl_launch_dependents();
+  pdl_wait();
+  rng_resolve(rng);
+  const float c = out_scale_dev ? __ldg(out_scale_dev) : 1.0f;
+  const int64_t stride = (int64_t)gridDim.x * RT;
+  for (int k = 0; k < t.nt; ++k) {
+    const int64_t n = t.n[k], nq = (n + 3) >> 2;
+    for (int64_t q = (int64_t)blockIdx.x * RT + threadIdx.x; q < nq; q += stride) {
+      const int64_t i = q << 2;
+      const int valid = (int)(n - i < 4 ? n - i : 4);
+      float m[4], r[4], pm[4], pr[4];
+      ld4(t.mu[k], i, valid, t.vec[k], m);
+      ld4(t.rho[k], i, valid, t.vec[k], r);
+      ld4(t.pm[k], i, valid, t.vec[k], pm);
+      ld4(t.pr[k], i, valid, t.vec[k], pr);
+      float sg[4], isp[4], gm[4], gr[4];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        sg[j] = softplus_f(r[j]);
+        isp[j] = 1.0f / softplus_f(pr[j]);
+        gm[j] = gr[j] = 0.0f;
+      }
+      float gq_sum = 0.0f;
+      for (int64_t s = 0; s < S; ++s) {
+        const float gps = gp_dev ? gp * __ldg(gp_dev + s * gstride) : gp;
+        gq_sum += gq_dev ? gq * __ldg(gq_dev + s * gstride) : gq;
+        float e[4];
+        gp_eps(t, k, rng, s, q, valid, e);
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          const float w = __fadd_rn(m[j], __fmul_rn(sg[j], e[j]));
+          const float tt = -gps * ((w - pm[j]) * isp[j]) * isp[j];
+          gm[j] += tt;
+          gr[j] = fmaf(tt, e[j], gr[j]);
+        }
+      }
+      float om[4], orh[4];
+      ld4_rw(t.gm[k], i, valid, t.vec[k], om);
+      ld4_rw(t.gr[k], i, valid, t.vec[k], orh);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        om[j] = fmaf(c, gm[j], om[j]);
+        orh[j] = fmaf(c * sigmoid_f(r[j]), gr[j] - gq_sum / sg[j], orh[j]);
+      }
+      st4(t.gm[k], i, valid, t.vec[k], om);
+      st4(t.gr[k], i, valid, t.vec[k], orh);
+    }
+  }
+}
+
+// The scale part of one element's KL, (u^2 - 1)/2 - log u with u = sigma/sp and v = u - 1 = (sigma - sp)/sp (formed
+// from the difference, exact near u = 1).  For |v| < 0.1 the closed form cancels; there it is the series
+// v^2 - v^3/3 + v^4/4 - ... to v^9 (truncation < 1e-8 relative), exactly 0 at v = 0.
+__device__ __forceinline__ float kl_scale_term(float u, float v) {
+  if (fabsf(v) >= 0.1f) return fmaf(0.5f * u, u, -0.5f) - logf(u);
+  float p = -1.0f / 9.0f;
+  p = fmaf(p, v, 1.0f / 8.0f);
+  p = fmaf(p, v, -1.0f / 7.0f);
+  p = fmaf(p, v, 1.0f / 6.0f);
+  p = fmaf(p, v, -1.0f / 5.0f);
+  p = fmaf(p, v, 1.0f / 4.0f);
+  p = fmaf(p, v, -1.0f / 3.0f);
+  p = fmaf(p, v, 1.0f);
+  return p * v * v;
+}
+
+// bwd == false: *kl += sum [f(v) + d^2/2], v = (sigma - sp)/sp, d = (mu - m)/sp  (= log(sp/sigma) + (sigma^2 +
+// (mu - m)^2)/(2 sp^2) - 1/2);  bwd == true: grad_mu += c d/sp, grad_rho += c sigmoid(rho) v (1/sp + 1/sigma)
+// (= c sigmoid(rho) (sigma/sp^2 - 1/sigma)).  q == p gives v = d = 0: exactly zero terms and gradients.
+template <bool kBwd>
+__global__ void __launch_bounds__(RT) gauss_prior_kl_kernel(const GpTable t, double *kl, float g_kl,
+                                                            const float *g_kl_dev, const float *out_scale_dev) {
+  pdl_launch_dependents();
+  pdl_wait();
+  __shared__ float red[64];
+  float c = 0.0f;
+  if (kBwd) c = g_kl * (g_kl_dev ? __ldg(g_kl_dev) : 1.0f) * (out_scale_dev ? __ldg(out_scale_dev) : 1.0f);
+  float acc = 0.0f;
+  const int64_t stride = (int64_t)gridDim.x * RT;
+  for (int k = 0; k < t.nt; ++k) {
+    const int64_t n = t.n[k], nq = (n + 3) >> 2;
+    for (int64_t q = (int64_t)blockIdx.x * RT + threadIdx.x; q < nq; q += stride) {
+      const int64_t i = q << 2;
+      const int valid = (int)(n - i < 4 ? n - i : 4);
+      float m[4], r[4], pm[4], pr[4];
+      ld4(t.mu[k], i, valid, t.vec[k], m);
+      ld4(t.rho[k], i, valid, t.vec[k], r);
+      ld4(t.pm[k], i, valid, t.vec[k], pm);
+      ld4(t.pr[k], i, valid, t.vec[k], pr);
+      float om[4], orh[4];
+      if (kBwd) {
+        ld4_rw(t.gm[k], i, valid, t.vec[k], om);
+        ld4_rw(t.gr[k], i, valid, t.vec[k], orh);
+      }
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const float sg = softplus_f(r[j]), sp = softplus_f(pr[j]);
+        const float v = __fdiv_rn(sg - sp, sp), d = __fdiv_rn(m[j] - pm[j], sp);
+        if (kBwd) {
+          om[j] = fmaf(c, __fdiv_rn(d, sp), om[j]);
+          orh[j] = fmaf(c * sigmoid_f(r[j]), v * (__fdiv_rn(1.0f, sp) + __fdiv_rn(1.0f, sg)), orh[j]);
+        } else if (j < valid) {
+          acc += fmaf(0.5f * d, d, kl_scale_term(__fdiv_rn(sg, sp), v));
+        }
+      }
+      if (kBwd) {
+        st4(t.gm[k], i, valid, t.vec[k], om);
+        st4(t.gr[k], i, valid, t.vec[k], orh);
+      }
+    }
+  }
+  if (!kBwd) block_sum2_atomic(acc, 0.0f, red, kl, nullptr);
+}
+
 inline int grid_for(int64_t work_items, int per_cta) {
+
   int64_t need = (work_items + per_cta - 1) / per_cta;
   int64_t cap = (int64_t)sm_count() * 8;  // 8 resident CTAs of 256 threads per SM
   if (need < 1) need = 1;
@@ -300,6 +527,89 @@ extern "C" int bbb_kl_gauss(const float *mu, const float *rho, float sigma_p, in
   if (n == 0) return BBB_OK;
   kl_gauss_kernel<<<grid_for(n >> 2, RT * 4), RT, 0, (cudaStream_t)stream>>>(
       mu, rho, logf(sigma_p), 1.0f / (sigma_p * sigma_p), n, kl);
+  BBB_CHECK_LAUNCH();
+  return BBB_OK;
+}
+
+namespace bbb { namespace {
+// the by-value kernel table of a bbb_gauss_prior_* call, and the quads it covers (0: nothing to launch); BBB_EINVAL
+// for a bad table (see bbb.h)
+int gp_table(const bbb_gauss_prior_tensor *t, int32_t n_tensors, bool bwd, GpTable &g, int64_t &quads) {
+  BBB_CHECK_ARG(n_tensors >= 0 && n_tensors <= kGpMax, "n_tensors outside [0, 64]");
+  BBB_CHECK_ARG(t || n_tensors == 0, "null tensor table");
+  g.nt = 0;
+  quads = 0;
+  for (int32_t k = 0; k < n_tensors; ++k) {
+    const bbb_gauss_prior_tensor &x = t[k];
+    BBB_CHECK_ARG(x.n >= 0, "negative size");
+    if (x.n == 0) continue;
+    BBB_CHECK_ARG(x.mu && x.rho && x.prior_mu && x.prior_rho, "null mu / rho / prior_mu / prior_rho");
+    BBB_CHECK_ARG(!bwd || (x.grad_mu && x.grad_rho), "null grad_mu / grad_rho");
+    const int i = g.nt++;
+    g.mu[i] = x.mu; g.rho[i] = x.rho; g.pm[i] = x.prior_mu; g.pr[i] = x.prior_rho; g.eps[i] = x.eps;
+    g.gm[i] = bwd ? x.grad_mu : nullptr; g.gr[i] = bwd ? x.grad_rho : nullptr;
+    g.n[i] = x.n;
+    g.id[i] = x.tensor_id;
+    g.vec[i] = aligned16(x.mu) && aligned16(x.rho) && aligned16(x.prior_mu) && aligned16(x.prior_rho) &&
+               (!x.eps || (aligned16(x.eps) && x.n % 4 == 0)) && (!bwd || (aligned16(x.grad_mu) && aligned16(x.grad_rho)));
+    quads += (x.n + 3) >> 2;
+  }
+  return BBB_OK;
+}
+} }
+
+extern "C" int bbb_gauss_prior_logprob(const bbb_gauss_prior_tensor *t, int32_t n_tensors, int64_t S,
+                                       const bbb_rng *rng, double *logp, double *logq, void *stream) {
+  BBB_CHECK_ARG(S > 0, "S <= 0");
+  BBB_CHECK_ARG(rng && logp && logq, "null rng / logp / logq");
+  GpTable g;
+  int64_t quads;
+  if (int st = gp_table(t, n_tensors, false, g, quads)) return st;
+  if (quads == 0) return BBB_OK;
+  BBB_CHECK_CUDA(launch_pdl(gauss_prior_logprob_kernel, dim3(grid_for(quads, RT), (unsigned)((S + kGpS - 1) / kGpS)),
+                            dim3(RT), 0, (cudaStream_t)stream, g, S, make_rng_dev(rng), logp, logq));
+  BBB_CHECK_LAUNCH();
+  return BBB_OK;
+}
+
+extern "C" int bbb_gauss_prior_logprob_bwd(const bbb_gauss_prior_tensor *t, int32_t n_tensors, int64_t S,
+                                           const bbb_rng *rng, float gp, float gq, const float *gp_dev,
+                                           const float *gq_dev, int64_t g_dev_stride, const float *out_scale_dev,
+                                           void *stream) {
+  BBB_CHECK_ARG(S > 0, "S <= 0");
+  BBB_CHECK_ARG(rng, "null rng");
+  BBB_CHECK_ARG(g_dev_stride >= 0, "negative g_dev_stride");
+  GpTable g;
+  int64_t quads;
+  if (int st = gp_table(t, n_tensors, true, g, quads)) return st;
+  if (quads == 0) return BBB_OK;
+  BBB_CHECK_CUDA(launch_pdl(gauss_prior_logprob_bwd_kernel, dim3(grid_for(quads, RT)), dim3(RT), 0,
+                            (cudaStream_t)stream, g, S, make_rng_dev(rng), gp, gq, gp_dev, gq_dev, g_dev_stride,
+                            out_scale_dev));
+  BBB_CHECK_LAUNCH();
+  return BBB_OK;
+}
+
+extern "C" int bbb_gauss_prior_kl(const bbb_gauss_prior_tensor *t, int32_t n_tensors, double *kl, void *stream) {
+  BBB_CHECK_ARG(kl, "null kl");
+  GpTable g;
+  int64_t quads;
+  if (int st = gp_table(t, n_tensors, false, g, quads)) return st;
+  if (quads == 0) return BBB_OK;
+  BBB_CHECK_CUDA(launch_pdl(gauss_prior_kl_kernel<false>, dim3(grid_for(quads, RT)), dim3(RT), 0, (cudaStream_t)stream,
+                            g, kl, 0.0f, (const float *)nullptr, (const float *)nullptr));
+  BBB_CHECK_LAUNCH();
+  return BBB_OK;
+}
+
+extern "C" int bbb_gauss_prior_kl_bwd(const bbb_gauss_prior_tensor *t, int32_t n_tensors, float g_kl,
+                                      const float *g_kl_dev, const float *out_scale_dev, void *stream) {
+  GpTable g;
+  int64_t quads;
+  if (int st = gp_table(t, n_tensors, true, g, quads)) return st;
+  if (quads == 0) return BBB_OK;
+  BBB_CHECK_CUDA(launch_pdl(gauss_prior_kl_kernel<true>, dim3(grid_for(quads, RT)), dim3(RT), 0, (cudaStream_t)stream,
+                            g, (double *)nullptr, g_kl, g_kl_dev, out_scale_dev));
   BBB_CHECK_LAUNCH();
   return BBB_OK;
 }

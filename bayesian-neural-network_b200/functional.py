@@ -147,6 +147,36 @@ def plan_eps(shapes, S, device, sample=True):
 
 
 # =========================================================================================
+# per-weight Gaussian priors p(w) = N(m, softplus(r)^2) (bbb_gauss_prior_*)
+# =========================================================================================
+def _gauss_prior_table(params, gauss, eps, sample, S, grads=None, layer_ids=None):
+    """The tensor table of a bbb_gauss_prior_* call: every layer's weight and bias with its prior (gauss[l] =
+    (weight m, weight r, bias m, bias r)), eps (injected, zeros for an unsampled call, or Philox: NULL) and, for a
+    backward, the gradient views it adds into.  Returns (table, count, tensors the call must keep alive)."""
+    n = 2 * len(params)
+    if n > L.GAUSS_PRIOR_MAX_TENSORS:
+        raise ValueError(f'a per-weight prior covers at most {L.GAUSS_PRIOR_MAX_TENSORS // 2} layers, got {n // 2}')
+    tab, keep = (L.GaussPriorTensor * n)(), []
+    for l, (p, pr) in enumerate(zip(params, gauss)):
+        lid = l if layer_ids is None else layer_ids[l]
+        inj = eps.ptrs(lid)
+        for j in (0, 1):
+            t = tab[2 * l + j]
+            t.mu, t.rho = p[2 * j].data_ptr(), p[2 * j + 1].data_ptr()
+            t.prior_mu, t.prior_rho = pr[2 * j].data_ptr(), pr[2 * j + 1].data_ptr()
+            t.n, t.tensor_id = p[2 * j].numel(), 2 * lid + j
+            if not sample:                   # w = mu: log-probs of the mean weights
+                z = torch.zeros((S, t.n), dtype=torch.float32, device=p[0].device)
+                keep.append(z)
+                t.eps = z.data_ptr()
+            else:
+                t.eps = inj[j]
+            if grads is not None:
+                t.grad_mu, t.grad_rho = grads[l][2 * j].data_ptr(), grads[l][2 * j + 1].data_ptr()
+    return tab, n, keep
+
+
+# =========================================================================================
 # the two estimators: everything that differs between their C-ABI families
 # =========================================================================================
 def _zeroed_views(shapes, device):
@@ -221,11 +251,13 @@ def _mlp_layer_table(params, eps, ys, dzs, grads):
     return tab
 
 
-def _mlp_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, need_grad, beta_h, beta_d, out4):
+def _mlp_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, need_grad, beta_h, beta_d, out4,
+                      gauss_fwd=None):
     """sample_elbo's forward as ONE C call (bbb_mlp_fwd): TMA-fed tcgen05 kernels for the hidden layers + the fused
     head.  Returns (ys, dxs, d_out): ys[l] the pre-activation output of layer l (the hidden ones live in the zero-filled
     workspace: their split-K partial tiles are reduce-added into it), dxs[l] the zero-filled gradient buffer w.r.t.
-    layer l's pre-activation input."""
+    layer l's pre-activation input.  gauss_fwd(logp, logq), when given, adds the per-weight prior terms to the zeroed
+    accumulators before the call, which then runs without BBB_F_LOGPROB: its head assembles the four scalars from them."""
     dev = x2.device
     nl = len(params)
     hidden = [p[0].shape[0] for p in params[:-1]]
@@ -245,9 +277,11 @@ def _mlp_forward_call(x2, target, params, eps, prior, S, B, sigma, mode, need_gr
     tab = _mlp_layer_table(params, eps, ys, list(dzs) + [d_out], None)
     kind = L.NLL_CE if mode == 'classification' else L.NLL_GAUSS
     tgt = target if mode == 'classification' else _f32c(target)
+    if gauss_fwd is not None:
+        gauss_fwd(logp, logq)
     rng = eps.rng(0)
     L.check(L.lib().bbb_mlp_fwd(tab, nl, L.ptr(x2), S, B, C.byref(rng), C.byref(prior),
-                                L.F_SAMPLE | L.F_LOGPROB | L.F_TF32, kind, L.ptr(tgt), float(sigma), 1.0 / S,
+                                L.F_SAMPLE | (0 if gauss_fwd is not None else L.F_LOGPROB) | L.F_TF32, kind, L.ptr(tgt), float(sigma), 1.0 / S,
                                 L.ptr(d_out), L.ptr(logp), L.ptr(logq), L.ptr(nll), beta_h, L.ptr(beta_d),
                                 L.ptr(out4), L.ptr(done), L.stream()), 'bbb_mlp_fwd')
     return ys, ([None] + list(dzs) if need_grad else None), d_out
@@ -262,7 +296,7 @@ class _WeightSampling:
     """Weight sampling (networks.py:48-88, 192-209): weights [out, in] sampled per sample, log prior and log posterior
     of the sampled weights accumulated per sample (2S fp64 values), their gradient taken through the prior-gradient
     scalars gp / gq of the backward (BBB_F_LOGPROB is a forward flag only)."""
-    __slots__ = ('prior',)
+    __slots__ = ('prior', 'gauss')
     has_delta = False            # no per-layer buffer besides the output
     eps_per_row = False          # one eps per weight: every input row sees the same S networks
     reuse_error = ('sample_elbo: this graph was already differentiated (retain_graph=True is not supported by the '
@@ -270,8 +304,36 @@ class _WeightSampling:
     prezero = staticmethod(_prezero)
     relu_out = staticmethod(_relu_out_layers)
 
-    def __init__(self, prior):
+    def __init__(self, prior, gauss=None):
         self.prior = prior
+        self.gauss = gauss       # per layer (weight m, weight r, bias m, bias r) of a per-weight prior, or None
+
+    def with_gauss(self, gauss):
+        """This estimator with the per-weight Gaussian prior `gauss` in place of the shared prior (None: as is)."""
+        return self if gauss is None else _WeightSampling(self.prior, gauss)
+
+    @staticmethod
+    def layer_grad_args(pg):
+        """The prior-gradient arguments of the layer calls when the per-weight prior kernels take the prior terms:
+        gp = gq = 0, no device multipliers."""
+        gflags, gargs = pg
+        return gflags, (0.0, 0.0, None, None, gargs[4])
+
+    def gauss_fwd(self, params, eps, S, sample, lp, layer_ids=None):
+        tab, n, keep = _gauss_prior_table(params, self.gauss, eps, sample, S, layer_ids=layer_ids)
+        rng = eps.rng(0)
+        L.check(L.lib().bbb_gauss_prior_logprob(tab, n, S, C.byref(rng), L.ptr(lp[0]), L.ptr(lp[1]), L.stream()),
+                'bbb_gauss_prior_logprob')
+
+    def gauss_bwd(self, params, eps, S, sample, pg, out_scale, grads, layer_ids=None):
+        gp, gq, gp_dev, gq_dev, g_stride = pg[1]
+        if gp == 0.0 and gq == 0.0:
+            return
+        tab, n, keep = _gauss_prior_table(params, self.gauss, eps, sample, S, grads, layer_ids)
+        rng = eps.rng(0)
+        L.check(L.lib().bbb_gauss_prior_logprob_bwd(tab, n, S, C.byref(rng), gp, gq, L.ptr(gp_dev), L.ptr(gq_dev),
+                                                    g_stride, L.ptr(out_scale), L.stream()),
+                'bbb_gauss_prior_logprob_bwd')
 
     @staticmethod
     def shape(w):
@@ -396,20 +458,28 @@ class _WeightSampling:
                 mode in ('classification', 'regression') and L.mlp_supported(dims, S, B, L.F_TF32))
 
     def network_forward(self, x2, target, params, eps, S, B, sigma, mode, need_grad, beta_h, beta_d, out4):
+        gauss_fwd = None
+        if self.gauss is not None:
+            def gauss_fwd(logp, logq):
+                self.gauss_fwd(params, eps, S, True, (logp, logq))
         return _mlp_forward_call(x2, target, params, eps, self.prior, S, B, sigma, mode, need_grad, beta_h, beta_d,
-                                 out4)
+                                 out4, gauss_fwd)
 
     def network_backward(self, x2, ys, dxs, d_out, params, S, eps, gargs, scale):
         """ONE C call for the whole backward (bbb_mlp_bwd): ys are the stored hidden pre-activations, dxs[l + 1] the
-        zero-filled gradient w.r.t. hidden layer l's pre-activation output."""
+        zero-filled gradient w.r.t. hidden layer l's pre-activation output.  A per-weight prior's terms are added by
+        their own kernel after it, before any layer's gradients are reported."""
         nl = len(params)
         grads = _alloc_grads(params)
         tab = _mlp_layer_table(params, eps, list(ys) + [None], list(dxs[1:nl]) + [d_out], grads)
         rng = eps.rng(0)
-        gp, gq, gp_dev, gq_dev, g_stride = gargs
+        pg = (0, gargs)
+        gp, gq, gp_dev, gq_dev, g_stride = gargs if self.gauss is None else self.layer_grad_args(pg)[1]
         L.check(L.lib().bbb_mlp_bwd(tab, nl, L.ptr(x2), S, x2.shape[0], C.byref(rng), C.byref(self.prior),
                                     L.F_SAMPLE | L.F_TF32, gp, gq, L.ptr(gp_dev), L.ptr(gq_dev), g_stride,
                                     L.ptr(scale), L.stream()), 'bbb_mlp_bwd')
+        if self.gauss is not None:
+            self.gauss_bwd(params, eps, S, True, pg, scale, grads)
         if grad_ready_hook is not None:
             for l in reversed(range(nl)):
                 grad_ready_hook(l, grads[l].flat)
@@ -420,14 +490,37 @@ class _LocalReparam:
     """Local reparameterisation (networks.py:90-138, 211-225): weights [in, out], the pre-activation sampled per row
     from its mean x mu and variance delta = x^2 sigma^2 (kept per layer for the backward), one closed-form KL for the
     whole call, its gradient taken through BBB_F_LOGPROB in the backward."""
-    __slots__ = ('sigma_p',)
+    __slots__ = ('sigma_p', 'gauss')
     has_delta = True
     eps_per_row = True           # the noise is drawn per input row: a chunked pass draws it chunk by chunk
     reuse_error = ('sample_elbo_lr: this graph was already differentiated (retain_graph=True is not supported by the '
                    'TF32 local-reparameterisation path: its saved state is single-use)')
 
-    def __init__(self, sigma_p):
+    def __init__(self, sigma_p, gauss=None):
         self.sigma_p = float(sigma_p)
+        self.gauss = gauss       # per layer (weight m, weight r, bias m, bias r) of a per-weight prior, or None
+
+    def with_gauss(self, gauss):
+        """This estimator with the per-weight Gaussian prior `gauss` in place of N(0, sigma_p) (None: as is)."""
+        return self if gauss is None else _LocalReparam(self.sigma_p, gauss)
+
+    @staticmethod
+    def layer_grad_args(pg):
+        """The layer calls run without BBB_F_LOGPROB when the per-weight prior kernels take the KL terms."""
+        gflags, gargs = pg
+        return gflags & ~L.F_LOGPROB, gargs
+
+    def gauss_fwd(self, params, eps, S, sample, lp, layer_ids=None):
+        tab, n, _ = _gauss_prior_table(params, self.gauss, _EpsPlan(), True, S, layer_ids=layer_ids)
+        L.check(L.lib().bbb_gauss_prior_kl(tab, n, L.ptr(lp[0]), L.stream()), 'bbb_gauss_prior_kl')
+
+    def gauss_bwd(self, params, eps, S, sample, pg, out_scale, grads, layer_ids=None):
+        gflags, (g_kl, g_kl_dev) = pg
+        if not gflags & L.F_LOGPROB:
+            return
+        tab, n, _ = _gauss_prior_table(params, self.gauss, _EpsPlan(), True, S, grads, layer_ids)
+        L.check(L.lib().bbb_gauss_prior_kl_bwd(tab, n, g_kl, L.ptr(g_kl_dev), L.ptr(out_scale), L.stream()),
+                'bbb_gauss_prior_kl_bwd')
 
     @staticmethod
     def shape(w):
@@ -543,10 +636,13 @@ def _forward(est, x2, params, S, eps, sample, logprob, tf32, lp, ys=None, deltas
     given, runs the last layer instead of the layer call (the fused ELBO tail)."""
     B = x2.shape[0]
     ro = est.relu_out(params, B, tf32)
-    base = ((L.F_SAMPLE if sample else 0) | (L.F_LOGPROB if logprob else 0) | (L.F_TF32 if tf32 else 0) |
+    gauss = logprob and est.gauss is not None       # the per-weight prior kernel takes the log-prob terms
+    base = ((L.F_SAMPLE if sample else 0) | (L.F_LOGPROB if logprob and not gauss else 0) | (L.F_TF32 if tf32 else 0) |
             (L.F_OUT_ZEROED if est.prezero(B) else 0))
     if ys is None:
         ys, deltas = _activations(est, params, S, B, sample, x2.device)
+    if gauss:
+        est.gauss_fwd(params, eps, S, sample, lp)
     inp, stride = x2, 0
     for l, p in enumerate(params):
         flags = base | (L.F_RELU_IN if l > 0 and not ro[l - 1] else 0) | (L.F_RELU_OUT if ro[l] else 0)
@@ -565,7 +661,7 @@ def _backward(est, x2, ys, deltas, d_out, params, S, eps, sample, tf32, pg, out_
     layer needs a separate mask pass over dy."""
     B = x2.shape[0]
     ro = est.relu_out(params, B, tf32)
-    gflags, gargs = pg
+    gflags, gargs = pg if est.gauss is None else est.layer_grad_args(pg)
     base = ((L.F_SAMPLE if sample else 0) | (L.F_TF32 if tf32 else 0) | (L.F_OUT_ZEROED if est.prezero(B) else 0) |
             gflags)
     grads = _alloc_grads(params)
@@ -586,11 +682,17 @@ def _backward(est, x2, ys, deltas, d_out, params, S, eps, sample, tf32, pg, out_
             flags |= L.F_SCALE_DX
         x_in, stride = (x2, 0) if l == 0 else (ys[l - 1], B * est.shape(p[0])[0])
         est.bwd(dy, x_in, stride, p, eps, l, deltas[l], S, B, flags, gargs, out_scale, dx, g)
-        if grad_ready_hook is not None:
+        if grad_ready_hook is not None and est.gauss is None:
             grad_ready_hook(l, g.flat)
         dy = dx
         if l == 0:
             dx0 = dx
+    if est.gauss is not None:
+        # one launch adds the prior terms of every layer; only then are the gradients complete and reported
+        est.gauss_bwd(params, eps, S, sample, pg, out_scale, grads)
+        if grad_ready_hook is not None:
+            for l in reversed(range(len(params))):
+                grad_ready_hook(l, grads[l].flat)
     return dx0, grads
 
 
@@ -638,7 +740,11 @@ class _Linear(torch.autograd.Function):
         acc = torch.zeros(est.acc_len(1), dtype=torch.float64, device=x2.device)
         y = torch.empty((1, B, out), dtype=torch.float32, device=x2.device)
         delta = torch.empty_like(y) if sample and est.has_delta else None
-        flags = (L.F_SAMPLE if sample else 0) | (L.F_LOGPROB if logprob else 0) | (L.F_TF32 if tf32 else 0)
+        gauss = logprob and est.gauss is not None
+        if gauss:
+            est.gauss_fwd([p], eps, 1, sample, est.lp(acc, 1), [layer_id])
+        flags = ((L.F_SAMPLE if sample else 0) | (L.F_LOGPROB if logprob and not gauss else 0) |
+                 (L.F_TF32 if tf32 else 0))
         est.fwd(x2, 0, p, eps, layer_id, 1, B, flags, y, delta, est.lp(acc, 1))
         _save(ctx, x2=x2, p=p, delta=delta, eps=eps.tensors())
         ctx.est, ctx.sample, ctx.logprob, ctx.layer_id, ctx.tf32, ctx.eps = est, sample, logprob, layer_id, tf32, eps
@@ -658,19 +764,26 @@ class _Linear(torch.autograd.Function):
         dy = _f32c(dy).reshape(1, B, out)
         g = tuple(torch.empty_like(t) for t in p)
         dx = torch.empty((1, B, inn), dtype=torch.float32, device=x2.device) if ctx.x_rg else None
-        gflags, gargs = est.grad_args(dlp, ctx.logprob, True)
+        pg = est.grad_args(dlp, ctx.logprob, True)
+        gflags, gargs = pg if est.gauss is None else est.layer_grad_args(pg)
         flags = ((L.F_SAMPLE if ctx.sample else 0) | (L.F_TF32 if ctx.tf32 else 0) | (0 if ctx.x_rg else L.F_NO_DX) |
                  gflags)
         est.bwd(dy, x2, 0, p, ctx.eps, ctx.layer_id, s['delta'], 1, B, flags, gargs, None, dx, g)
+        if est.gauss is not None:
+            est.gauss_bwd([p], ctx.eps, 1, ctx.sample, pg, None, [g], [ctx.layer_id])
         return (None, dx.view(ctx.xshape) if ctx.x_rg else None, *g, None, None, None, None)
 
 
-def bayes_linear(x, wm, wr, bm, br, prior, sample, logprob, layer_id=0, tf32=False):
-    return _Linear.apply(_WeightSampling(prior), x, wm, wr, bm, br, sample, logprob, layer_id, tf32)
+def bayes_linear(x, wm, wr, bm, br, prior, sample, logprob, layer_id=0, tf32=False, gauss=None):
+    """gauss: (weight m, weight r, bias m, bias r) of a per-weight prior N(m, softplus(r)^2), replacing `prior`."""
+    est = _WeightSampling(prior, None if gauss is None else [gauss])
+    return _Linear.apply(est, x, wm, wr, bm, br, sample, logprob, layer_id, tf32)
 
 
-def lr_linear(x, wm, wr, bm, br, sigma_p, sample, calc_kl, layer_id=0):
-    return _Linear.apply(_LocalReparam(sigma_p), x, wm, wr, bm, br, sample, calc_kl, layer_id, False)
+def lr_linear(x, wm, wr, bm, br, sigma_p, sample, calc_kl, layer_id=0, gauss=None):
+    """gauss: as bayes_linear's, replacing N(0, sigma_p)."""
+    est = _LocalReparam(sigma_p, None if gauss is None else [gauss])
+    return _Linear.apply(est, x, wm, wr, bm, br, sample, calc_kl, layer_id, False)
 
 
 # =========================================================================================

@@ -52,6 +52,22 @@ class GaussianNode:
                 - ((input - self.mu) ** 2) / (2 * self.sigma ** 2)).sum()
 
 
+PRIOR_BUFFERS = ('prior_weight_mu', 'prior_weight_rho', 'prior_bias_mu', 'prior_bias_rho')
+
+
+def _register_prior_buffers(layer):
+    """The optional per-weight Gaussian prior N(prior_mu, softplus(prior_rho)^2) of a layer, in the posterior's own
+    parametrisation and layout.  Not persistent: the state_dict keeps the reference's keys."""
+    for name in PRIOR_BUFFERS:
+        layer.register_buffer(name, None, persistent=False)
+
+
+def gauss_prior(layer):
+    """(weight m, weight r, bias m, bias r) of the layer's per-weight prior, or None."""
+    bufs = tuple(getattr(layer, name) for name in PRIOR_BUFFERS)
+    return None if bufs[0] is None else bufs
+
+
 class BayesianLinear(nn.Module):
     """Weight-sampling Bayesian FC layer (networks.py:48-88)."""
 
@@ -74,6 +90,7 @@ class BayesianLinear(nn.Module):
         self.log_variational_posterior = 0
         self.layer_id = 0          # Philox tensor-id base; BayesianNetwork numbers its layers
         self.tf32 = False
+        _register_prior_buffers(self)
 
     def params(self):
         return (self.weight_mu, self.weight_rho, self.bias_mu, self.bias_rho)
@@ -81,7 +98,8 @@ class BayesianLinear(nn.Module):
     def forward(self, input, sample=False, calculate_log_probs=False):
         do_sample = self.training or sample
         do_logp = self.training or calculate_log_probs
-        y, lp, lq = F.bayes_linear(input, *self.params(), self._prior, do_sample, do_logp, self.layer_id, self.tf32)
+        y, lp, lq = F.bayes_linear(input, *self.params(), self._prior, do_sample, do_logp, self.layer_id, self.tf32,
+                                   gauss_prior(self))
         if do_logp:
             self.log_prior, self.log_variational_posterior = lp, lq
         else:
@@ -105,6 +123,7 @@ class BayesianLinearLR(nn.Module):
         self.bias_kl_cost = 0
         self.kl_cost = 0
         self.layer_id = 0
+        _register_prior_buffers(self)
 
     def params(self):
         return (self.weight_mu, self.weight_rho, self.bias_mu, self.bias_rho)
@@ -121,7 +140,8 @@ class BayesianLinearLR(nn.Module):
         # without sampling reads an undefined w_sigma (networks.py:134); both are fixed here (SURVEY B-4).
         do_sample = self.training or sample
         do_kl = self.training or calculate_log_probs
-        y, kl = F.lr_linear(input, *self.params(), self.weight_prior[1], do_sample, do_kl, self.layer_id)
+        y, kl = F.lr_linear(input, *self.params(), self.weight_prior[1], do_sample, do_kl, self.layer_id,
+                            gauss_prior(self))
         if do_kl:
             self.kl_cost = kl
         return y

@@ -9,7 +9,7 @@ import torch
 from torch import nn
 
 from . import functional as F
-from .layers import BayesianLinear, BayesianLinearLR
+from .layers import PRIOR_BUFFERS, BayesianLinear, BayesianLinearLR, gauss_prior
 
 _HALF_LOG_2PI = 0.5 * math.log(2 * math.pi)
 
@@ -73,6 +73,17 @@ class BayesianNetwork(nn.Module):
     'heteroscedastic', a learned per-input noise (Kendall & Gal 2017): the last layer has 2 * classes outputs [f | r],
     the mean f and a raw scale r, and sigma(x) = sigma_min + softplus(r) with 'sigma_min' (default 1e-3) > 0.  `classes`
     still counts the targets D; forward / sample_predict return the raw [.., 2D] outputs.
+
+    Per-weight Gaussian priors (posterior_to_prior, set_prior, clear_prior): every weight and bias w_i can get its own
+    prior N(m_i, sp_i^2), which replaces the model_params prior in the ELBO of both estimators (sample_elbo: Monte Carlo
+    log p of the sampled weights; sample_elbo_lr: the closed-form KL) and in log_prior() / kl_cost() after a training
+    forward.  posterior_to_prior() makes the current posterior the prior of the next task (variational continual
+    learning, Nguyen et al. 2018).  The prior lives in non-persistent buffers of each layer (prior_weight_mu / _rho,
+    prior_bias_mu / _rho, sp = softplus(rho)): it is NOT part of state_dict, which keeps the reference's keys.
+    Prediction (sample_predict, predictive) and evaluation mode do not read it.  A captured GraphedTrainStep reads the
+    buffers by pointer, so refreshing them in place (posterior_to_prior or set_prior on a net that already has a
+    per-weight prior of the same shapes) is seen by later replays; switching between no per-weight prior and one
+    changes the launch sequence and needs a new capture.
     """
 
     def __init__(self, model_params):
@@ -122,6 +133,78 @@ class BayesianNetwork(nn.Module):
 
     def layers(self):
         return [getattr(self, f'l{i + 1}') for i in range(self.n_layers)]
+
+    # ---- per-weight Gaussian priors -------------------------------------------------------------------------------
+    def _store_prior(self, layer, values):
+        """Write a layer's four prior tensors: in place where the buffers exist with the same shape and device (a
+        captured graph keeps reading them), else as new buffers."""
+        for name, v in zip(PRIOR_BUFFERS, values):
+            cur = getattr(layer, name)
+            if cur is not None and cur.shape == v.shape and cur.device == v.device:
+                cur.copy_(v)
+            else:
+                setattr(layer, name, v.detach().to(torch.float32).contiguous().clone())
+
+    def posterior_to_prior(self):
+        """Make the current posterior q(w) = N(mu, softplus(rho)^2) of every weight and bias its prior: a copy of
+        (mu, rho) into the layer's prior buffers (in place when they exist)."""
+        with torch.no_grad():
+            for l in self.layers():
+                self._store_prior(l, l.params())
+
+    def set_prior(self, layers):
+        """Set a per-weight Gaussian prior: `layers` holds one (weight_mean, weight_sigma, bias_mean, bias_sigma) per
+        layer, each a tensor of the shape of that layer's weight_mu / bias_mu (its own layout: [out, in] for weight
+        sampling, [in, out] for local reparameterisation) on the parameters' device, or a python number for all of
+        them.  sigma is stored as rho = log(expm1(sigma)), formed in float64.  Raises ValueError for a wrong number of
+        layers, a shape or device mismatch, or a sigma that is not finite and > 0; nothing is changed then."""
+        ls = self.layers()
+        layers = list(layers)
+        if len(layers) != len(ls):
+            raise ValueError(f'set_prior: expected one (weight_mean, weight_sigma, bias_mean, bias_sigma) per layer, '
+                             f'{len(ls)} layers, got {len(layers)}')
+        staged = []
+        for i, (l, entry) in enumerate(zip(ls, layers)):
+            entry = tuple(entry)
+            if len(entry) != 4:
+                raise ValueError(f'set_prior: layer {i + 1}: expected (weight_mean, weight_sigma, bias_mean, '
+                                 f'bias_sigma), got {len(entry)} values')
+            vals = []
+            for k, (v, ref) in enumerate(zip(entry, (l.weight_mu, l.weight_mu, l.bias_mu, l.bias_mu))):
+                what = f'set_prior: layer {i + 1} {("weight_mean", "weight_sigma", "bias_mean", "bias_sigma")[k]}'
+                if torch.is_tensor(v):
+                    if tuple(v.shape) != tuple(ref.shape):
+                        raise ValueError(f'{what}: shape {tuple(v.shape)}, expected {tuple(ref.shape)}')
+                    if v.device != ref.device:
+                        raise ValueError(f'{what}: device {v.device}, expected {ref.device}')
+                    v = v.detach().to(torch.float64)
+                else:
+                    v = torch.full(tuple(ref.shape), float(v), dtype=torch.float64, device=ref.device)
+                if k % 2:
+                    if not bool(torch.isfinite(v).all()) or not bool((v > 0).all()):
+                        raise ValueError(f'{what}: every sigma must be finite and > 0')
+                    v = v + torch.log(-torch.expm1(-v))      # log(expm1(sigma)), stable for large sigma
+                vals.append(v.to(torch.float32).contiguous())
+            staged.append(vals)
+        with torch.no_grad():
+            for l, vals in zip(ls, staged):
+                self._store_prior(l, vals)
+
+    def clear_prior(self):
+        """Drop the per-weight priors: the model_params prior applies again."""
+        for l in self.layers():
+            for name in PRIOR_BUFFERS:
+                setattr(l, name, None)
+
+    def _gauss_priors(self):
+        """Per layer (weight m, weight r, bias m, bias r) of the per-weight prior, or None when no layer has one."""
+        ps = [gauss_prior(l) for l in self.layers()]
+        if all(p is None for p in ps):
+            return None
+        if any(p is None for p in ps):
+            raise ValueError('a per-weight prior must be set on every layer of the network or on none '
+                             '(posterior_to_prior / set_prior set all of them)')
+        return ps
 
     def forward(self, x, sample=False):
         if self.mode == 'classification':
@@ -270,16 +353,17 @@ class BayesianNetwork(nn.Module):
         forward's log-prob outputs, the NLL summed over the samples) for the caller to assemble."""
         x2 = self._flat_input(input)
         params = [l.params() for l in self.layers()]
+        est = self._est.with_gauss(self._gauss_priors())
         if self._het:
             self._check_no_sigma(sigma)
             target = self._het_target(target, x2.shape[0])
             if self.fused:
-                return F._elbo(self._est, x2, target, beta, samples, self.sigma_min, self.mode, params, self.tf32,
+                return F._elbo(est, x2, target, beta, samples, self.sigma_min, self.mode, params, self.tf32,
                                self.likelihood), None, None
         elif self._fusable(x2, target):
-            return F._elbo(self._est, x2, target, beta, samples, sigma, self.mode, params, self.tf32, 'gaussian'), \
+            return F._elbo(est, x2, target, beta, samples, sigma, self.mode, params, self.tf32, 'gaussian'), \
                 None, None
-        outs, *lp = F._network_forward(self._est, x2, params, samples, True, True, self.tf32)
+        outs, *lp = F._network_forward(est, x2, params, samples, True, True, self.tf32)
         negative_log_likelihood = torch.zeros(1, device=outs.device)
         for i in range(samples):
             negative_log_likelihood = negative_log_likelihood + self.get_nll(outs[i], target, sigma)

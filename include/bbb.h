@@ -163,6 +163,46 @@ int bbb_kl_gauss(const float *mu, const float *rho, float sigma_p, int64_t n, do
 int bbb_philox_fill_normal(float *out, int64_t n, uint64_t seed, uint32_t step, uint32_t sample,
                            uint32_t tensor_id, void *stream);
 
+/* ---- per-weight Gaussian priors p(w_i) = N(m_i, sp_i^2), sp_i = softplus(r_i) -----------------------------------------
+ * The prior is stored in the posterior's own parametrisation, so a trained posterior becomes the next task's prior by a
+ * copy of (mu, rho) (variational continual learning, Nguyen et al. 2018).  The layer kernels do not read it: a caller
+ * runs them WITHOUT BBB_F_LOGPROB (weight sampling: gp = gq = 0 and no gp_dev / gq_dev in the backward) and adds the
+ * prior terms with the calls below, one launch for all tensors of a network (at most BBB_GAUSS_PRIOR_MAX_TENSORS).
+ * One tensor of the table: */
+#define BBB_GAUSS_PRIOR_MAX_TENSORS 64
+typedef struct bbb_gauss_prior_tensor {
+  const float *mu, *rho;             /* q: a layer's weight or bias parameters, n elements                               */
+  const float *prior_mu, *prior_rho; /* p = N(prior_mu, softplus(prior_rho)^2), n elements                              */
+  const float *eps;                  /* [S, n] injected eps (parity mode) or NULL: Philox                               */
+  float *grad_mu, *grad_rho;         /* backward only: ADDED to                                                         */
+  int64_t n;
+  uint32_t tensor_id;                /* Philox counter word 2: 2l for a weight, 2l+1 for its bias                       */
+} bbb_gauss_prior_tensor;
+/* weight sampling (Monte Carlo, as sample_elbo): w_s = mu + softplus(rho) eps_s, eps_s regenerated at
+ * (element/4, rng->sample_base + s, tensor_id, rng->step [+ *rng->step_dev]), i.e. the SAME eps the layer kernels drew
+ * (rng->layer is ignored: every tensor carries its own id).
+ *   logp[s] += sum log N(w_s; m, sp^2),  logq[s] += sum log N(w_s; mu, sigma^2)          (logp, logq: [S] fp64)   */
+int bbb_gauss_prior_logprob(const bbb_gauss_prior_tensor *t, int32_t n_tensors, int64_t S, const bbb_rng *rng,
+                            double *logp, double *logq, void *stream);
+/* its gradient, gp_s / gq_s / out_scale exactly as bbb_linear_bwd defines them (gp_s = gp * gp_dev[s * g_dev_stride]
+ * when gp_dev is given, likewise gq_s; c = out_scale_dev ? *out_scale_dev : 1):
+ *   grad_mu  += c sum_s gp_s (-(w_s - m) / sp^2)
+ *   grad_rho += c sigmoid(rho) sum_s [ gp_s (-(w_s - m) / sp^2) eps_s - gq_s / sigma ]                                */
+int bbb_gauss_prior_logprob_bwd(const bbb_gauss_prior_tensor *t, int32_t n_tensors, int64_t S, const bbb_rng *rng,
+                                float gp, float gq, const float *gp_dev, const float *gq_dev, int64_t g_dev_stride,
+                                const float *out_scale_dev, void *stream);
+/* local reparameterisation: closed-form KL(q || p) = sum [ log(sp/sigma) + (sigma^2 + (mu - m)^2) / (2 sp^2) - 1/2 ]
+ * (networks.py:109-114 with p_mu = m), *kl += it; exactly 0 per element when (mu, rho) == (m, r).
+ * bwd: grad_mu += c (mu - m)/sp^2,  grad_rho += c sigmoid(rho) (sigma/sp^2 - 1/sigma),
+ *   c = g_kl * (g_kl_dev ? *g_kl_dev : 1) * (out_scale_dev ? *out_scale_dev : 1)
+ * All four: any n (n % 4 tails, pointers without 16-byte alignment), n == 0 is a no-op for that tensor; launched with
+ * programmatic dependent launch.  BBB_EINVAL before any device work for n_tensors outside [0, 64], a null table with
+ * n_tensors > 0, n < 0, a null mu / rho / prior_mu / prior_rho (grad_mu / grad_rho in a backward) of a non-empty
+ * tensor, a null logp / logq / rng / kl, or S <= 0 on the log-prob calls. */
+int bbb_gauss_prior_kl(const bbb_gauss_prior_tensor *t, int32_t n_tensors, double *kl, void *stream);
+int bbb_gauss_prior_kl_bwd(const bbb_gauss_prior_tensor *t, int32_t n_tensors, float g_kl, const float *g_kl_dev,
+                           const float *out_scale_dev, void *stream);
+
 /* ---- consumers of the (mu, rho) stream: SNR pruning (weight_pruning.py:81-115) -------------------------------------------
  * bbb_snr:       snr_out[i] = 10 log10(|mu_i| / softplus(rho_i))   (compute_snr, weight_pruning.py:81-83; decibels)
  * bbb_snr_prune: mu_i, rho_i *= (snr_i > threshold_db), in place (prune_weights, weight_pruning.py:85-115: the same mask
